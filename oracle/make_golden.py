@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY.  Generates tests/golden/*.npz by running the UNMODIFIED reference
-code (imported from /root/reference through oracle/ref_stub.py) on CPU in fp32, with the
-deterministic synthetic weights / inputs of cmtcoop_b200.synth.  Run in the build container:
+code (imported through oracle/ref_stub.py from the checkout CMT_REFERENCE_ROOT names) on CPU in fp32, with
+the deterministic synthetic weights / inputs of cmtcoop_b200.synth:
 
-    python oracle/make_golden.py
+    CMT_REFERENCE_ROOT=<checkout of the original project> python oracle/make_golden.py
 
 Each file holds the reference outputs for one head class on the "mini" case
 (synth.mini_case): outs_dec, every task-head tensor, top-k indices/scores, and for the

@@ -1,19 +1,19 @@
 """TEST INFRASTRUCTURE ONLY -- never imported by the product path.
 
-Loader that imports the *unmodified* reference hot-path files straight from
-``/root/reference`` (read-only) so that their CPU/fp32 output can be dumped as
+Loader that imports the *unmodified* reference hot-path files straight from the
+checkout ``$CMT_REFERENCE_ROOT`` names (read-only) so that their CPU/fp32 output can be dumped as
 golden vectors (``oracle/make_golden.py``) and used to pin the restatement in
 ``oracle/cmt_oracle.py``.
 
 The reference needs mmcv-full 1.6.2 / mmdet 2.28.2 / mmdet3d 1.0.0rc6 /
 flash-attn 0.2.2 (reference ``Dockerfile:47-70``), none of which is installed
-and none of which lives under ``/root/reference``.  The handful of entry points
+and none of which lives in the reference tree.  The handful of entry points
 the seven hot-path files import are restated here from those packages'
 published behaviour (SURVEY.md appendix B lists every name).  Because that
 third-party arithmetic is a restatement, parity for it is "unpinned by a
 reference test" -- the reference ships no tests at all (SURVEY.md section 4).
 
-``/root/reference`` does not exist on the GPU box; nothing under ``tests -m gpu``,
+The reference tree is not part of this repository; nothing under ``tests -m gpu``,
 ``bench.py`` or ``__graft_entry__.smoke`` may import this module.
 """
 from __future__ import annotations
@@ -27,11 +27,12 @@ import types
 import torch
 import torch.nn as nn
 
-REFERENCE_ROOT = os.environ.get("CMT_REFERENCE_ROOT", "/root/reference")
+# a checkout of the original CMT-Cooperative-Perception project; unset: the tests that run it are skipped
+REFERENCE_ROOT = os.environ.get("CMT_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "projects", "mmdet3d_plugin"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "projects", "mmdet3d_plugin"))
 
 
 # --------------------------------------------------------------------------
@@ -350,12 +351,12 @@ _INSTALLED = False
 
 def install_stubs():
     """Seed sys.modules with the stub packages + namespace packages that point
-    into /root/reference (skipping its heavy __init__.py files)."""
+    into REFERENCE_ROOT (skipping its heavy __init__.py files)."""
     global _INSTALLED
     if _INSTALLED:
         return
     if not reference_available():
-        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference tree not found at CMT_REFERENCE_ROOT={REFERENCE_ROOT!r}")
     plug = os.path.join(REFERENCE_ROOT, "projects", "mmdet3d_plugin")
 
     def ns(name, path):

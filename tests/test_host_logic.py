@@ -12,6 +12,7 @@ from hypothesis import given, settings, strategies as st
 from cmtcoop_b200 import _lib, ops, parallel, synth
 from cmtcoop_b200 import plugin
 from oracle import cmt_oracle as O
+from oracle import ref_stub
 
 
 @pytest.mark.parametrize("kind", synth.HEAD_KINDS)
@@ -202,8 +203,8 @@ def test_graph_runner_calibration_key():
 
 
 # ---------------------------------------------------------------------------------------------
-# the reference's own configs (when the reference tree is present: this container, not the GPU box)
-REF_CONFIGS = "/root/reference/projects/configs"
+# the reference's own configs (when CMT_REFERENCE_ROOT names a checkout of the original project)
+REF_CONFIGS = os.path.join(ref_stub.REFERENCE_ROOT, "projects", "configs")
 
 
 def _reference_config_files():
@@ -211,7 +212,8 @@ def _reference_config_files():
     return sorted(glob.glob(os.path.join(REF_CONFIGS, "**", "*.py"), recursive=True))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CONFIGS), reason="reference tree not present")
+@pytest.mark.skipif(not ref_stub.reference_available(),
+                    reason="CMT_REFERENCE_ROOT does not name a checkout of the original project")
 def test_every_reference_config_builds_its_head_unchanged():
     """All 13 config files of the reference: exec the file (plain python dicts, no _base_ inheritance), take
     model['pts_bbox_head'] with the detector's train/test cfg folded in exactly as MVXTwoStageDetector.__init__ does

@@ -1,5 +1,7 @@
-"""Where /root/reference exists (the build container), run the UNMODIFIED reference live against the
-oracle on a shape that is NOT among the committed goldens.  Skipped on the GPU box."""
+"""Where CMT_REFERENCE_ROOT names a checkout of the original project, run the UNMODIFIED reference live against
+the oracle on a shape that is NOT among the committed goldens (B=1, 13x13 BEV map, 60 queries, 3 camera views,
+2 vehicle + 1 infrastructure views).  Skipped otherwise: the committed goldens (test_oracle_golden.py) compare with
+the reference on the mini case only (B=2, 24x24 BEV map, 96 queries)."""
 import numpy as np
 import pytest
 import torch
@@ -8,7 +10,8 @@ from cmtcoop_b200 import synth
 from oracle import cmt_oracle as O
 from oracle import ref_stub
 
-pytestmark = pytest.mark.skipif(not ref_stub.reference_available(), reason="/root/reference not present")
+pytestmark = pytest.mark.skipif(not ref_stub.reference_available(),
+                                reason="CMT_REFERENCE_ROOT does not name a checkout of the original project")
 
 
 @pytest.mark.parametrize("kind", ["CmtHead", "CmtImageHeadCoop"])
