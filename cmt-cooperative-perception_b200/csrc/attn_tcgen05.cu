@@ -155,21 +155,7 @@ __global__ void pack_key_mask_kernel(const unsigned char* keep, unsigned long lo
 }
 
 namespace attndb {
-#ifndef CMT_ATTN_NWG
-#define CMT_ATTN_NWG 3
-#endif
-// CMT_ATTN_PIPE=1: software-pipelined static softmax loop (half a score tile exponentiated while the other half's TMEM load
-// is in flight).  Measured in-step (B=8, 56 400 tokens): 880 us per launch against 824 us for the plain loop -- the wait
-// instructions between the halves split the 32-pair region the compiler otherwise interleaves freely (MUFU, FMA-pipe
-// polynomial and conversion work of both halves), and that instruction-level parallelism is worth more than the hidden
-// tcgen05.ld round trip.  Kept off, for the record.
-#ifndef CMT_ATTN_PIPE
-#define CMT_ATTN_PIPE 0
-#endif
-#ifndef CMT_ATTN_NACC
-#define CMT_ATTN_NACC 1     // independent row-sum accumulators per thread (breaks the 32-long dependent FADD2 chain)
-#endif
-constexpr int NWG = CMT_ATTN_NWG;
+constexpr int NWG = 3;                  // softmax warpgroups (one 128-row Q tile each)
 constexpr int QBLK = NWG * 128;
 constexpr int KT = 64;
 constexpr int NK = 8, NV = 8;
@@ -181,22 +167,8 @@ constexpr int KV_BYTES = 64 * 32 * 2;   // 4 KB per K tile / V^T tile
 // sub-partitions, and the issuers sleep in hardware on their P waits (try_wait with a suspend hint) instead of
 // polling: their wake-up latency hides under the double-buffered scores, their issue slots do not.
 // Measured (B=8, 56 400 tokens, us per launch): 1 polling issuer 1058, 1 sleeping 1056, 3 polling 992, 3 sleeping 983.
-#ifndef CMT_ATTN_NISS
-#define CMT_ATTN_NISS 3
-#endif
-#ifndef CMT_ISSUER_WAIT
-#define CMT_ISSUER_WAIT mbar_wait_sleep
-#endif
-#ifndef CMT_S_WAIT
-#define CMT_S_WAIT mbar_wait              // softmax warps: scores ready
-#endif
-#ifndef CMT_KV_WAIT
-#define CMT_KV_WAIT mbar_wait_sleep       // issuer: K / V stage full
-#endif
-#ifndef CMT_PROD_WAIT
-#define CMT_PROD_WAIT mbar_wait_sleep     // TMA producer: K / V stage empty
-#endif
-constexpr int NISS = CMT_ATTN_NISS;                    // MMA issuer warps (warpgroup i is served by issuer i % NISS)
+// The TMA producer waits sleep as well; only the softmax warps' wait on their scores polls (mbar_wait).
+constexpr int NISS = 3;                                // MMA issuer warps (warpgroup i is served by issuer i % NISS)
 constexpr int THREADS = NWG * 128 + 32 + NISS * 32;   // softmax warps, TMA warp, issuer warps
 constexpr int OFF_Q = 0;
 constexpr int OFF_K = OFF_Q + NWG * Q_BYTES;
@@ -210,17 +182,14 @@ constexpr float RESCALE_THRESHOLD = 8.0f;
 // DB_POLY - 1 of every 16-pair chunk use the packed cubic (ex2_poly_pair).  Measured (B=8, 56 400 tokens, same
 // box): off 1100 us, 1/16 1110, 1/8 1056, 1/6 1029, 1/5 1077, 1/4 1106, 1/3 1140, 1/2 1190; with the three sleeping
 // issuers (below): off 1041, i%8 969, i%6 958, i%5 946 (shipped: 6 of 32 pairs), i%4 976, i%3 1033.
-#ifndef CMT_ATTN_DB_POLY
-#define CMT_ATTN_DB_POLY 5
-#endif
-constexpr int DB_POLY = CMT_ATTN_DB_POLY;
+constexpr int DB_POLY = 5;
 // Static softmax shift (see the softmax warps below): items whose Cauchy-Schwarz score bound is at most STATIC_LIMIT
 // skip the row maximum and the rescale machinery; their freed ALU / issue slots take more polynomial exponentials.
 // Measured with a fixed shift (B=8, 56 400 tokens): online i%5 946 us; static i%5 896, i%4 892, i%3 865.
-#ifndef CMT_ATTN_ST_POLY
-#define CMT_ATTN_ST_POLY 3
-#endif
-constexpr int ST_POLY = CMT_ATTN_ST_POLY;
+constexpr int ST_POLY = 3;
+// The lone active warp of a tail tile (see lone_warp below).  Measured (B=8, static kernel): every second pair
+// polynomial 806 us, all pairs 913.
+constexpr int LONE_POLY = 2;
 constexpr float STATIC_LIMIT = 60.0f;
 // pair i of a 16-pair chunk is polynomial when i % period == period - 1 (period 0: none)
 constexpr uint32_t poly_mask(int period) {
@@ -229,20 +198,9 @@ constexpr uint32_t poly_mask(int period) {
         if (period > 0 && i % period == period - 1) m |= 1u << i;
     return m;
 }
-// explicit masks override the periods: -DCMT_ATTN_ST_MASK=0x5555 puts every other pair on the FMA pipes
-#ifdef CMT_ATTN_ST_MASK
-constexpr uint32_t ST_MASK = CMT_ATTN_ST_MASK;
-#else
 constexpr uint32_t ST_MASK = poly_mask(ST_POLY);
-#endif
-#ifdef CMT_ATTN_DB_MASK
-constexpr uint32_t DB_MASK = CMT_ATTN_DB_MASK;
-#else
 constexpr uint32_t DB_MASK = poly_mask(DB_POLY);
-#endif
-#ifndef CMT_ATTN_LONE_POLY
-#define CMT_ATTN_LONE_POLY 2
-#endif
+constexpr uint32_t LONE_MASK = poly_mask(LONE_POLY);
 }  // namespace attndb
 
 // kMask: key padding mask variant (the unmasked instantiation carries none of its code: even an untaken mask
@@ -279,11 +237,7 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
 
     const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);   // provably warp-uniform
     const int lane = threadIdx.x & 31;
-#ifdef CMT_ATTN_TMA_LAST
-    constexpr int W_MMA = NWG * 4, W_TMA = NWG * 4 + NISS;   // issuers: W_MMA .. W_MMA + NISS - 1
-#else
-    constexpr int W_TMA = NWG * 4, W_MMA = NWG * 4 + 1;   // issuers: W_MMA .. W_MMA + NISS - 1
-#endif
+    constexpr int W_TMA = NWG * 4, W_MMA = W_TMA + 1;   // issuers: W_MMA .. W_MMA + NISS - 1
 
     if (warp == W_MMA && lane == 0) {
         tma_prefetch_desc(&tma_q);
@@ -350,7 +304,7 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
             for (int jj = 0; jj < n + 2; ++jj) {
                 if (jj < n) {
                     const uint32_t ks = kc % NK;
-                    CMT_PROD_WAIT(&k_empty[ks], ((kc / NK) & 1) ^ 1);
+                    mbar_wait_sleep(&k_empty[ks], ((kc / NK) & 1) ^ 1);
                     if (leader) {
                         mbar_arrive_expect_tx(&k_full[ks], KV_BYTES);
                         tma_load_4d(smem + OFF_K + ks * KV_BYTES, &tma_k, &k_full[ks], 0, tok_base + jj * KT, h, b);
@@ -359,7 +313,7 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
                 }
                 if (jj >= 2) {
                     const uint32_t vs = vc % NV;
-                    CMT_PROD_WAIT(&v_empty[vs], ((vc / NV) & 1) ^ 1);
+                    mbar_wait_sleep(&v_empty[vs], ((vc / NV) & 1) ^ 1);
                     if (leader) {
                         mbar_arrive_expect_tx(&v_full[vs], KV_BYTES);
                         tma_load_4d(smem + OFF_V + vs * KV_BYTES, &tma_v, &v_full[vs], tok_base + (jj - 2) * KT, 0, h, b);
@@ -420,8 +374,8 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
                 const uint32_t vs = vc % NV;
                 const uint32_t ks = kc % NK;
                 if (leader) CMT_TRACE(ii, g[ii], 6);
-                CMT_KV_WAIT(&v_full[vs], (vc / NV) & 1);
-                if (has2) CMT_KV_WAIT(&k_full[ks], (kc / NK) & 1);
+                mbar_wait_sleep(&v_full[vs], (vc / NV) & 1);
+                if (has2) mbar_wait_sleep(&k_full[ks], (kc / NK) & 1);
                 if (leader) CMT_TRACE(ii, g[ii], 7);
                 const uint64_t vdesc = make_kmajor_desc(smem_u32(smem + OFF_V + vs * KV_BYTES), 128);
                 const uint64_t kdesc = make_kmajor_desc(smem_u32(smem + OFF_K + ks * KV_BYTES), 64);
@@ -430,7 +384,7 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
                     if ((i % NISS) == ii && i < nact) {
                         const uint32_t bsel = g[i] & 1;
                         if (leader) CMT_TRACE(i, g[i], 11);
-                        CMT_ISSUER_WAIT(&p_full[2 * i + bsel], (g[i] >> 1) & 1);
+                        mbar_wait_sleep(&p_full[2 * i + bsel], (g[i] >> 1) & 1);
                         tc_fence_after();
                         if (leader) {
                             CMT_TRACE(i, g[i], 4);
@@ -510,7 +464,7 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
                 constexpr uint32_t PMASK = decltype(poly_tag)::value;
                 const uint32_t bsel = g & 1;
                 const uint32_t t_sb = t_s + bsel * 64;
-                CMT_S_WAIT(&my_s_full[bsel], (g >> 1) & 1);
+                mbar_wait(&my_s_full[bsel], (g >> 1) & 1);
                 if (tracer) CMT_TRACE(wg, g, 0);
                 tc_fence_after();
                 uint32_t s[2][32];
@@ -576,9 +530,7 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
                 // One PAIR of exponentials in POLY runs on the FMA pipes (packed cubic) instead of the MUFU; without
                 // the row-max work there are issue slots for more of them.
                 const uint64_t neg_m2 = pack_f32x2(-m, -m);
-                uint64_t l2v[CMT_ATTN_NACC];
-#pragma unroll
-                for (int a = 0; a < CMT_ATTN_NACC; ++a) l2v[a] = pack_f32x2(0.f, 0.f);
+                uint64_t l2 = pack_f32x2(0.f, 0.f);
 #pragma unroll
                 for (int c = 0; c < 2; ++c) {
                     uint32_t pk[16];
@@ -595,19 +547,14 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
                             e0 = ex2_approx(x0);
                             e1 = ex2_approx(x1);
                         }
-                        l2v[i % CMT_ATTN_NACC] = add_f32x2(l2v[i % CMT_ATTN_NACC], pack_f32x2(e0, e1));
+                        l2 = add_f32x2(l2, pack_f32x2(e0, e1));
                         pk[i] = pack_bf16x2(e0, e1);
                     }
                     tmem_st16(t_sb + c * 16, pk);
                 }
-                {
-                    uint64_t l2 = l2v[0];
-#pragma unroll
-                    for (int a = 1; a < CMT_ATTN_NACC; ++a) l2 = add_f32x2(l2, l2v[a]);
-                    float l0, l1;
-                    unpack_f32x2(l2, l0, l1);
-                    l += l0 + l1;
-                }
+                float l0, l1;
+                unpack_f32x2(l2, l0, l1);
+                l += l0 + l1;
                 tc_wait_st();
                 if (lane == 0) CMT_TRACE(wg, g, (warp & 3) == 0 ? 3 : 7 + (warp & 3));
                 tc_fence_before();
@@ -621,83 +568,13 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
             if (kStatic) m = 0.0f;
             // A tile with at most 32 queries (the 4-query tail of 900 = 7 * 128 + 4) has ONE active warp, and that warp
             // shares its sub-partition's MUFU with the full tile next door: the pass is then bound by that one
-            // sub-partition (trace: 957 of 1165 cycles per step in the shared warp).  The lone warp therefore takes ALL
-            // its exponentials through the polynomial on the otherwise idle FMA pipes and leaves the MUFU to its neighbour.
+            // sub-partition (trace: 957 of 1165 cycles per step in the shared warp).  The lone warp therefore takes every
+            // second pair of exponentials (LONE_POLY) through the polynomial on the otherwise idle FMA pipes and leaves
+            // more of the MUFU to its neighbour.
             const bool lone_warp = p.Nq - (qb * QBLK + wg * 128) <= 32;
-#if CMT_ATTN_PIPE
-            // Static-shift path, software-pipelined over the two 32-column halves of a score tile: the exponentials need no
-            // row statistic, so the first half can be exponentiated (and its P stored) while the TMEM load of the second
-            // half is in flight, and the first half of the NEXT step is loaded under the second half's exponentials.  A
-            // softmax warp then never sits on a tcgen05.ld round trip (three warps per scheduler cannot hide it).
-            auto run_static = [&](auto poly_tag) {
-                constexpr uint32_t PMASK = decltype(poly_tag)::value;
-                uint32_t s0[32], s1[32];
-                uint64_t l2 = pack_f32x2(0.f, 0.f);
-                auto half = [&](uint32_t (&sc)[32], uint32_t t_dst, int valid_c, uint32_t mbits) {
-                    if (kMask) {
-#pragma unroll
-                        for (int i = 0; i < 32; ++i)
-                            if (!((mbits >> i) & 1u)) sc[i] = 0xff800000u;
-                    } else if (valid_c < 32) {
-#pragma unroll
-                        for (int i = 0; i < 32; ++i)
-                            if (i >= valid_c) sc[i] = 0xc2fc0000u;   // -126: nothing next to weights >= 2^-60
-                    }
-                    uint32_t pk[16];
-#pragma unroll
-                    for (int i = 0; i < 16; ++i) {
-                        const uint64_t x2 = pack_f32x2(__uint_as_float(sc[2 * i]), __uint_as_float(sc[2 * i + 1]));
-                        float e0, e1;
-                        if ((PMASK >> i) & 1u) {
-                            ex2_poly_pair<kMask>(x2, e0, e1);
-                        } else {
-                            float x0, x1;
-                            unpack_f32x2(x2, x0, x1);
-                            e0 = ex2_approx(x0);
-                            e1 = ex2_approx(x1);
-                        }
-                        l2 = add_f32x2(l2, pack_f32x2(e0, e1));
-                        pk[i] = pack_bf16x2(e0, e1);
-                    }
-                    tmem_st16(t_dst, pk);
-                };
-                CMT_S_WAIT(&my_s_full[g & 1], (g >> 1) & 1);
-                tc_fence_after();
-                tmem_ld32(t_s + (g & 1) * 64, s0);
-                tc_wait_ld_regs(s0);
-                for (int jj = 0; jj < n; ++jj) {
-                    const uint32_t bsel = g & 1;
-                    const uint32_t t_sb = t_s + bsel * 64;
-                    tmem_ld32(t_sb + 32, s1);                       // second half in flight under the first half's work
-                    const int valid = p.kv_end - (p.kv_begin + (j0 + jj) * KT);
-                    unsigned long long mb = ~0ull;
-                    if (kMask) mb = __ldg(mask_row + j0 + jj);
-                    half(s0, t_sb, valid, static_cast<uint32_t>(mb));
-                    tc_wait_ld_regs(s1);
-                    if (jj + 1 < n) {                               // first half of the next step under the second half's work
-                        const uint32_t g1 = g + 1;
-                        CMT_S_WAIT(&my_s_full[g1 & 1], (g1 >> 1) & 1);
-                        tc_fence_after();
-                        tmem_ld32(t_s + (g1 & 1) * 64, s0);
-                    }
-                    half(s1, t_sb + 16, valid - 32, static_cast<uint32_t>(mb >> 32));
-                    tc_wait_st();
-                    tc_fence_before();
-                    mbar_arrive(&my_p_full[bsel]);
-                    ++g;
-                    if (jj + 1 < n) tc_wait_ld_regs(s0);
-                }
-                float l0, l1;
-                unpack_f32x2(l2, l0, l1);
-                l += l0 + l1;
-            };
-            if (kStatic) {
-                if (lone_warp) run_static(std::integral_constant<uint32_t, poly_mask(CMT_ATTN_LONE_POLY)>{});
-                else run_static(std::integral_constant<uint32_t, ST_MASK>{});
-            } else
-#endif
+            // A software-pipelined static loop over the two 32-column halves measured slower (DESIGN.md §3, round 2).
             if (lone_warp) {
-                for (int jj = 0; jj < n; ++jj) step(std::integral_constant<uint32_t, poly_mask(CMT_ATTN_LONE_POLY)>{}, jj);
+                for (int jj = 0; jj < n; ++jj) step(std::integral_constant<uint32_t, LONE_MASK>{}, jj);
             } else {
                 for (int jj = 0; jj < n; ++jj) step(std::integral_constant<uint32_t, (kStatic ? ST_MASK : DB_MASK)>{}, jj);
             }
@@ -804,16 +681,10 @@ static void attn_plan(int B, int H, int Nq, int n_tok, int sms, bool static_shif
     const int rows_last = Nq - (p->qblocks - 1) * p->qblk;
     // with every warpgroup active a step is MUFU-bound; with an idle warpgroup it is bound by one warpgroup's
     // own chain, ~3/4 of that
-#ifndef CMT_ATTN_ST_WFULL
-#define CMT_ATTN_ST_WFULL 10
-#define CMT_ATTN_ST_WLAST 7
-#endif
-#ifndef CMT_ATTN_ON_WFULL
-#define CMT_ATTN_ON_WFULL 4
-#define CMT_ATTN_ON_WLAST 3
-#endif
-    const long long w_full = static_shift ? CMT_ATTN_ST_WFULL : CMT_ATTN_ON_WFULL;
-    const long long w_last = (rows_last + 127) / 128 < attndb::NWG ? (static_shift ? CMT_ATTN_ST_WLAST : CMT_ATTN_ON_WLAST) : w_full;
+    constexpr long long ST_WFULL = 10, ST_WLAST = 7;   // static-shift kernel
+    constexpr long long ON_WFULL = 4, ON_WLAST = 3;    // online kernel
+    const long long w_full = static_shift ? ST_WFULL : ON_WFULL;
+    const long long w_last = (rows_last + 127) / 128 < attndb::NWG ? (static_shift ? ST_WLAST : ON_WLAST) : w_full;
     const long long S = static_cast<long long>(p->BH) * p->T;   // steps of one band
     const int nbf = p->qblocks - 1;                              // full bands
     long long n_full = 0, n_last = sms;

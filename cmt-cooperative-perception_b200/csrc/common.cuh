@@ -161,22 +161,10 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t by
                  "r"(bytes)
                  : "memory");
 }
-// CMT_MBAR_MODE: 0 = try_wait with a suspend-time hint, 1 = plain try_wait (default: measured 3 % faster on the
-// attention kernel than the hinted form, whose wake-up is slower), 2 = test_wait (pure spin).
-#ifndef CMT_MBAR_MODE
-#define CMT_MBAR_MODE 1
-#endif
+// Plain try_wait.  Also tried: try_wait with a suspend-time hint, 3 % slower on the attention kernel (slower wake-up),
+// and test_wait (pure spin).
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
     uint32_t ok;
-#if CMT_MBAR_MODE == 0
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity), "r"(0x989680u)  // suspend-time hint: sleep in hardware, do not re-poll
-        : "memory");
-#elif CMT_MBAR_MODE == 1
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
@@ -184,22 +172,11 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
         : "=r"(ok)
         : "r"(smem_u32(bar)), "r"(parity)
         : "memory");
-#else
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-#endif
     return ok != 0;
 }
 // A protocol bug must surface as a launch failure, never as a hung GPU: every wait is bounded
 // (try_wait itself suspends for a HW-defined interval, so the bound is tens of seconds).
-#ifndef CMT_SPIN_LIMIT
-#define CMT_SPIN_LIMIT (1u << 24)
-#endif
+constexpr uint32_t SPIN_LIMIT = 1u << 24;
 #ifdef CMT_TRAP_REPORT
 // debug builds: before trapping, record which barrier timed out into a HOST-mapped buffer (it survives the dead context):
 // cmt_dbg_host[0] = record count, then 4 words per record: blockIdx | warp << 16, barrier smem offset, parity, line.
@@ -225,7 +202,7 @@ static __device__ __noinline__ void cmt_wait_timeout(uint32_t bar_off, uint32_t 
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     uint32_t spins = 0;
     while (!mbar_try_wait(bar, parity)) {
-        if (++spins > CMT_SPIN_LIMIT) CMT_WAIT_TIMEOUT(bar, parity);
+        if (++spins > SPIN_LIMIT) CMT_WAIT_TIMEOUT(bar, parity);
     }
 }
 // Latency-tolerant waiters (producers, issuers that run a buffer ahead): let the hardware suspend the warp
@@ -242,7 +219,7 @@ __device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity) 
             : "r"(smem_u32(bar)), "r"(parity), "r"(0x989680u)
             : "memory");
         if (ok) break;
-        if (++spins > CMT_SPIN_LIMIT) CMT_WAIT_TIMEOUT(bar, parity);
+        if (++spins > SPIN_LIMIT) CMT_WAIT_TIMEOUT(bar, parity);
     }
 }
 
@@ -307,17 +284,6 @@ __device__ __forceinline__ void tc_fence_after() {
 }
 __device__ __forceinline__ void tc_wait_ld() {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-// wait::ld that also names the destination registers of the load(s) it completes: the compiler then cannot schedule a
-// consumer of those registers above the wait (the load asm alone makes them look ready at once)
-__device__ __forceinline__ void tc_wait_ld_regs(uint32_t (&v)[32]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]), "+r"(v[8]),
-                   "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15]), "+r"(v[16]),
-                   "+r"(v[17]), "+r"(v[18]), "+r"(v[19]), "+r"(v[20]), "+r"(v[21]), "+r"(v[22]), "+r"(v[23]), "+r"(v[24]),
-                   "+r"(v[25]), "+r"(v[26]), "+r"(v[27]), "+r"(v[28]), "+r"(v[29]), "+r"(v[30]), "+r"(v[31])
-                 :
-                 : "memory");
 }
 __device__ __forceinline__ void tc_wait_st() {
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");

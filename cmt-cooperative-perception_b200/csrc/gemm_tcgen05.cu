@@ -32,11 +32,8 @@ constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
 // m-tile run on neighbouring CTAs at the same time, so A comes from DRAM once and from L2 the other n_tiles - 1 times.
 constexpr int RES_KB = 4;                       // K blocks the resident B can hold (K <= 256)
 constexpr int B_RES_BYTES = RES_KB * B_BYTES;   // 128 KB
-#ifndef CMT_GEMM_RES_STAGES
-#define CMT_GEMM_RES_STAGES 5
-#endif
-constexpr int STREAM_STAGES = 4;                    // streaming mode: 4 x (A 16 KB + B 32 KB)
-constexpr int RES_STAGES = CMT_GEMM_RES_STAGES;     // B-resident mode: A-only stages of 16 KB after the 128 KB of B
+constexpr int STREAM_STAGES = 4;   // streaming mode: 4 x (A 16 KB + B 32 KB)
+constexpr int RES_STAGES = 5;      // B-resident mode: A-only stages of 16 KB after the 128 KB of B
 constexpr int MAX_STAGES = STREAM_STAGES > RES_STAGES ? STREAM_STAGES : RES_STAGES;
 constexpr int RING_BYTES = (STREAM_STAGES * STAGE_BYTES > B_RES_BYTES + RES_STAGES * A_BYTES)
                                ? STREAM_STAGES * STAGE_BYTES : B_RES_BYTES + RES_STAGES * A_BYTES;
@@ -46,9 +43,8 @@ constexpr int BIAS_CAP = 2048;
 constexpr int SMEM_BYTES = RING_BYTES + BIAS_CAP * 4 + 1024 /*align slack*/ + 256 /*barriers*/;
 static_assert(SMEM_BYTES <= 232448, "shared memory budget");
 constexpr int THREADS = 384;  // 4 control warps + 8 epilogue warps
-#ifndef CMT_GEMM_WAIT
-#define CMT_GEMM_WAIT mbar_wait_sleep   // producer / accumulator hand-over waits: sleep in hardware, leave the issue slots to the epilogue
-#endif
+// The producer and accumulator hand-over waits use mbar_wait_sleep: they sleep in hardware and leave the issue slots
+// to the epilogue.
 }  // namespace gemm
 
 constexpr int MAX_SEG = 18;
@@ -195,7 +191,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                         acol = p.seg_acol[seg] + (kb - seg * p.kb_per_seg) * BK;
                         arow += p.a_row_off + p.seg_shift[seg];
                     }
-                    CMT_GEMM_WAIT(&empty_bar[stage], phase ^ 1);
+                    mbar_wait_sleep(&empty_bar[stage], phase ^ 1);
                     if (leader) {
                         uint8_t* sa = ring + stage * ring_stride;
                         if (p.b_resident) {
@@ -226,7 +222,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                 tc_fence_after();
             }
             for (TileWalk w(p); w.valid(); w.next()) {
-                CMT_GEMM_WAIT(&tmem_empty[acc], acc_phase ^ 1);
+                mbar_wait_sleep(&tmem_empty[acc], acc_phase ^ 1);
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_base + acc * BN;
                 for (int kb = 0; kb < p.num_kb; ++kb) {
@@ -269,7 +265,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             const int tok = (y - 1) * p.conv_W + (x - 1);
             const bool ok = m < p.M && y >= 1 && y <= p.conv_H && x >= 1 && x <= p.conv_W && tok >= p.conv_tok_begin && tok < p.conv_tok_end;
             const long long orow = static_cast<long long>(z) * p.conv_frame_stride + static_cast<long long>(tok - p.conv_tok_begin) * p.N;
-            CMT_GEMM_WAIT(&tmem_full[acc], acc_phase);
+            mbar_wait_sleep(&tmem_full[acc], acc_phase);
             tc_fence_after();
             const int n_first = nt * BN + half * (BN / 2);
             const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + acc * BN + half * (BN / 2);
@@ -360,7 +356,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             long long nb = n_first / p.cb;
             long long rem = n_first - nb * p.cb;
             const long long row_off = z * p.strideC + (p.transpose_c ? static_cast<long long>(m) : static_cast<long long>(m) * p.ldc);
-            CMT_GEMM_WAIT(&tmem_full[acc], acc_phase);
+            mbar_wait_sleep(&tmem_full[acc], acc_phase);
             tc_fence_after();
             const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + acc * BN + half * (BN / 2);
             // software pipeline over the warp's four 32-column chunks: the TMEM load of chunk c + 1 is in flight while
@@ -477,7 +473,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             const int m = mt * BM + quad * 32 + lane;
             const bool m_ok = m < p.M;
             const float row_bias = (has_bias && p.bias_per_row && m_ok) ? __ldg(p.bias + m) : 0.0f;
-            CMT_GEMM_WAIT(&tmem_full[acc], acc_phase);
+            mbar_wait_sleep(&tmem_full[acc], acc_phase);
             tc_fence_after();
             const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + acc * BN;
             // column-block addressing without a 64-bit division per chunk: one division per tile, then the

@@ -4,7 +4,10 @@
 # what runs around it, so back-to-back launches of the kernel alone (tools/ab.sh) rank variants differently.
 lib=cmt-cooperative-perception_b200/libcmtcoop_b200.so
 mkdir -p gpurun_out
-cp $lib /tmp/lib_shipped.so
+shipped=$(mktemp)
+cp $lib $shipped || exit 1
+# put the shipped library back however the script ends, so that no variant is left in the tree
+trap 'cp $shipped $lib; rm -f $shipped' EXIT
 for v in "$@"; do
   cp build_variants/lib_$v.so $lib
   timeout 300 python bench.py --steps 20 --warmup 4 --no-cpu-baseline --no-parity --no-shared-conv-leg > /tmp/ab_$v.json 2> /tmp/ab_$v.err
@@ -19,4 +22,3 @@ except Exception as e:
     print(f"== {v}: FAILED {e}", open(f"/tmp/ab_{v}.err").read()[-500:])
 PY
 done
-cp /tmp/lib_shipped.so $lib
