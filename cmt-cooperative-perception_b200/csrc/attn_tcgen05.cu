@@ -578,6 +578,18 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
             } else {
                 for (int jj = 0; jj < n; ++jj) step(std::integral_constant<uint32_t, (kStatic ? ST_MASK : DB_MASK)>{}, jj);
             }
+            if (kMask) {
+                // A segment without an attended key is no partial at all: l = 0 gives o = 0 and LSE = m + log2(0) = -inf
+                // (m is finite), i.e. weight 0 in the merge.  Its padded scores still gave the clamped polynomial lanes
+                // 2^-125 each, so l > 0 on its own.
+                // The segment's mask words, addressed afresh from pos (already past the segment) and item: keeping
+                // mask_row + j0 live across the step loop made the static kernel spill more.
+                const unsigned long long* seg_bits = p.mask_bits + static_cast<long long>((item % p.BH) / p.H) * p.T +
+                                                     (pos - n - static_cast<long long>(item) * p.T);
+                unsigned long long keep = 0;
+                for (int j = lane; j < n; j += 32) keep |= __ldg(seg_bits + j);
+                if (!__any_sync(0xffffffffu, keep != 0)) l = 0.0f;
+            }
             // segment epilogue: normalised partial + log2-sum-exp into the workspace
             mbar_wait(&o_full[wg], seg & 1);
             ++seg;

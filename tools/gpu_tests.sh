@@ -12,6 +12,7 @@ run() {
 run simple tests/test_gpu_kernels.py -k "not gemm and not attention"
 run gemm tests/test_gpu_kernels.py -k "gemm"
 run attn tests/test_gpu_kernels.py -k "attention"
+run attn_edges tests/test_gpu_attention_edges.py
 run heads tests/test_gpu_heads.py
 run decoder tests/test_gpu_decoder.py
 run multi tests/test_gpu_multi.py
