@@ -9,14 +9,15 @@
 //   warp 1      MMA issuer    : one elected thread, tcgen05.mma cta_group::1 kind::f16,
 //                               M=128 x N=256 x K=16 per instruction, accumulator in TMEM
 //   warp 2      TMEM allocator (512 columns = two 128x256 fp32 accumulators, ping-pong)
-//   warps 4..11 epilogue      : tcgen05.ld 32x32b -> bias (cached in shared memory) / alpha / ReLU -> bf16|fp32 ->
-//                               256-bit global stores straight from registers (a thread owns 32 consecutive
-//                               columns of one row: 64 / 128 contiguous bytes), overlapped with the next tile's
-//                               main loop.  No shared-memory staging: the MMAs already read 96 of the 128 B/clk.
+//   warps 4..11 epilogue      : one loop for every output layout: tcgen05.ld 32x32b -> bias (cached in shared memory,
+//                               or per row) / alpha / ReLU -> bf16|fp32 -> global stores straight from registers (a
+//                               thread owns 32 consecutive columns of one row: 64 / 128 contiguous bytes), overlapped
+//                               with the next tile's main loop.  Store form (one instantiation each): 256-bit where the
+//                               layout is 32-byte aligned, masked scalar, transposed for V^T, or the shared_conv token
+//                               pair.  No shared-memory staging: the MMAs already read 96 of the 128 B/clk.
 //
 // Replaces F.linear in models/utils/attention.py:21-27,138 and the PE MLPs of
 // models/dense_heads/cmt_head.py:292-301 (reference runs them as fp32 cuBLAS SGEMMs).
-#include <cstdlib>
 #include "kernels.cuh"
 
 namespace cmt {
@@ -47,38 +48,51 @@ constexpr int THREADS = 384;  // 4 control warps + 8 epilogue warps
 // to the epilogue.
 }  // namespace gemm
 
-constexpr int MAX_SEG = 18;
+constexpr int MAX_SEG = sizeof(GemmArgs::seg_acol) / sizeof(int);
 
+// The caller's arguments and what the host derives from them.
 struct TcGemmParams {
-    const float* bias;
-    void* C;
-    int M, N, K;
-    long long ldc, cb, cb_stride, strideC;
-    float alpha;
-    int relu, bias_per_row, out_bf16;
+    GemmArgs g;        // b_batch_div normalised to >= 1
     int a_batched, b_batched;
     int m_tiles, n_tiles, total_tiles, num_kb;
-    int direct;     // 1: lean epilogue, 256-bit stores straight from registers (alignment / bias conditions hold)
-    float* norm2_max; // [batch][N/32]: atomicMax of the squared norm of every row's 32-column block (attention score bound), or nullptr
-    int transpose_c; // 1: element (m, n) of batch z is stored at z*strideC + (n / cb)*cb_stride + (n % cb)*ldc + m (bf16)
-    int b_resident; // 1: gridDim.x = Gm * n_tiles, CTA c owns n-tile c % n_tiles and the (batch, m-tile) pairs c / n_tiles + i * Gm
-    // Segmented K (implicit convolutions and split-precision products): K block kb belongs to segment s = kb / kb_per_seg;
-    // its A tile is read at column seg_acol[s] + (kb % kb_per_seg) * BK and at row m0 + a_row_off + seg_shift[s] of the
-    // batch's A matrix (rows outside it are zero-filled by the TMA unit), while B is read at column kb * BK as usual.
-    // n_seg == 0: ordinary GEMM.
-    int n_seg, kb_per_seg, a_row_off;
-    int seg_acol[MAX_SEG], seg_shift[MAX_SEG];
-    int b_batch_div;   // batch z reads B of batch z / b_batch_div (task heads: one weight set per decoder layer, B frames each)
-    // Token epilogue of the 3x3 shared_conv (conv_xv != nullptr): output row m is position (y, x) = (m / conv_Wp, m % conv_Wp)
-    // of the zero-padded map of frame z; interior positions become token t = (y - 1) * conv_W + (x - 1) and are stored as
-    // xv[z][t - tok_begin] = bf16(v), xk[z][t - tok_begin] = bf16(v + pos[t]) (v = ReLU(acc + bias)); border rows are dropped.
-    void* conv_xk;
-    void* conv_xv;
-    const float* conv_pos;
-    int conv_W, conv_H, conv_Wp, conv_tok_begin, conv_tok_end;
-    long long conv_frame_stride;   // elements between frames in xk / xv
-    int mt_off;                    // first m-tile (conv with a token sub-range computes only the rows that hold its tokens)
+    int kb_per_seg;    // segmented K: K block kb belongs to segment kb / kb_per_seg (B is read at column kb * BK as usual)
+    int mt_off;        // first m-tile (conv with a token sub-range computes only the rows that hold its tokens)
+    int b_resident;    // 1: gridDim.x = Gm * n_tiles, CTA c owns n-tile c % n_tiles and the (batch, m-tile) pairs c / n_tiles + i * Gm
+    int vec_store;     // 1: C, ldc, cb_stride and strideC put every full 32-column chunk of a row on a 32-byte boundary
 };
+
+// How the epilogue stores a chunk.  The host picks one instantiation of the kernel per launch, so the hot layouts run
+// a loop body with no tests for the forms they do not use.
+enum class Store {
+    Vec,          // row-major, 32-byte aligned layout, N % 32 == 0, no column bias too wide for the cache: 256-bit stores
+    Masked,       // row-major otherwise: 256-bit stores for the full chunks of an aligned layout, masked scalar stores else;
+                  // the only form that reads a column bias too wide for the cache
+    Transposed,   // C^T inside each column block (V^T), bf16
+    Conv,         // shared_conv token pair xv / xk
+};
+
+// 32 consecutive outputs of one row as 256-bit stores (dst 32-byte aligned): bf16, 64 bytes / fp32, 128 bytes
+__device__ __forceinline__ void st_bf16x32(uint8_t* dst, const float (&f)[32]) {
+#pragma unroll
+    for (int i = 0; i < 2; ++i)
+        asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst + 32 * i),
+                     "r"(pack_bf16x2(f[16 * i + 0], f[16 * i + 1])), "r"(pack_bf16x2(f[16 * i + 2], f[16 * i + 3])),
+                     "r"(pack_bf16x2(f[16 * i + 4], f[16 * i + 5])), "r"(pack_bf16x2(f[16 * i + 6], f[16 * i + 7])),
+                     "r"(pack_bf16x2(f[16 * i + 8], f[16 * i + 9])), "r"(pack_bf16x2(f[16 * i + 10], f[16 * i + 11])),
+                     "r"(pack_bf16x2(f[16 * i + 12], f[16 * i + 13])), "r"(pack_bf16x2(f[16 * i + 14], f[16 * i + 15]))
+                     : "memory");
+}
+
+__device__ __forceinline__ void st_f32x32(uint8_t* dst, const float (&f)[32]) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst + 32 * i),
+                     "r"(__float_as_uint(f[8 * i + 0])), "r"(__float_as_uint(f[8 * i + 1])),
+                     "r"(__float_as_uint(f[8 * i + 2])), "r"(__float_as_uint(f[8 * i + 3])),
+                     "r"(__float_as_uint(f[8 * i + 4])), "r"(__float_as_uint(f[8 * i + 5])),
+                     "r"(__float_as_uint(f[8 * i + 6])), "r"(__float_as_uint(f[8 * i + 7]))
+                     : "memory");
+}
 
 // The three roles walk the same tile sequence.
 struct TileWalk {
@@ -114,10 +128,12 @@ struct TileWalk {
     }
 };
 
+template <Store S>
 __global__ void __launch_bounds__(gemm::THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                const TcGemmParams p) {
     using namespace gemm;
+    const GemmArgs& g = p.g;
     pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -157,12 +173,12 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
         fence_barrier_init();
     }
     if (warp == 2) tmem_alloc(tmem_slot, 512);
-    const bool bias_cached = p.bias != nullptr && !p.bias_per_row && p.N <= BIAS_CAP - 64;
+    const bool bias_cached = g.bias != nullptr && !g.bias_per_row && g.N <= BIAS_CAP - 64;
     pdl_wait();   // everything above (barriers, TMEM, descriptor prefetch) overlapped the predecessor
     // the bias may have been produced on the stream by a predecessor (C-ABI callers, rebuilt weight caches): read it
     // only after the dependency wait (plain loads: __ldg's non-coherent path could serve a stale line)
     if (bias_cached)
-        for (int i = threadIdx.x; i < BIAS_CAP; i += THREADS) bias_s[i] = i < p.N ? p.bias[i] : 0.0f;
+        for (int i = threadIdx.x; i < BIAS_CAP; i += THREADS) bias_s[i] = i < g.N ? g.bias[i] : 0.0f;
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -183,13 +199,13 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             for (; w.valid(); w.next()) {
                 int z, mt, nt;
                 w.decode(p, z, mt, nt);
-                const int zb = p.b_batched ? z / p.b_batch_div : 0;
+                const int zb = p.b_batched ? z / g.b_batch_div : 0;
                 for (int kb = 0; kb < p.num_kb; ++kb) {
                     int acol = kb * BK, arow = mt * BM;
-                    if (p.n_seg > 0) {
+                    if (g.n_seg > 0) {
                         const int seg = kb / p.kb_per_seg;
-                        acol = p.seg_acol[seg] + (kb - seg * p.kb_per_seg) * BK;
-                        arow += p.a_row_off + p.seg_shift[seg];
+                        acol = g.seg_acol[seg] + (kb - seg * p.kb_per_seg) * BK;
+                        arow += g.a_row_off + g.seg_shift[seg];
                     }
                     mbar_wait_sleep(&empty_bar[stage], phase ^ 1);
                     if (leader) {
@@ -247,101 +263,28 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
         }
-    } else if (warp >= 4 && p.conv_xv != nullptr) {
-        // ------------------- epilogue of the 3x3 shared_conv: ReLU(acc + bias) -> token-major bf16 xv, xk = xv + pos -------------------
-        // (cmt_head.py:280-287,481 + cmt_transformer.py:105-110 + petr_transformer.py:296-299 for the BEV tokens: the NCHW
-        // fp32 map the reference writes and re-reads never exists.)  A thread owns one padded position and 32 consecutive
-        // channels per chunk: 64 contiguous bytes of each output row, 128 contiguous bytes of the position encoding.
-        const int quad = warp & 3;
-        const int half = (warp - 4) >> 2;
-        const uint32_t bias_addr = smem_u32(bias_s);
-        int acc = 0;
-        uint32_t acc_phase = 0;
-        for (TileWalk w(p); w.valid(); w.next()) {
-            int z, mt, nt;
-            w.decode(p, z, mt, nt);
-            const int m = mt * BM + quad * 32 + lane;
-            const int y = m / p.conv_Wp, x = m - y * p.conv_Wp;
-            const int tok = (y - 1) * p.conv_W + (x - 1);
-            const bool ok = m < p.M && y >= 1 && y <= p.conv_H && x >= 1 && x <= p.conv_W && tok >= p.conv_tok_begin && tok < p.conv_tok_end;
-            const long long orow = static_cast<long long>(z) * p.conv_frame_stride + static_cast<long long>(tok - p.conv_tok_begin) * p.N;
-            mbar_wait_sleep(&tmem_full[acc], acc_phase);
-            tc_fence_after();
-            const int n_first = nt * BN + half * (BN / 2);
-            const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + acc * BN + half * (BN / 2);
-            const int n_chunks = min(4, (p.N - n_first + 31) >> 5);
-            uint32_t v[2][32];
-            if (n_chunks > 0) {
-                tmem_ld32(t_row, v[0]);
-                tc_wait_ld();
-            }
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                if (c >= n_chunks) break;
-                if (c + 1 < n_chunks) tmem_ld32(t_row + (c + 1) * 32, v[(c + 1) & 1]);
-                const int n0 = n_first + c * 32;
-                if (ok) {
-                    const uint32_t (&vc)[32] = v[c & 1];
-                    float f[32];
-                    const uint32_t baddr = bias_addr + n0 * 4;
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        float4 b;
-                        asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w) : "r"(baddr + i * 16));
-                        f[4 * i] = fmaxf(b.x + __uint_as_float(vc[4 * i]), 0.0f);
-                        f[4 * i + 1] = fmaxf(b.y + __uint_as_float(vc[4 * i + 1]), 0.0f);
-                        f[4 * i + 2] = fmaxf(b.z + __uint_as_float(vc[4 * i + 2]), 0.0f);
-                        f[4 * i + 3] = fmaxf(b.w + __uint_as_float(vc[4 * i + 3]), 0.0f);
-                    }
-                    uint8_t* dv = reinterpret_cast<uint8_t*>(p.conv_xv) + (orow + n0) * 2;
-                    uint8_t* dk = reinterpret_cast<uint8_t*>(p.conv_xk) + (orow + n0) * 2;
-                    const float4* pp = reinterpret_cast<const float4*>(p.conv_pos + static_cast<long long>(tok) * p.N + n0);
-#pragma unroll
-                    for (int i = 0; i < 2; ++i) {
-                        asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dv + 32 * i),
-                                     "r"(pack_bf16x2(f[16 * i + 0], f[16 * i + 1])), "r"(pack_bf16x2(f[16 * i + 2], f[16 * i + 3])),
-                                     "r"(pack_bf16x2(f[16 * i + 4], f[16 * i + 5])), "r"(pack_bf16x2(f[16 * i + 6], f[16 * i + 7])),
-                                     "r"(pack_bf16x2(f[16 * i + 8], f[16 * i + 9])), "r"(pack_bf16x2(f[16 * i + 10], f[16 * i + 11])),
-                                     "r"(pack_bf16x2(f[16 * i + 12], f[16 * i + 13])), "r"(pack_bf16x2(f[16 * i + 14], f[16 * i + 15]))
-                                     : "memory");
-                    }
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const float4 q = __ldg(pp + i);
-                        f[4 * i] += q.x; f[4 * i + 1] += q.y; f[4 * i + 2] += q.z; f[4 * i + 3] += q.w;
-                    }
-#pragma unroll
-                    for (int i = 0; i < 2; ++i) {
-                        asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dk + 32 * i),
-                                     "r"(pack_bf16x2(f[16 * i + 0], f[16 * i + 1])), "r"(pack_bf16x2(f[16 * i + 2], f[16 * i + 3])),
-                                     "r"(pack_bf16x2(f[16 * i + 4], f[16 * i + 5])), "r"(pack_bf16x2(f[16 * i + 6], f[16 * i + 7])),
-                                     "r"(pack_bf16x2(f[16 * i + 8], f[16 * i + 9])), "r"(pack_bf16x2(f[16 * i + 10], f[16 * i + 11])),
-                                     "r"(pack_bf16x2(f[16 * i + 12], f[16 * i + 13])), "r"(pack_bf16x2(f[16 * i + 14], f[16 * i + 15]))
-                                     : "memory");
-                    }
-                }
-                if (c + 1 < n_chunks) tc_wait_ld();
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tmem_empty[acc]);
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-    } else if (warp >= 4 && p.direct) {
-        // ------------------- epilogue, lean path: registers -> 256-bit global stores -------------------
+    } else if (warp >= 4) {
+        // ---------------------- epilogue: TMEM -> bias / alpha / ReLU -> global, straight from registers ----------------------
         // ncu on the K projection: l1tex (shared-memory) throughput 78 %, tensor pipe 42 %.  With cta_group::1 the MMAs
         // alone read 96 B/clk of operands out of the 128 B/clk shared memory (A 4 KB + B 8 KB per 128-cycle
         // instruction), so an epilogue that stages the tile in shared memory for a TMA store (64 KB written +
-        // 64 KB read per tile) competes for the kernel's scarcest resource.  A thread owns one output row and 32
-        // consecutive columns of it, i.e. 64 contiguous bytes of bf16 (128 of fp32) in EVERY layout this kernel
-        // writes: two (four) st.global.v8.b32 per chunk are full-sector writes with no staging at all.
+        // 64 KB read per tile) competes for the kernel's scarcest resource.  Warp w reads TMEM lane quadrant (w & 3) and
+        // column half ((w - 4) >> 2), so every scheduler has two epilogue warps.  A thread owns one output row and 32
+        // consecutive columns of it per chunk, i.e. 64 contiguous bytes of bf16 (128 of fp32): where the host found the
+        // layout 32-byte aligned, two (four) st.global.v8.b32 per chunk are full-sector writes with no staging at all;
+        // other layouts and the ragged last chunk take masked scalar stores.
         // Transposed output (V^T: element (m, n) at (n % cb) * ldc + m): a warp instruction writes the 32 rows of
         // one column, 64 contiguous bytes.
+        // shared_conv tokens (cmt_head.py:280-287,481 + cmt_transformer.py:105-110 + petr_transformer.py:296-299 for the
+        // BEV tokens: the NCHW fp32 map the reference writes and re-reads never exists): the thread's row is a padded
+        // position, stored as xv = bf16(ReLU(acc + bias)) and xk = bf16(that + pos), 64 contiguous bytes each.
         const int quad = warp & 3;
         const int half = (warp - 4) >> 2;
-        const bool scale = p.alpha != 1.0f;
-        const bool relu = p.relu != 0;
-        const int esz = p.out_bf16 ? 2 : 4;
+        constexpr bool conv = S == Store::Conv;   // ReLU(acc + bias) with the bias cached (host checks), no alpha
+        const bool col_bias = g.bias != nullptr && !g.bias_per_row;   // from bias_s when bias_cached, else from global
+        const bool scale = !conv && g.alpha != 1.0f;
+        const bool relu = conv || g.relu != 0;
+        const int esz = g.out_bf16 ? 2 : 4;
         const uint32_t bias_addr = smem_u32(bias_s);
         int acc = 0;
         uint32_t acc_phase = 0;
@@ -349,20 +292,29 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             int z, mt, nt;
             w.decode(p, z, mt, nt);
             const int m = mt * BM + quad * 32 + lane;
-            const bool m_ok = m < p.M;
-            const float row_bias = (p.bias != nullptr && p.bias_per_row && m_ok) ? __ldg(p.bias + m) : 0.0f;
+            bool row_ok = m < g.M;
+            long long row_off;   // element offset of the thread's row
+            int tok = 0;
+            if constexpr (conv) {
+                const int y = m / g.conv_Wp, x = m - y * g.conv_Wp;
+                tok = (y - 1) * g.conv_W + (x - 1);
+                row_ok = row_ok && y >= 1 && y <= g.conv_H && x >= 1 && x <= g.conv_W && tok >= g.conv_tok_begin && tok < g.conv_tok_end;
+                row_off = static_cast<long long>(z) * g.conv_frame_stride + static_cast<long long>(tok - g.conv_tok_begin) * g.N;
+            } else {
+                row_off = z * g.strideC + (S == Store::Transposed ? static_cast<long long>(m) : static_cast<long long>(m) * g.ldc);
+            }
+            const float row_bias = (g.bias != nullptr && g.bias_per_row && row_ok) ? __ldg(g.bias + m) : 0.0f;
             // column block of the warp's first chunk: one division per tile, then +32 columns per chunk
             const int n_first = nt * BN + half * (BN / 2);
-            long long nb = n_first / p.cb;
-            long long rem = n_first - nb * p.cb;
-            const long long row_off = z * p.strideC + (p.transpose_c ? static_cast<long long>(m) : static_cast<long long>(m) * p.ldc);
+            long long nb = n_first / g.cb;
+            long long rem = n_first - nb * g.cb;
             mbar_wait_sleep(&tmem_full[acc], acc_phase);
             tc_fence_after();
             const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + acc * BN + half * (BN / 2);
             // software pipeline over the warp's four 32-column chunks: the TMEM load of chunk c + 1 is in flight while
             // chunk c is biased / packed / stored (tcgen05.wait::ld waits for every outstanding load, so the wait
             // comes after the work on the current chunk)
-            const int n_chunks = min(4, (p.N - n_first + 31) >> 5);   // warp-uniform; <= 0: nothing to do
+            const int n_chunks = min(4, (g.N - n_first + 31) >> 5);   // warp-uniform; <= 0: nothing to do
             uint32_t v[2][32];
             if (n_chunks > 0) {
                 tmem_ld32(t_row, v[0]);
@@ -376,7 +328,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                 {
                     float f[32];
                     const uint32_t (&vc)[32] = v[c & 1];
-                    if (bias_cached) {
+                    if (conv || bias_cached) {
                         const uint32_t baddr = bias_addr + n0 * 4;
 #pragma unroll
                         for (int i = 0; i < 8; ++i) {
@@ -387,191 +339,71 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                             f[4 * i + 2] = b.z + __uint_as_float(vc[4 * i + 2]);
                             f[4 * i + 3] = b.w + __uint_as_float(vc[4 * i + 3]);
                         }
+                    } else if (S == Store::Masked && col_bias) {
+                        // wider than the cache (N > BIAS_CAP - 64)
+#pragma unroll
+                        for (int i = 0; i < 32; ++i) f[i] = (n0 + i < g.N ? __ldg(g.bias + n0 + i) : 0.0f) + __uint_as_float(vc[i]);
                     } else {
 #pragma unroll
                         for (int i = 0; i < 32; ++i) f[i] = row_bias + __uint_as_float(vc[i]);
                     }
                     if (scale) {
 #pragma unroll
-                        for (int i = 0; i < 32; ++i) f[i] *= p.alpha;
+                        for (int i = 0; i < 32; ++i) f[i] *= g.alpha;
                     }
                     if (relu) {
 #pragma unroll
                         for (int i = 0; i < 32; ++i) f[i] = fmaxf(f[i], 0.0f);
                     }
-                    if (p.norm2_max != nullptr) {
+                    if (!conv && g.norm2_max != nullptr) {
                         // max over the tile's rows of |row block|^2 (non-negative floats order like their bit patterns)
                         float n2 = 0.0f;
 #pragma unroll
                         for (int i = 0; i < 32; ++i) n2 = fmaf(f[i], f[i], n2);
-                        const unsigned int wmax = __reduce_max_sync(0xffffffffu, m_ok ? __float_as_uint(n2) : 0u);
+                        const unsigned int wmax = __reduce_max_sync(0xffffffffu, row_ok ? __float_as_uint(n2) : 0u);
                         if (lane == 0)
-                            atomicMax(reinterpret_cast<unsigned int*>(p.norm2_max) + static_cast<long long>(z) * (p.N >> 5) + (n0 >> 5), wmax);
+                            atomicMax(reinterpret_cast<unsigned int*>(g.norm2_max) + static_cast<long long>(z) * (g.N >> 5) + (n0 >> 5), wmax);
                     }
-                    const long long blk_off = nb * p.cb_stride;
-                    if (p.transpose_c) {
-                        // element (m, n) -> blk_off + (n % cb) * ldc + m  (bf16 only)
-                        uint16_t* dst = reinterpret_cast<uint16_t*>(p.C) + row_off + blk_off + rem * p.ldc;
-                        if (m_ok) {
+                    const long long blk_off = row_off + nb * g.cb_stride;
+                    if (row_ok) {
+                        if constexpr (conv) {
+                            st_bf16x32(reinterpret_cast<uint8_t*>(g.conv_xv) + (row_off + n0) * 2, f);
+                            const float4* pp = reinterpret_cast<const float4*>(g.conv_pos + static_cast<long long>(tok) * g.N + n0);
+#pragma unroll
+                            for (int i = 0; i < 8; ++i) {
+                                const float4 q = __ldg(pp + i);
+                                f[4 * i] += q.x; f[4 * i + 1] += q.y; f[4 * i + 2] += q.z; f[4 * i + 3] += q.w;
+                            }
+                            st_bf16x32(reinterpret_cast<uint8_t*>(g.conv_xk) + (row_off + n0) * 2, f);
+                        } else if constexpr (S == Store::Transposed) {
+                            // element (m, n) -> blk_off + (n % cb) * ldc + m  (bf16 only)
+                            uint16_t* dst = reinterpret_cast<uint16_t*>(g.C) + blk_off + rem * g.ldc;
 #pragma unroll
                             for (int i = 0; i < 16; ++i) {
                                 const uint32_t w2 = pack_bf16x2(f[2 * i], f[2 * i + 1]);
-                                dst[static_cast<long long>(2 * i) * p.ldc] = static_cast<uint16_t>(w2 & 0xffffu);
-                                dst[static_cast<long long>(2 * i + 1) * p.ldc] = static_cast<uint16_t>(w2 >> 16);
+                                dst[static_cast<long long>(2 * i) * g.ldc] = static_cast<uint16_t>(w2 & 0xffffu);
+                                dst[static_cast<long long>(2 * i + 1) * g.ldc] = static_cast<uint16_t>(w2 >> 16);
                             }
-                        }
-                    } else if (p.out_bf16) {
-                        uint8_t* dst = reinterpret_cast<uint8_t*>(p.C) + (row_off + blk_off + rem) * esz;
-                        if (m_ok) {
+                        } else if (S == Store::Vec || (p.vec_store && n0 + 32 <= g.N)) {
+                            uint8_t* dst = reinterpret_cast<uint8_t*>(g.C) + (blk_off + rem) * esz;
+                            if (g.out_bf16) st_bf16x32(dst, f);
+                            else st_f32x32(dst, f);
+                        } else if (g.out_bf16) {
+                            __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(g.C) + blk_off + rem;
 #pragma unroll
-                            for (int i = 0; i < 2; ++i)
-                                asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst + 32 * i),
-                                             "r"(pack_bf16x2(f[16 * i + 0], f[16 * i + 1])), "r"(pack_bf16x2(f[16 * i + 2], f[16 * i + 3])),
-                                             "r"(pack_bf16x2(f[16 * i + 4], f[16 * i + 5])), "r"(pack_bf16x2(f[16 * i + 6], f[16 * i + 7])),
-                                             "r"(pack_bf16x2(f[16 * i + 8], f[16 * i + 9])), "r"(pack_bf16x2(f[16 * i + 10], f[16 * i + 11])),
-                                             "r"(pack_bf16x2(f[16 * i + 12], f[16 * i + 13])), "r"(pack_bf16x2(f[16 * i + 14], f[16 * i + 15]))
-                                             : "memory");
-                        }
-                    } else {
-                        uint8_t* dst = reinterpret_cast<uint8_t*>(p.C) + (row_off + blk_off + rem) * esz;
-                        if (m_ok) {
+                            for (int i = 0; i < 32; ++i)
+                                if (n0 + i < g.N) dst[i] = __float2bfloat16_rn(f[i]);
+                        } else {
+                            float* dst = reinterpret_cast<float*>(g.C) + blk_off + rem;
 #pragma unroll
-                            for (int i = 0; i < 4; ++i)
-                                asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst + 32 * i),
-                                             "r"(__float_as_uint(f[8 * i + 0])), "r"(__float_as_uint(f[8 * i + 1])),
-                                             "r"(__float_as_uint(f[8 * i + 2])), "r"(__float_as_uint(f[8 * i + 3])),
-                                             "r"(__float_as_uint(f[8 * i + 4])), "r"(__float_as_uint(f[8 * i + 5])),
-                                             "r"(__float_as_uint(f[8 * i + 6])), "r"(__float_as_uint(f[8 * i + 7]))
-                                             : "memory");
+                            for (int i = 0; i < 32; ++i)
+                                if (n0 + i < g.N) dst[i] = f[i];
                         }
                     }
                     rem += 32;
-                    if (rem >= p.cb) { rem -= p.cb; ++nb; }
+                    if (rem >= g.cb) { rem -= g.cb; ++nb; }
                 }
                 if (c + 1 < n_chunks) tc_wait_ld();
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tmem_empty[acc]);
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-    } else if (warp >= 4) {
-        // ------------------------------- epilogue -------------------------------
-        // 8 warps: warp w reads TMEM lane quadrant (w & 3) and column half ((w - 4) >> 2), so every
-        // scheduler has two epilogue warps to overlap TMEM / global latencies.  All option tests
-        // (bias kind, alpha, relu, dtype) are hoisted out of the per-element loops.
-        const int quad = warp & 3;
-        const int half = (warp - 4) >> 2;
-        const bool has_bias = p.bias != nullptr;
-        const bool col_bias = has_bias && !p.bias_per_row;
-        const bool scale = p.alpha != 1.0f;
-        int acc = 0;
-        uint32_t acc_phase = 0;
-        for (TileWalk w(p); w.valid(); w.next()) {
-            int z, mt, nt;
-            w.decode(p, z, mt, nt);
-            const int m = mt * BM + quad * 32 + lane;
-            const bool m_ok = m < p.M;
-            const float row_bias = (has_bias && p.bias_per_row && m_ok) ? __ldg(p.bias + m) : 0.0f;
-            mbar_wait_sleep(&tmem_full[acc], acc_phase);
-            tc_fence_after();
-            const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + acc * BN;
-            // column-block addressing without a 64-bit division per chunk: one division per tile, then the
-            // (block, offset-in-block) pair advances by 32 columns per chunk
-            const int c_first = half * (BN / 64);
-            const long long n_first = static_cast<long long>(nt) * BN + c_first * 32;
-            long long blk = n_first / p.cb;
-            long long rem = n_first - blk * p.cb;
-            const long long row_off = z * p.strideC + static_cast<long long>(m) * p.ldc;
-            // bias for one 32-column chunk (independent of the accumulator: issued before the TMEM wait)
-            auto load_bias = [&](int n0, float (&f)[32]) {
-                if (bias_cached) {
-                    // n0 + 32 may pass N in the last tile: the extra values only reach columns the store clips
-                    const float4* b4 = reinterpret_cast<const float4*>(bias_s + n0);
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const float4 b = (n0 + 4 * i + 4 <= BIAS_CAP) ? b4[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-                        f[4 * i] = b.x; f[4 * i + 1] = b.y; f[4 * i + 2] = b.z; f[4 * i + 3] = b.w;
-                    }
-                } else if (col_bias) {
-                    if (n0 + 32 <= p.N) {
-                        const float4* b4 = reinterpret_cast<const float4*>(p.bias + n0);  // n0 % 32 == 0
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            const float4 b = __ldg(b4 + i);
-                            f[4 * i] = b.x; f[4 * i + 1] = b.y; f[4 * i + 2] = b.z; f[4 * i + 3] = b.w;
-                        }
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < 32; ++i) f[i] = (n0 + i < p.N) ? __ldg(p.bias + n0 + i) : 0.0f;
-                    }
-                } else {
-#pragma unroll
-                    for (int i = 0; i < 32; ++i) f[i] = row_bias;
-                }
-            };
-            auto finish = [&](int n0, long long off, const uint32_t (&v)[32], float (&f)[32]) {
-                const bool full = (n0 + 32 <= p.N);
-#pragma unroll
-                for (int i = 0; i < 32; ++i) f[i] += __uint_as_float(v[i]);
-                if (scale) {
-#pragma unroll
-                    for (int i = 0; i < 32; ++i) f[i] *= p.alpha;
-                }
-                if (p.relu) {
-#pragma unroll
-                    for (int i = 0; i < 32; ++i) f[i] = fmaxf(f[i], 0.0f);
-                }
-                if (!m_ok) return;
-                if (p.out_bf16) {
-                    __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(p.C) + off;
-                    if (full && ((reinterpret_cast<uintptr_t>(dst) & 15) == 0)) {
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            uint4 w;
-                            w.x = pack_bf16x2(f[8 * i + 0], f[8 * i + 1]);
-                            w.y = pack_bf16x2(f[8 * i + 2], f[8 * i + 3]);
-                            w.z = pack_bf16x2(f[8 * i + 4], f[8 * i + 5]);
-                            w.w = pack_bf16x2(f[8 * i + 6], f[8 * i + 7]);
-                            reinterpret_cast<uint4*>(dst)[i] = w;
-                        }
-                    } else {
-                        for (int i = 0; i < 32; ++i)
-                            if (n0 + i < p.N) dst[i] = __float2bfloat16_rn(f[i]);
-                    }
-                } else {
-                    float* dst = reinterpret_cast<float*>(p.C) + off;
-                    if (full && ((reinterpret_cast<uintptr_t>(dst) & 15) == 0)) {
-#pragma unroll
-                        for (int i = 0; i < 8; ++i)
-                            reinterpret_cast<float4*>(dst)[i] = make_float4(f[4 * i], f[4 * i + 1], f[4 * i + 2], f[4 * i + 3]);
-                    } else {
-                        for (int i = 0; i < 32; ++i)
-                            if (n0 + i < p.N) dst[i] = f[i];
-                    }
-                }
-            };
-            // two 32-column chunks per round: both TMEM loads and both bias fetches are in flight together
-#pragma unroll 1
-            for (int c = c_first; c < c_first + BN / 64; c += 2) {
-                const int n0a = nt * BN + c * 32, n0b = n0a + 32;
-                if (n0a >= p.N) break;  // warp-uniform
-                const bool has_b = n0b < p.N;
-                const long long offa = row_off + blk * p.cb_stride + rem;
-                rem += 32;
-                if (rem >= p.cb) { rem -= p.cb; ++blk; }
-                const long long offb = row_off + blk * p.cb_stride + rem;
-                rem += 32;
-                if (rem >= p.cb) { rem -= p.cb; ++blk; }
-                uint32_t va[32], vb[32];
-                float fa[32], fb[32];
-                tmem_ld32(t_row + c * 32, va);
-                if (has_b) tmem_ld32(t_row + (c + 1) * 32, vb);
-                load_bias(n0a, fa);
-                if (has_b) load_bias(n0b, fb);
-                tc_wait_ld();
-                finish(n0a, offa, va, fa);
-                if (has_b) finish(n0b, offb, vb, fb);
             }
             tc_fence_before();
             __syncwarp();
@@ -602,15 +434,20 @@ int launch_tc_gemm(const GemmArgs& g, int batch, cudaStream_t stream) {
                   "cmt_gemm_bias_act(bf16): column block must be >= N or a multiple of 32");
     CMT_CHECK_ARG(g.strideA % 8 == 0 && g.strideB % 8 == 0, "cmt_gemm_bias_act(bf16): batch strides must be multiples of 8");
 
+    // one instantiation per store form, in the order of Store
+    static void (*const kernels[])(CUtensorMap, CUtensorMap, TcGemmParams) = {
+        tc_gemm_kernel<Store::Vec>, tc_gemm_kernel<Store::Masked>, tc_gemm_kernel<Store::Transposed>, tc_gemm_kernel<Store::Conv>};
     static DeviceOnce attr_once;
     int attr_dev;
     if (attr_once.need(&attr_dev)) {
-        cudaError_t e = cudaFuncSetAttribute(tc_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             SMEM_BYTES);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(tc_gemm)");
+        for (auto kernel : kernels) {
+            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+            if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(tc_gemm)");
+        }
         attr_once.mark(attr_dev);
     }
 
+    const int b_div = g.b_batch_div > 1 ? g.b_batch_div : 1;
     CUtensorMap ta, tb;
     {
         const bool batched = g.strideA != 0 && batch > 1;
@@ -625,7 +462,6 @@ int launch_tc_gemm(const GemmArgs& g, int batch, cudaStream_t stream) {
     }
     {
         const bool batched = g.strideB != 0 && batch > 1;
-        const int b_div = g.b_batch_div > 1 ? g.b_batch_div : 1;
         uint64_t dims[3] = {static_cast<uint64_t>(g.K), static_cast<uint64_t>(g.N),
                             static_cast<uint64_t>(batched ? (batch + b_div - 1) / b_div : 1)};
         uint64_t strides[2] = {static_cast<uint64_t>(g.ldb) * 2,
@@ -637,59 +473,31 @@ int launch_tc_gemm(const GemmArgs& g, int batch, cudaStream_t stream) {
 
     const int esz = g.out_bf16 ? 2 : 4;
     const bool plain = g.cb >= g.N;
-
-    TcGemmParams p{};
-    p.transpose_c = g.transpose_c;
-    p.norm2_max = g.norm2_max;
-    p.n_seg = g.n_seg;
-    p.kb_per_seg = g.n_seg > 0 ? g.seg_k / BK : 0;
-    p.a_row_off = g.a_row_off;
-    for (int i = 0; i < g.n_seg; ++i) {
-        p.seg_acol[i] = g.seg_acol[i];
-        p.seg_shift[i] = g.seg_shift[i];
-    }
-    p.b_batch_div = g.b_batch_div > 1 ? g.b_batch_div : 1;
-    p.conv_xk = g.conv_xk;
-    p.conv_xv = g.conv_xv;
-    p.conv_pos = g.conv_pos;
-    p.conv_W = g.conv_W;
-    p.conv_H = g.conv_H;
-    p.conv_Wp = g.conv_Wp;
-    p.conv_tok_begin = g.conv_tok_begin;
-    p.conv_tok_end = g.conv_tok_end;
-    p.conv_frame_stride = g.conv_frame_stride;
     if (g.conv_xv != nullptr)
         CMT_CHECK_ARG(g.conv_xk && g.conv_pos && g.bias && !g.bias_per_row && g.N % 32 == 0 && g.N <= BIAS_CAP - 64 &&
                           (reinterpret_cast<uintptr_t>(g.conv_xk) & 31) == 0 && (reinterpret_cast<uintptr_t>(g.conv_xv) & 31) == 0 &&
                           (reinterpret_cast<uintptr_t>(g.conv_pos) & 15) == 0 && g.conv_frame_stride % 16 == 0,
                       "cmt_shared_conv_tokens: bias, pos, 32-byte aligned outputs and N %% 32 == 0 required");
-    static const bool no_direct = getenv("CMT_GEMM_NO_DIRECT") != nullptr;
     const bool bias_ok = g.bias == nullptr || g.bias_per_row || g.N <= BIAS_CAP - 64;
-    if (g.transpose_c) {
+    if (g.transpose_c)
         CMT_CHECK_ARG(g.out_bf16 && g.cb % 32 == 0 && g.N % 32 == 0 && bias_ok && !plain,
                       "cmt_gemm_bias_act(bf16): transposed output needs bf16, cb %% 32 == 0, N %% 32 == 0, N <= %d", BIAS_CAP - 64);
-        p.direct = 1;
-    } else {
-        const bool aligned = (reinterpret_cast<uintptr_t>(g.C) & 31) == 0 && (g.ldc * esz) % 32 == 0 &&
-                             (plain || ((g.cb_stride * esz) % 32 == 0 && g.cb % 32 == 0)) &&
-                             (batch == 1 || (g.strideC * esz) % 32 == 0);
-        p.direct = (aligned && g.N % 32 == 0 && bias_ok && !no_direct) ? 1 : 0;
-    }
-    CMT_CHECK_ARG(g.norm2_max == nullptr || p.direct, "cmt_gemm_bias_act(bf16): norm2_max needs N %% 32 == 0, 32-byte aligned C rows "
-                                                      "and N <= %d with a column bias", BIAS_CAP - 64);
-    p.bias = g.bias;
-    p.C = g.C;
-    p.M = g.M;
-    p.N = g.N;
-    p.K = g.K;
-    p.ldc = g.ldc;
-    p.cb = g.cb;
-    p.cb_stride = g.cb_stride;
-    p.strideC = g.strideC;
-    p.alpha = g.alpha;
-    p.relu = g.relu;
-    p.bias_per_row = g.bias_per_row;
-    p.out_bf16 = g.out_bf16;
+    const bool aligned = (reinterpret_cast<uintptr_t>(g.C) & 31) == 0 && (g.ldc * esz) % 32 == 0 &&
+                         (plain || ((g.cb_stride * esz) % 32 == 0 && g.cb % 32 == 0)) &&
+                         (batch == 1 || (g.strideC * esz) % 32 == 0);
+    CMT_CHECK_ARG(g.norm2_max == nullptr || g.transpose_c || (aligned && g.N % 32 == 0 && bias_ok),
+                  "cmt_gemm_bias_act(bf16): norm2_max needs N %% 32 == 0, 32-byte aligned C rows and N <= %d with a column bias",
+                  BIAS_CAP - 64);
+
+    const Store form = g.conv_xv != nullptr ? Store::Conv
+                       : g.transpose_c        ? Store::Transposed
+                       : (aligned && g.N % 32 == 0 && bias_ok) ? Store::Vec : Store::Masked;
+
+    TcGemmParams p{};
+    p.g = g;
+    p.g.b_batch_div = b_div;
+    p.vec_store = aligned;
+    p.kb_per_seg = g.n_seg > 0 ? g.seg_k / BK : 0;
     p.a_batched = (g.strideA != 0 && batch > 1) ? 1 : 0;
     p.b_batched = (g.strideB != 0 && batch > 1) ? 1 : 0;
     p.m_tiles = (g.M + BM - 1) / BM;
@@ -708,15 +516,14 @@ int launch_tc_gemm(const GemmArgs& g, int batch, cudaStream_t stream) {
     int grid = device_sm_count();
     if (grid > p.total_tiles) grid = p.total_tiles;
     const long long mz = static_cast<long long>(p.m_tiles) * batch;
-    static const bool no_resident = getenv("CMT_GEMM_NO_B_RESIDENT") != nullptr;
-    if (p.num_kb <= RES_KB && !p.b_batched && p.n_tiles <= device_sm_count() && !no_resident) {
+    if (p.num_kb <= RES_KB && !p.b_batched && p.n_tiles <= device_sm_count()) {
         long long gm = device_sm_count() / p.n_tiles;
         if (gm > mz) gm = mz;
         p.b_resident = 1;
         grid = static_cast<int>(gm) * p.n_tiles;
     }
     {
-        cudaError_t e = launch_pdl(tc_gemm_kernel, dim3(grid), dim3(THREADS), SMEM_BYTES, stream, ta, tb, p);
+        cudaError_t e = launch_pdl(kernels[static_cast<int>(form)], dim3(grid), dim3(THREADS), SMEM_BYTES, stream, ta, tb, p);
         if (e != cudaSuccess) return cuda_fail(e, "cmt_gemm_bias_act(tcgen05) launch");
     }
     CMT_LAUNCH_CHECK("cmt_gemm_bias_act(tcgen05)");

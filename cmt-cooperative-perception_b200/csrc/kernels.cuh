@@ -14,22 +14,29 @@ struct GemmArgs {
     long long strideA, strideB, strideC;
     float alpha;
     int relu, bias_per_row, out_bf16;
-    int transpose_c;   // bf16 tensor-core path only: store C^T inside each column block (see cmt_gemm_bias_act)
-    float* norm2_max;  // bf16 tensor-core path only: [batch][N/32] running max of the squared row norms per 32-column block, or nullptr
+    // bf16 tensor-core path only: element (m, n) of batch z is stored at z*strideC + (n / cb)*cb_stride + (n % cb)*ldc + m
+    // (C^T inside each column block, see cmt_gemm_bias_act)
+    int transpose_c;
+    // bf16 tensor-core path only: [batch][N/32] atomicMax of the squared norm of every row's 32-column block (attention
+    // score bound), or nullptr
+    float* norm2_max;
     // ---- bf16 tensor-core path only: segmented K (n_seg == 0: ordinary GEMM) ----
     // K = n_seg * seg_k columns of B; segment s multiplies B[:, s*seg_k : (s+1)*seg_k] with the A columns
     // [seg_acol[s], seg_acol[s] + seg_k) read at row (m + a_row_off + seg_shift[s]) of the batch's A matrix, which has
-    // a_rows rows and a_cols columns (rows outside [0, a_rows) read as zero).
+    // a_rows rows and a_cols columns (rows outside [0, a_rows) are zero-filled by the TMA unit).
     int n_seg, seg_k, a_row_off, a_cols;
     long long a_rows;
     int seg_acol[18], seg_shift[18];
     int b_batch_div;   // batch z uses B of batch z / b_batch_div (0 or 1: z)
-    // ---- token epilogue of the 3x3 shared_conv (conv_xv != nullptr), see TcGemmParams ----
+    // ---- token epilogue of the 3x3 shared_conv (conv_xv != nullptr) ----
+    // Output row m is position (y, x) = (m / conv_Wp, m % conv_Wp) of the zero-padded map of frame z; interior positions
+    // become token t = (y - 1) * conv_W + (x - 1) and are stored as xv[z][t - tok_begin] = bf16(v),
+    // xk[z][t - tok_begin] = bf16(v + pos[t]) (v = ReLU(acc + bias)); border rows are dropped.
     void* conv_xk;
     void* conv_xv;
     const float* conv_pos;
     int conv_W, conv_H, conv_Wp, conv_tok_begin, conv_tok_end;
-    long long conv_frame_stride;
+    long long conv_frame_stride;   // elements between frames in xk / xv
 };
 
 struct AttnArgs {

@@ -320,6 +320,52 @@ def test_gemm_plain(M, N, K, relu, bias, alpha, mode):
         assert _rel(got16, want) < 4e-3  # one bf16 rounding of the output (2^-9 relative per element)
 
 
+GEMM_LAYOUTS = [
+    # M, N, K, batch, ldc, cb (None: N), cb_stride, strideC, bias ("col" / "row" / None), relu, alpha
+    (200, 72, 128, 1, 72, None, 0, 0, "col", True, 0.5),             # N % 32 != 0 with a bias: ragged last chunk
+    (200, 72, 128, 1, 80, None, 0, 0, "col", True, 0.5),             # ... 32-byte aligned rows: 256-bit chunks + ragged tail
+    (150, 256, 64, 1, 260, None, 0, 0, "col", False, 1.0),           # row pitch not a multiple of 32 bytes
+    (130, 96, 64, 3, 96, None, 0, 130 * 96 + 4, "row", False, 1.0),  # batch stride not a multiple of 32 bytes
+    (140, 2304, 64, 1, 2304, None, 0, 0, "col", True, 1.0),          # column bias wider than the shared-memory cache
+    (140, 2088, 64, 1, 2092, None, 0, 0, "col", False, 0.5),         # ... with ragged N and an unaligned row pitch
+    (170, 128, 64, 2, 32, 32, 170 * 32 + 4, 4 * (170 * 32 + 4), "col", False, 1.0),  # column blocks, unaligned cb_stride
+]
+
+
+@pytest.mark.parametrize("M,N,K,batch,ldc,cb,cb_stride,strideC,bias,relu,alpha", GEMM_LAYOUTS)
+@pytest.mark.parametrize("dt", [torch.bfloat16, torch.float32])
+def test_gemm_output_layouts(M, N, K, batch, ldc, cb, cb_stride, strideC, bias, relu, alpha, dt):
+    """cmt_gemm_bias_act (tcgen05) into output layouts the 256-bit row stores cannot write: every element lands at
+    z*strideC + (n // cb)*cb_stride + m*ldc + n % cb, and nothing else in the buffer is touched."""
+    g = torch.Generator().manual_seed(M + N + K + batch)
+    a = torch.randn(batch, M, K, generator=g).bfloat16()
+    w = (torch.randn(N, K, generator=g) / math.sqrt(K)).bfloat16()
+    b = torch.randn(M if bias == "row" else N, generator=g) if bias else None
+    want = a.double() @ w.double().t()
+    if bias == "row":
+        want = want + b.double()[:, None]
+    elif bias == "col":
+        want = want + b.double()
+    want = want * alpha
+    if relu:
+        want = want.clamp_min(0)
+    cb = cb or N
+    z, m, n = torch.meshgrid(torch.arange(batch), torch.arange(M), torch.arange(N), indexing="ij")
+    idx = z * strideC + (n // cb) * cb_stride + m * ldc + n % cb
+    size = int(idx.max()) + 1 + 8
+    C = torch.full((size,), -7.0, dtype=dt, device=DEV)
+    ops.gemm(a.to(DEV), w.to(DEV), None if b is None else b.to(DEV), C, M, N, K, lda=K, ldb=K, ldc=ldc, cb=cb,
+             cb_stride=cb_stride, batch=batch, strideA=M * K if batch > 1 else 0, strideC=strideC, alpha=alpha, relu=relu,
+             bias_per_row=bias == "row")
+    torch.cuda.synchronize()
+    out = C.cpu().float()
+    # fp32: K products accumulated in fp32; bf16: one rounding of the output (2^-9 relative per element)
+    assert _rel(out[idx], want) < (4e-3 if dt == torch.bfloat16 else 5e-6)
+    untouched = torch.ones(size, dtype=torch.bool)
+    untouched[idx.flatten()] = False
+    assert bool((out[untouched] == -7.0).all())
+
+
 @pytest.mark.parametrize("dt", [torch.bfloat16, torch.float32])
 def test_gemm_head_layouts(dt):
     """All-layer K projection into [B,L,H,N_kv,32] and V^T projection into [B,L,H,32,ld]."""
