@@ -412,6 +412,17 @@ int cmt_add_layernorm(const float* x, const float* r, const float* gamma, const 
                                 static_cast<cudaStream_t>(stream));
 }
 
+int cmt_bbox_topk_decode(const float* const* task_ptrs_host, const int* task_classes_host, int T, int B, int Nq,
+                         int num_classes, int max_num, const float* post_center_range_host, float score_threshold,
+                         int use_score_threshold, int bottom_center, float* boxes, float* scores, int64_t* labels,
+                         int32_t* count, int64_t* topk_index, void* stream) {
+    CMT_REQUIRE_DEVICE();
+    return launch_bbox_topk_decode(task_ptrs_host, task_classes_host, T, B, Nq, num_classes, max_num, post_center_range_host,
+                                   score_threshold, use_score_threshold, bottom_center, boxes, scores,
+                                   reinterpret_cast<long long*>(labels), count, reinterpret_cast<long long*>(topk_index),
+                                   static_cast<cudaStream_t>(stream));
+}
+
 int cmt_coop_max(const float* a, const float* b, float* out, int64_t n, void* stream) {
     CMT_REQUIRE_DEVICE();
     return launch_coop_max(a, b, out, n, static_cast<cudaStream_t>(stream));

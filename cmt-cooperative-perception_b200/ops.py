@@ -631,3 +631,58 @@ def task_head_tail(h, gamma, beta, w2, b2, eps, ksize=1, Nq=None, ref_logit=None
     if head_couts is not None:
         return [out[s:s + n].view(L, M, int(c)) for s, n, c in zip(starts, sizes, head_couts)]
     return out
+
+
+BOX_DECODE_FIELDS = ("cls_logits", "center", "height", "dim", "rot", "vel")
+_BOX_DECODE_WIDTH = {"center": 2, "height": 1, "dim": 3, "rot": 2, "vel": 2}
+
+
+def bbox_topk_decode(tasks, num_classes, max_num, post_center_range, score_threshold=None, bottom_center=False):
+    """MultiTaskBBoxCoder.decode_single for every frame in one launch (cmt_bbox_topk_decode; multi_task_bbox_coder.py:46-141,
+    util.py:37-68, with bottom_center the z shift of cmt_head.py:912).  tasks: one dict per task of its last decoder
+    layer's fp32 outputs {cls_logits [B,Nq,C_t], center [B,Nq,2], height [B,Nq,1], dim [B,Nq,3], rot [B,Nq,2],
+    vel [B,Nq,2]}.  score_threshold: applied (strict >) only when truthy, like the coder.  Returns the fixed-shape dict
+    {boxes [B,K,9] fp32, scores [B,K] fp32, labels [B,K] int64, count [B] int32, topk_index [B,K] int64}: the kept
+    detections of frame b are the first count[b] slots, in score order; the other slots are zero with label -1."""
+    if not 1 <= len(tasks) <= 8:
+        raise ValueError(f"bbox_topk_decode: {len(tasks)} tasks (1..8 supported)")
+    B, Nq = tasks[0]["cls_logits"].shape[:2]
+    ptrs, classes, keep = [], [], []
+    for ti, d in enumerate(tasks):
+        for name in BOX_DECODE_FIELDS:
+            t = d[name]
+            if not isinstance(t, torch.Tensor) or not t.is_cuda:
+                raise _lib.CmtLibraryError(f"task {ti} {name} must be a CUDA tensor: libcmtcoop_b200 has no CPU fallback")
+            if t.dtype != torch.float32:
+                raise TypeError(f"task {ti} {name} must be torch.float32, got {t.dtype}")
+            width = _BOX_DECODE_WIDTH.get(name, t.shape[-1])
+            if t.dim() != 3 or tuple(t.shape) != (B, Nq, width) or t.device != tasks[0]["cls_logits"].device:
+                raise ValueError(f"task {ti} {name}: expected [{B},{Nq},{width}] on {tasks[0]['cls_logits'].device}, "
+                                 f"got {tuple(t.shape)} on {t.device}")
+            t = t.contiguous()
+            keep.append(t)
+            ptrs.append(t.data_ptr())
+        classes.append(int(d["cls_logits"].shape[-1]))
+    if sum(classes) != num_classes:
+        raise ValueError(f"bbox_topk_decode: num_classes {num_classes} != sum of the tasks' classes {sum(classes)}")
+    if len(post_center_range) != 6:
+        raise ValueError("post_center_range must have 6 entries")
+    K = int(max_num)   # 1 <= K <= min(1024, Nq * num_classes), checked by the library
+    dev = keep[0].device
+    out = dict(boxes=torch.empty((B, K, 9), dtype=torch.float32, device=dev),
+               scores=torch.empty((B, K), dtype=torch.float32, device=dev),
+               labels=torch.empty((B, K), dtype=torch.int64, device=dev),
+               count=torch.empty((B,), dtype=torch.int32, device=dev),
+               topk_index=torch.empty((B, K), dtype=torch.int64, device=dev))
+    p_arr = (ctypes.c_void_p * len(ptrs))(*ptrs)
+    c_arr = (ctypes.c_int * len(classes))(*classes)
+    lib = _lib.load()
+    with torch.cuda.device(dev):
+        rc = lib.cmt_bbox_topk_decode(ctypes.cast(p_arr, ctypes.c_void_p), ctypes.cast(c_arr, ctypes.c_void_p), len(tasks), B,
+                                      Nq, int(num_classes), K, ctypes.cast(_pc(post_center_range), ctypes.c_void_p),
+                                      float(score_threshold or 0.0), 1 if score_threshold else 0, 1 if bottom_center else 0,
+                                      *[_ptr(out[n]) for n in ("boxes", "scores", "labels", "count", "topk_index")],
+                                      _stream(keep[0]))
+    _lib.check(rc, "cmt_bbox_topk_decode")
+    _count()
+    return out

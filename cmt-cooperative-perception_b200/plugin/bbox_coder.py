@@ -1,10 +1,16 @@
 """MultiTaskBBoxCoder (projects/mmdet3d_plugin/core/bbox/coders/multi_task_bbox_coder.py:15-141) and
-denormalize_bbox (core/bbox/util.py:37-68).  Negligible work; stays PyTorch.  The flat top-k over
-sigmoid(cls) and `label = idx % C`, `query = idx // C` are what "identical top-k query indices" checks."""
+denormalize_bbox (core/bbox/util.py:37-68).  The flat top-k over sigmoid(cls) and `label = idx % C`,
+`query = idx // C` are what "identical top-k query indices" checks.
+
+`decode` is the reference's per-frame torch loop: few FLOPs, but about 30 launches and three `nonzero` host
+synchronisations per frame (`boxes[mask]`, ...), so it cannot be captured in a CUDA graph; it also serves CPU tensors.
+`decode_batched` computes the same detections for every frame in one library launch (`cmt_bbox_topk_decode`) with no
+host synchronisation, into fixed-shape outputs that can live in a graph."""
 from __future__ import annotations
 
 import torch
 
+from .. import ops
 from .registry import BBOX_CODERS
 
 
@@ -60,6 +66,22 @@ class MultiTaskBBoxCoder:
         all_bbox = torch.cat(bbox_l, dim=1)
         all_tids = torch.cat(tid_l, dim=-1)
         return [self.decode_single(all_logits[i], all_bbox[i], all_tids[i]) for i in range(all_logits.shape[0])]
+
+
+    def decode_batched(self, preds_dicts, bottom_center=False):
+        """Fixed-shape counterpart of `decode` on CUDA tensors, one launch for the whole batch (ops.bbox_topk_decode).
+        Returns {boxes [B,K,9], scores [B,K], labels [B,K], count [B], topk_index [B,K]}: frame b's detections are
+        boxes[b, :count[b]] (= decode(...)[b]["bboxes"]), the remaining slots are zero with label -1.  Boxes are before
+        CmtHead.get_bboxes' z shift unless bottom_center (then z -= h / 2 in the kernel)."""
+        if self.post_center_range is None:
+            raise NotImplementedError("Need to reorganize output as a batch, only support "
+                                      "post_center_range is not None for now!")
+        tasks = [{n: preds_dicts[t][0][n][-1] for n in ops.BOX_DECODE_FIELDS} for t in range(len(preds_dicts))]
+        n_cls = sum(int(d["cls_logits"].shape[-1]) for d in tasks)
+        if n_cls != self.num_classes:
+            raise ValueError(f"MultiTaskBBoxCoder: num_classes {self.num_classes} != {n_cls} classes of the task heads")
+        return ops.bbox_topk_decode(tasks, self.num_classes, self.max_num, self.post_center_range, self.score_threshold,
+                                    bottom_center)
 
 
 def build_bbox_coder(cfg):

@@ -603,6 +603,13 @@ class _CmtHeadBase(nn.Module):
             ret_list.append([bboxes, preds["scores"], preds["labels"]])
         return ret_list
 
+    def get_bboxes_batched(self, preds_dicts, img_metas):
+        """Fixed-shape counterpart of `get_bboxes` for CUDA tensors: every frame decoded in one launch with the z shift
+        applied, no host synchronisation (can be captured in a CUDA graph).  Returns the device-tensor dict
+        {boxes [B,K,9], scores [B,K], labels [B,K], count [B], topk_index [B,K]} of `bbox_coder.decode_batched`;
+        detector_glue.batched_to_results turns it into per-frame result dicts."""
+        return self.bbox_coder.decode_batched(preds_dicts, bottom_center=True)
+
 
 @HEADS.register_module()
 class CmtHead(_CmtHeadBase):

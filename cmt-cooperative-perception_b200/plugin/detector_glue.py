@@ -5,6 +5,8 @@ the reference drives its own.
 
 * `simple_test_pts` / `coop_simple_test_pts`: head forward -> get_bboxes -> bbox3d2result, same argument meaning and
   result dicts as the reference methods (`self` replaced by the head).
+* `batched_to_results`: the fixed-shape batched decode (`get_bboxes_batched`) -> the per-frame result dicts of
+  `simple_test_pts`, with one device->host copy for the whole batch.
 * `device_calibration`: lidar2img -> (lidar2img, img2lidar) fp32 device tensors built ON the device in float64 --
   including the vehicle -> infrastructure fold `lidar2img @ inv(vehicle2infrastructure)` that the reference does in its
   CPU data pipeline (datasets/pipelines/transforms_3d_coop.py:213-222) and the float64 inverse the head does with numpy
@@ -24,6 +26,28 @@ def bbox3d2result(bboxes, scores, labels, attrs=None):
     if attrs is not None:
         result["attrs_3d"] = attrs.cpu()
     return result
+
+
+def batched_to_results(batched, img_metas):
+    """batched: CmtHead.get_bboxes_batched(...) (device tensors).  Returns per frame dict(boxes_3d, scores_3d, labels_3d)
+    as CPU tensors, equal to what simple_test_pts returns for the same head outputs (box_type_3d applied when the frame's
+    metas carry one).  The boxes, scores, labels and counts of all frames travel in ONE device->host copy."""
+    boxes, scores, labels, count = batched["boxes"], batched["scores"], batched["labels"], batched["count"]
+    B, K = scores.shape
+    parts = [boxes.reshape(B, K * 9), scores, labels, count.reshape(B, 1)]
+    host = torch.cat([t.contiguous().view(torch.uint8).reshape(B, -1) for t in parts], 1).cpu()
+    widths = [K * 36, K * 4, K * 8, 4]
+    results = []
+    for i in range(B):
+        row = host[i].split(widths)
+        n = int(row[3].clone().view(torch.int32))
+        bboxes = row[0][:n * 36].clone().view(torch.float32).view(n, 9)
+        box_type = img_metas[i].get("box_type_3d")
+        if box_type is not None:
+            bboxes = box_type(bboxes, bboxes.size(-1))
+        results.append(bbox3d2result(bboxes, row[1][:n * 4].clone().view(torch.float32),
+                                     row[2][:n * 8].clone().view(torch.int64)))
+    return results
 
 
 def simple_test_pts(head, x, x_img, img_metas, rescale=False):

@@ -6,7 +6,7 @@ three CUDA streams and double buffering:
 
     copy-in stream : pinned host features -> device buffer[i % 2]
     compute stream : head.forward_single(device buffer[i % 2]) -> task-head tensors
-    copy-out stream: task-head tensors -> pinned host result[i % 2]
+    copy-out stream: task-head tensors (or, with outputs="boxes", the batched box decode) -> pinned host result[i % 2]
 
 This is plumbing (torch streams / events), not a kernel; it is what bench.py's end-to-end number uses.
 
@@ -60,7 +60,7 @@ class numa_local_to_gpu:
 
 class PipelinedRunner:
     def __init__(self, head, img_metas, example_inputs: dict, device, use_cuda_graph: bool = False,
-                 keep_results: bool = True, partial_upload=None):
+                 keep_results: bool = True, partial_upload=None, outputs: str = "heads"):
         """example_inputs: {name: pinned CPU tensor} with the feature tensors `forward_single` takes
         (pts_feats / img_feats, or the four vehicle_/infrastructure_ entries for the coop heads); fp32, bf16 or
         fp16 -- the gather kernel rounds every feature to the compute dtype on arrival, so 16-bit features halve
@@ -71,7 +71,15 @@ class PipelinedRunner:
         batches), for callers that consume results through `on_result`.
         partial_upload: under the KV-token split a rank reads only the map rows that hold its tokens, so only those
         rows are copied to the device (a few strided cudaMemcpy2DAsync per tensor, parallel.token_rows_copy_plan); the rest of
-        the device buffers is never read.  None = do so whenever the split is enabled on a non-cooperative head."""
+        the device buffers is never read.  None = do so whenever the split is enabled on a non-cooperative head.
+        outputs: what each batch hands back.  "heads": the task-head outputs of every decoder layer (the list of per-task
+        dicts forward_single returns).  "boxes": the detections, head.get_bboxes_batched of those outputs, computed on
+        the device after the forward (inside the graph with use_cuda_graph) -- only that fixed-shape dict
+        {boxes, scores, labels, count, topk_index} is copied back (detector_glue.batched_to_results makes per-frame
+        results of it)."""
+        if outputs not in ("heads", "boxes"):
+            raise ValueError(f'outputs must be "heads" or "boxes", got {outputs!r}')
+        self.outputs = outputs
         self.head = head
         self.metas = img_metas
         self.dev = torch.device(device)
@@ -102,14 +110,23 @@ class PipelinedRunner:
                 for k in self.keys:
                     self.dbuf[slot][k].copy_(example_inputs[k], non_blocking=True)
             torch.cuda.current_stream(self.dev).synchronize()
-            self.graphs = [GraphedForward(head, img_metas, self.dbuf[slot], adopt_inputs=True) for slot in range(2)]
+            self.graphs = [GraphedForward(head, img_metas, self.dbuf[slot], adopt_inputs=True,
+                                          decode_boxes=outputs == "boxes") for slot in range(2)]
 
     def _forward(self, feats):
         g = feats.get
         if self.coop:
-            return self.head.forward_single(g("vehicle_pts_feats"), g("infrastructure_pts_feats"),
+            rets = self.head.forward_single(g("vehicle_pts_feats"), g("infrastructure_pts_feats"),
                                             g("vehicle_img_feats"), g("infrastructure_img_feats"), self.metas)
-        return self.head.forward_single(g("pts_feats"), g("img_feats"), self.metas)
+        else:
+            rets = self.head.forward_single(g("pts_feats"), g("img_feats"), self.metas)
+        if self.outputs == "boxes":
+            return rets, self.head.get_bboxes_batched([[r] for r in rets], self.metas)
+        return rets
+
+    def _payload(self, staging):
+        """What a batch hands out: the per-task list of head outputs, or the box dict."""
+        return staging[0] if self.outputs == "boxes" else staging
 
     def _plan_partial_upload(self, example_inputs):
         """Rectangles of the feature maps this rank's tokens live in (KV-token split)."""
@@ -158,12 +175,13 @@ class PipelinedRunner:
     def _collect(self, slot):
         """Host copy of the staging buffers of `slot` once its device->host transfer has landed."""
         self.ev_out[slot].synchronize()
-        return [{n: t.clone() for n, t in task.items()} for task in self.hout[slot]]
+        return self._payload([{n: t.clone() for n, t in task.items()} for task in self.hout[slot]])
 
     @torch.no_grad()
     def run(self, host_batches, on_result=None):
         """host_batches: iterable of {name: pinned CPU tensor}.  Returns one entry per batch: the list (one dict per
-        task) of head outputs as CPU tensors.  Every device->host copy has completed when this returns.
+        task) of head outputs as CPU tensors, or with outputs="boxes" the batched box-decode dict.  Every device->host
+        copy has completed when this returns.
         on_result(i, staging): optional callback invoked with the pinned staging dicts of batch i right after its
         transfer completed (zero-copy consumers); with keep_results=False the returned list holds None for every
         batch but the last two, whose entries are the staging buffers themselves."""
@@ -193,7 +211,7 @@ class PipelinedRunner:
                 j = pending[slot]
                 if on_result is not None:
                     self.ev_out[slot].synchronize()
-                    on_result(j, self.hout[slot])
+                    on_result(j, self._payload(self.hout[slot]))
                 if self.keep_results:
                     results[j] = self._collect(slot)
                 pending[slot] = None
@@ -204,6 +222,8 @@ class PipelinedRunner:
                 # next copy-out: both wait for the copy-out of the slot's previous batch
                 cur.wait_event(self.ev_out[slot])
             rets = self.graphs[slot]() if self.graphs is not None else self._forward(self.dbuf[slot])
+            if self.outputs == "boxes":
+                rets = [rets[1]]
             self.ev_free[slot].record(cur)
             self._primed[slot] = True
             if trace:
@@ -235,8 +255,8 @@ class PipelinedRunner:
             if j is None:
                 continue
             if on_result is not None:
-                on_result(j, self.hout[slot])
-            results[j] = self._collect(slot) if self.keep_results else self.hout[slot]
+                on_result(j, self._payload(self.hout[slot]))
+            results[j] = self._collect(slot) if self.keep_results else self._payload(self.hout[slot])
         return results
 
 
@@ -261,14 +281,20 @@ class GraphedForward:
         g = GraphedForward(head, img_metas, {"pts_feats": x, "img_feats": x_img})   # device tensors
         rets = g(inputs)          # copies `inputs` into the graph's static buffers (unless they ARE those buffers), replays
 
+    With decode_boxes=True the graph also holds `head.get_bboxes_batched` of the outputs, and a call returns
+    (head outputs, boxes dict), both static outputs of the graph.
+
     The graph bakes in device addresses, so the inputs live in static buffers (`g.static_inputs`) and the outputs are
     overwritten by the next replay.  The calibration matrices enter the forward as device tensors uploaded once per
     distinct `img_metas` (CmtHead._matrices); a call with different calibration re-captures.
     """
 
-    def __init__(self, head, img_metas, example_inputs: dict, warmup: int = 3, adopt_inputs: bool = False):
-        """adopt_inputs: use the given tensors themselves as the graph's static input buffers (no clone)."""
+    def __init__(self, head, img_metas, example_inputs: dict, warmup: int = 3, adopt_inputs: bool = False,
+                 decode_boxes: bool = False):
+        """adopt_inputs: use the given tensors themselves as the graph's static input buffers (no clone).
+        decode_boxes: capture the batched box decode (head.get_bboxes_batched) after the forward."""
         self.head = head
+        self.decode_boxes = decode_boxes
         self.coop = type(head).__name__.endswith("Coop")
         self.static_inputs = {k: (v if adopt_inputs else v.clone()) for k, v in example_inputs.items() if v is not None}
         self.graph = None
@@ -279,9 +305,13 @@ class GraphedForward:
     def _forward(self, metas):
         g = self.static_inputs.get
         if self.coop:
-            return self.head.forward_single(g("vehicle_pts_feats"), g("infrastructure_pts_feats"),
+            rets = self.head.forward_single(g("vehicle_pts_feats"), g("infrastructure_pts_feats"),
                                             g("vehicle_img_feats"), g("infrastructure_img_feats"), metas)
-        return self.head.forward_single(g("pts_feats"), g("img_feats"), metas)
+        else:
+            rets = self.head.forward_single(g("pts_feats"), g("img_feats"), metas)
+        if self.decode_boxes:
+            return rets, self.head.get_bboxes_batched([[r] for r in rets], metas)
+        return rets
 
     @torch.no_grad()
     def _capture(self, img_metas, warmup):

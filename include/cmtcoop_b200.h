@@ -260,6 +260,35 @@ int cmt_task_head_tail(const float* h, const float* gamma, const float* beta, co
  * out = max(nan_to_num(a), nan_to_num(b)) element-wise (cmt_head_coop.py:358,383-389). */
 int cmt_coop_max(const float* a, const float* b, float* out, int64_t n, void* stream);
 
+/* ---- box decode ------------------------------------------------------------------------
+ * MultiTaskBBoxCoder.decode_single for every frame of a batch in one launch, with no host synchronisation (graph
+ * capturable): replaces the per-frame sigmoid / top-k / gather / denormalize_bbox / mask loop of
+ * MultiTaskBBoxCoder.decode (core/bbox/coders/multi_task_bbox_coder.py:46-141, core/bbox/util.py:37-68) and, with
+ * bottom_center, the z shift of CmtHead.get_bboxes (models/dense_heads/cmt_head.py:912).
+ *   task_ptrs_host: HOST array of 6*T device pointers, per task t < T <= CMT_BOX_DECODE_MAX_TASKS the last decoder
+ *       layer's contiguous fp32 outputs {cls_logits [B,Nq,C_t], center [B,Nq,2], height [B,Nq,1], dim [B,Nq,3],
+ *       rot [B,Nq,2], vel [B,Nq,2]};  task_classes_host: HOST array of the T class counts C_t.
+ *   num_classes must equal sum C_t; the flat candidate index is q*num_classes + c, c running over the tasks' classes in
+ *   concatenation order (torch.cat(cls_logits, -1)).  Per frame:
+ *     score = 1 / (1 + expf(-logit)); the K = max_num largest scores in descending order, ties by ascending flat index
+ *     (torch.sort(descending=True, stable=True)[:K]; NaN ranks above +inf);
+ *     label = idx % num_classes, q = idx / num_classes; box = [cx, cy, cz, exp(w), exp(l), exp(h), atan2(rot0, rot1),
+ *     vx, vy] from the task that owns the label; kept when post_center_range_host[0..2] <= (cx, cy, cz) <=
+ *     post_center_range_host[3..5] and, if use_score_threshold, score > score_threshold;  bottom_center: z -= h * 0.5.
+ *   Outputs (caller-owned, fixed shape): boxes [B,K,9] fp32, scores [B,K] fp32, labels [B,K] int64 -- the kept slots
+ *     first, in score order, then zeros with label -1;  count [B] int32 kept slots;  topk_index [B,K] int64 every
+ *     selected flat index before the mask.
+ *   Limits (CMT_ERR_BAD_ARG otherwise): 1 <= K <= min(CMT_BOX_DECODE_MAX_K, Nq*num_classes), and
+ *     Nq*num_classes <= CMT_BOX_DECODE_MAX_CANDIDATES (one CTA per frame keeps every score in shared memory; nuScenes
+ *     is 900 x 10 = 9000). */
+#define CMT_BOX_DECODE_MAX_TASKS 8
+#define CMT_BOX_DECODE_MAX_K 1024
+#define CMT_BOX_DECODE_MAX_CANDIDATES 49152
+int cmt_bbox_topk_decode(const float* const* task_ptrs_host, const int* task_classes_host, int T, int B, int Nq,
+                         int num_classes, int max_num, const float* post_center_range_host, float score_threshold,
+                         int use_score_threshold, int bottom_center, float* boxes, float* scores, int64_t* labels,
+                         int32_t* count, int64_t* topk_index, void* stream);
+
 /* ---- diagnostics -----------------------------------------------------------------------
  * Cycle accounting of the tcgen05 attention kernel on the CURRENT device.  dev_buf: device buffer of
  * 3*96*16 + 148 int64 (or NULL to switch the hook off again).  While set, every CTA of every following

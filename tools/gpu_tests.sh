@@ -16,3 +16,4 @@ run attn_edges tests/test_gpu_attention_edges.py
 run heads tests/test_gpu_heads.py
 run decoder tests/test_gpu_decoder.py
 run multi tests/test_gpu_multi.py
+run decode tests/test_gpu_bbox_decode.py
