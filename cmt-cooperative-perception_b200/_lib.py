@@ -34,8 +34,8 @@ SIGNATURES = {
                                _i64, _i64, _i64, _f, _i, _i, _i, _vp, _vp]),
     "cmt_gemm_segmented": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _i, _i64, _i, _i64, _i64, _i64, _i, _i64, _i64, _i,
                                 _i64, _f, _i, _i, _vp]),
-    "cmt_nchw_to_padded_nhwc": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
-    "cmt_shared_conv_tokens": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i64, _i, _i, _vp]),
+    "cmt_nchw_to_padded_nhwc": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i]),
+    "cmt_shared_conv_tokens": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i64, _i, _i, _vp, _i]),
     "cmt_cross_attn_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "cmt_cross_attn_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i64, _i64, _i64,
                                 _i64, _i64, _i64, _vp, _vp, _vp, _i64, _i, _i, _vp, _sz, _vp]),

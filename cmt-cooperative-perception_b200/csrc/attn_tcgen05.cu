@@ -1,5 +1,5 @@
 // K3: flash-style cross-attention of the object queries over the BEV ++ image tokens on the
-// 5th-gen tensor cores (head dim 32, bf16 operands, fp32 accumulate / softmax statistics).
+// 5th-gen tensor cores (head dim 32, bf16 or fp16 operands, fp32 accumulate / softmax statistics).
 //
 // Replaces flash_attn_unpadded_kvpacked_func as called from
 // projects/mmdet3d_plugin/models/utils/attention.py:46-92 (softmax(QK^T/sqrt(d))V, non-causal).
@@ -17,6 +17,9 @@
 //   static  : when the caller passes the operand-norm maxima of the projections, |q.k| <= |q||k| bounds every score
 //             of a (frame, head); where the bound is <= 60 the weights 2^s need no shift at all (no row maximum, no
 //             subtraction, no rescale).  Items above the bound fall to the online kernel.
+// Each has bf16 and fp16 instantiations (Q, K, V^T and P in that dtype).  fp16 has 3 more mantissa bits but 5 exponent
+// bits: its static limit is 14 instead of 60 (every weight 2^s in [2^-14, 2^14], normal fp16), and the online kernel's
+// lazy rescale keeps P <= 2^8.
 #include <cstdlib>
 #include <cstring>
 #include <type_traits>
@@ -190,7 +193,8 @@ constexpr int ST_POLY = 3;
 // The lone active warp of a tail tile (see lone_warp below).  Measured (B=8, static kernel): every second pair
 // polynomial 806 us, all pairs 913.
 constexpr int LONE_POLY = 2;
-constexpr float STATIC_LIMIT = 60.0f;
+constexpr float STATIC_LIMIT = 60.0f;       // bf16 P: 2^[-60, 60] are normal bf16 numbers
+constexpr float STATIC_LIMIT_F16 = 14.0f;   // fp16 P: 2^[-14, 14] are normal fp16 numbers (largest finite 65504 < 2^16)
 // pair i of a 16-pair chunk is polynomial when i % period == period - 1 (period 0: none)
 constexpr uint32_t poly_mask(int period) {
     uint32_t m = 0;
@@ -210,7 +214,8 @@ constexpr uint32_t LONE_MASK = poly_mask(LONE_POLY);
 // STATIC_LIMIT and records per CTA whether it skipped any item; <false> processes exactly those (its CTAs return at
 // once when their flag is clear).  Keeping the two softmax loops in separate kernels matters for the same reason as
 // kMask: sharing a kernel cost the online loop 8 %.
-template <bool kMask, bool kStatic>
+// kF16: fp16 Q / K / V^T and P (static limit STATIC_LIMIT_F16), bf16 otherwise.
+template <bool kMask, bool kStatic, bool kF16>
 __global__ void __launch_bounds__(attndb::THREADS, 1)
 tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant__ CUtensorMap tma_k,
                   const __grid_constant__ CUtensorMap tma_v, const TcAttnParams p) {
@@ -270,12 +275,13 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
     const long long pos_end = range_start(p, blockIdx.x + 1, G);
     // Which items are this instantiation's?  Without norms: everything goes to the online kernel.  With norms: the item's
     // Cauchy-Schwarz score bound |q||k| (norms of the fp32 projection outputs; + 2^-7 covers the two bf16 roundings the
-    // MMA operands went through) decides.  Every role evaluates the same predicate, so skipped segments touch no barrier.
+    // MMA operands went through, and more than covers two fp16 roundings) decides.  Every role evaluates the same predicate,
+    // so skipped segments touch no barrier.
     auto mine = [&](int item) -> bool {
         if (p.q_norm2 == nullptr) return !kStatic;
         const int hb = item % p.BH;   // b * H + h
         const float bound = sqrtf(__ldg(p.q_norm2 + hb) * __ldg(p.k_norm2 + static_cast<long long>(hb / p.H) * p.kn_bstride + hb % p.H)) * 1.0079f + 1e-3f;
-        return (bound <= STATIC_LIMIT) == kStatic;
+        return (bound <= (kF16 ? STATIC_LIMIT_F16 : STATIC_LIMIT)) == kStatic;
     };
 
     if (warp == W_TMA) {
@@ -330,8 +336,8 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
         // ------------- MMA issuers: warp W_MMA + ii serves the warpgroups i with i % NISS == ii -------------
         const int ii = warp - W_MMA;
         const bool leader = elect_one();
-        constexpr uint32_t idesc_s = make_idesc_bf16(128, KT);
-        constexpr uint32_t idesc_o = make_idesc_bf16(128, 32);
+        constexpr uint32_t idesc_s = make_idesc(128, KT, kF16);
+        constexpr uint32_t idesc_o = make_idesc(128, 32, kF16);
         const uint32_t sq = smem_u32(smem + OFF_Q);
         uint32_t kc = 0, vc = 0, seg = 0;
         uint32_t g[NWG];                       // steps retired per warpgroup (buffer = g & 1, parity = (g >> 1) & 1)
@@ -548,7 +554,7 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
                             e1 = ex2_approx(x1);
                         }
                         l2 = add_f32x2(l2, pack_f32x2(e0, e1));
-                        pk[i] = pack_bf16x2(e0, e1);
+                        pk[i] = pack_lp2<kF16 ? CMT_F16 : CMT_BF16>(e0, e1);
                     }
                     tmem_st16(t_sb + c * 16, pk);
                 }
@@ -562,8 +568,8 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
                 ++g;
             };
 
-            // static variant: every score of the item lies in [-STATIC_LIMIT, STATIC_LIMIT] (see `mine`), so the weights
-            // 2^s are normal numbers as they are: the softmax is shift-invariant, hence no row maximum, no subtraction
+            // static variant: every score of the item lies in [-limit, limit] (see `mine`), so the weights 2^s are normal
+            // numbers of the P dtype as they are: the softmax is shift-invariant, hence no row maximum, no subtraction
             // and no rescale of O; the partial's LSE is just log2 of the sum (m = 0).
             if (kStatic) m = 0.0f;
             // A tile with at most 32 queries (the 4-query tail of 900 = 7 * 128 + 4) has ONE active warp, and that warp
@@ -581,7 +587,7 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
             if (kMask) {
                 // A segment without an attended key is no partial at all: l = 0 gives o = 0 and LSE = m + log2(0) = -inf
                 // (m is finite), i.e. weight 0 in the merge.  Its padded scores still gave the clamped polynomial lanes
-                // 2^-125 each, so l > 0 on its own.
+                // 2^-125 each, so l > 0 on its own (in fp16 those lanes round to 0 in P; l is summed in fp32 either way).
                 // The segment's mask words, addressed afresh from pos (already past the segment) and item: keeping
                 // mask_row + j0 live across the step loop made the static kernel spill more.
                 const unsigned long long* seg_bits = p.mask_bits + static_cast<long long>((item % p.BH) / p.H) * p.T +
@@ -623,7 +629,7 @@ tc_attn_db_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_consta
 
 // Merge the per-CTA segments of each item.  One block = 32 rows of one item, one thread = (row, 4 output dims); the
 // item's segment count (two 64-bit divisions) is computed once per block, not per thread (17 -> ~5 us per launch).
-template <bool kBf16>
+template <int kOut>
 __global__ void __launch_bounds__(256) tc_attn_merge_kernel(TcAttnParams p, long long G, void* o,
                                                             float* lse) {
     __shared__ int nseg_s;
@@ -664,10 +670,10 @@ __global__ void __launch_bounds__(256) tc_attn_merge_kernel(TcAttnParams p, long
     const float inv = den > 0.f ? 1.0f / den : 0.f;
     acc.x *= inv; acc.y *= inv; acc.z *= inv; acc.w *= inv;
     const long long oidx = ((static_cast<long long>(b) * p.Nq + row) * p.H + h) * 8 + q4;  // float4 units
-    if (kBf16) {
+    if (kOut != CMT_F32) {
         uint2 w;
-        w.x = pack_bf16x2(acc.x, acc.y);
-        w.y = pack_bf16x2(acc.z, acc.w);
+        w.x = pack_lp2<kOut>(acc.x, acc.y);
+        w.y = pack_lp2<kOut>(acc.z, acc.w);
         reinterpret_cast<uint2*>(o)[oidx] = w;
     } else {
         reinterpret_cast<float4*>(o)[oidx] = acc;
@@ -746,10 +752,10 @@ int launch_tc_attn(const AttnArgs& a, void* workspace, size_t workspace_bytes, c
     CMT_CHECK_ARG(n_tok > 0, "cmt_cross_attn_fwd: empty token range");
     CMT_CHECK_ARG(a.q_ld % 8 == 0 && a.v_ld % 8 == 0 && a.k_bstride % 8 == 0 && a.k_hstride % 8 == 0 &&
                       a.v_bstride % 8 == 0 && a.v_hstride % 8 == 0,
-                  "cmt_cross_attn_fwd(bf16): strides must be multiples of 8 elements");
+                  "cmt_cross_attn_fwd(tcgen05): strides must be multiples of 8 elements");
     CMT_CHECK_ARG(((reinterpret_cast<uintptr_t>(a.q) | reinterpret_cast<uintptr_t>(a.k) |
                     reinterpret_cast<uintptr_t>(a.vt) | reinterpret_cast<uintptr_t>(a.o)) & 15) == 0,
-                  "cmt_cross_attn_fwd(bf16): pointers must be 16-byte aligned");
+                  "cmt_cross_attn_fwd(tcgen05): pointers must be 16-byte aligned");
     TcAttnParams p{};
     int grid;
     long long G;
@@ -784,32 +790,37 @@ int launch_tc_attn(const AttnArgs& a, void* workspace, size_t workspace_bytes, c
     }
     p.unsafe_flags = reinterpret_cast<int*>(tail + static_cast<size_t>(a.B) * p.T * 8 + 8);
 
+    // [mask][static][f16]
+    static void (*const kernels[2][2][2])(CUtensorMap, CUtensorMap, CUtensorMap, TcAttnParams) = {
+        {{tc_attn_db_kernel<false, false, false>, tc_attn_db_kernel<false, false, true>},
+         {tc_attn_db_kernel<false, true, false>, tc_attn_db_kernel<false, true, true>}},
+        {{tc_attn_db_kernel<true, false, false>, tc_attn_db_kernel<true, false, true>},
+         {tc_attn_db_kernel<true, true, false>, tc_attn_db_kernel<true, true, true>}}};
     static DeviceOnce attr_once;
     int attr_dev;
     if (attr_once.need(&attr_dev)) {
-        const void* fns[4] = {reinterpret_cast<const void*>(&tc_attn_db_kernel<false, false>),
-                              reinterpret_cast<const void*>(&tc_attn_db_kernel<false, true>),
-                              reinterpret_cast<const void*>(&tc_attn_db_kernel<true, false>),
-                              reinterpret_cast<const void*>(&tc_attn_db_kernel<true, true>)};
-        for (const void* f : fns) {
-            cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, attndb::SMEM_BYTES);
-            if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(tc_attn_db)");
-        }
+        for (const auto& by_static : kernels)
+            for (const auto& by_dtype : by_static)
+                for (const auto f : by_dtype) {
+                    cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, attndb::SMEM_BYTES);
+                    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(tc_attn_db)");
+                }
         attr_once.mark(attr_dev);
     }
+    const int dt = a.f16 ? CMT_F16 : CMT_BF16;
     CUtensorMap tq, tk, tv;
     {
         uint64_t dims[4] = {32, static_cast<uint64_t>(a.Nq), static_cast<uint64_t>(a.H), static_cast<uint64_t>(a.B)};
         uint64_t strides[3] = {static_cast<uint64_t>(a.q_ld) * 2, 64, static_cast<uint64_t>(a.Nq) * a.q_ld * 2};
         uint32_t box[4] = {32, 128, 1, 1};
-        int rc = encode_tma_bf16(&tq, a.q, 4, dims, strides, box, 64);
+        int rc = encode_tma(&tq, a.q, dt, 4, dims, strides, box, 64);
         if (rc) return rc;
     }
     {
         uint64_t dims[4] = {32, static_cast<uint64_t>(a.kv_end), static_cast<uint64_t>(a.H), static_cast<uint64_t>(a.B)};
         uint64_t strides[3] = {64, static_cast<uint64_t>(a.k_hstride) * 2, static_cast<uint64_t>(a.k_bstride) * 2};
         uint32_t box[4] = {32, static_cast<uint32_t>(p.kt), 1, 1};
-        int rc = encode_tma_bf16(&tk, a.k, 4, dims, strides, box, 64);
+        int rc = encode_tma(&tk, a.k, dt, 4, dims, strides, box, 64);
         if (rc) return rc;
     }
     {
@@ -817,29 +828,29 @@ int launch_tc_attn(const AttnArgs& a, void* workspace, size_t workspace_bytes, c
         uint64_t strides[3] = {static_cast<uint64_t>(a.v_ld) * 2, static_cast<uint64_t>(a.v_hstride) * 2,
                                static_cast<uint64_t>(a.v_bstride) * 2};
         uint32_t box[4] = {64, 32, 1, 1};
-        int rc = encode_tma_bf16(&tv, a.vt, 4, dims, strides, box, 128);
+        int rc = encode_tma(&tv, a.vt, dt, 4, dims, strides, box, 128);
         if (rc) return rc;
     }
-    const bool masked = p.mask_bits != nullptr;
+    const int masked = p.mask_bits != nullptr ? 1 : 0, f16 = a.f16 ? 1 : 0;
     if (p.q_norm2 != nullptr) {
-        // static-shift kernel first (items with a score bound <= STATIC_LIMIT), then the online kernel for the rest
-        cudaError_t e = masked ? launch_pdl(tc_attn_db_kernel<true, true>, dim3(grid), dim3(attndb::THREADS), attndb::SMEM_BYTES, stream, tq, tk, tv, p)
-                               : launch_pdl(tc_attn_db_kernel<false, true>, dim3(grid), dim3(attndb::THREADS), attndb::SMEM_BYTES, stream, tq, tk, tv, p);
+        // static-shift kernel first (items with a score bound <= the dtype's static limit), then the online kernel for the rest
+        cudaError_t e = launch_pdl(kernels[masked][1][f16], dim3(grid), dim3(attndb::THREADS), attndb::SMEM_BYTES, stream, tq, tk, tv, p);
         if (e != cudaSuccess) return cuda_fail(e, "cmt_cross_attn_fwd(tcgen05, static shift) launch");
         CMT_LAUNCH_CHECK("cmt_cross_attn_fwd(tcgen05, static shift)");
     }
     {
-        cudaError_t e = masked ? launch_pdl(tc_attn_db_kernel<true, false>, dim3(grid), dim3(attndb::THREADS), attndb::SMEM_BYTES, stream, tq, tk, tv, p)
-                               : launch_pdl(tc_attn_db_kernel<false, false>, dim3(grid), dim3(attndb::THREADS), attndb::SMEM_BYTES, stream, tq, tk, tv, p);
+        cudaError_t e = launch_pdl(kernels[masked][0][f16], dim3(grid), dim3(attndb::THREADS), attndb::SMEM_BYTES, stream, tq, tk, tv, p);
         if (e != cudaSuccess) return cuda_fail(e, "cmt_cross_attn_fwd(tcgen05) launch");
     }
     CMT_LAUNCH_CHECK("cmt_cross_attn_fwd(tcgen05)");
     const long long mblocks = static_cast<long long>(a.B) * a.H * p.qblocks * (p.qblk / 32);
     CMT_CHECK_ARG(mblocks < (1ll << 31), "cmt_cross_attn_fwd: too many merge blocks");
-    if (a.o_bf16)
-        launch_pdl(tc_attn_merge_kernel<true>, dim3(static_cast<int>(mblocks)), dim3(256), 0, stream, p, G, a.o, a.lse);
+    if (a.o_dtype == CMT_BF16)
+        launch_pdl(tc_attn_merge_kernel<CMT_BF16>, dim3(static_cast<int>(mblocks)), dim3(256), 0, stream, p, G, a.o, a.lse);
+    else if (a.o_dtype == CMT_F16)
+        launch_pdl(tc_attn_merge_kernel<CMT_F16>, dim3(static_cast<int>(mblocks)), dim3(256), 0, stream, p, G, a.o, a.lse);
     else
-        launch_pdl(tc_attn_merge_kernel<false>, dim3(static_cast<int>(mblocks)), dim3(256), 0, stream, p, G, a.o, a.lse);
+        launch_pdl(tc_attn_merge_kernel<CMT_F32>, dim3(static_cast<int>(mblocks)), dim3(256), 0, stream, p, G, a.o, a.lse);
     CMT_LAUNCH_CHECK("cmt_cross_attn_fwd(merge)");
     return CMT_OK;
 }

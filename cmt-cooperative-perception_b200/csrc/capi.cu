@@ -76,11 +76,6 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 static EncodeTiledFn g_encode = nullptr;
 static std::once_flag g_encode_once;
 
-int encode_tma_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
-                    const uint64_t* strides_bytes, const uint32_t* box, int swizzle_bytes) {
-    return encode_tma(map, base, CMT_BF16, rank, dims, strides_bytes, box, swizzle_bytes);
-}
-
 int encode_tma(CUtensorMap* map, const void* base, int dtype, int rank, const uint64_t* dims,
                const uint64_t* strides_bytes, const uint32_t* box, int swizzle_bytes) {
     std::call_once(g_encode_once, []() {
@@ -108,7 +103,9 @@ int encode_tma(CUtensorMap* map, const void* base, int dtype, int rank, const ui
                                   : swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
                                   : swizzle_bytes == 32 ? CU_TENSOR_MAP_SWIZZLE_32B
                                                         : CU_TENSOR_MAP_SWIZZLE_NONE;
-    const CUtensorMapDataType dt = dtype == CMT_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    const CUtensorMapDataType dt = dtype == CMT_F32   ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
+                                   : dtype == CMT_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                                                      : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
     CUresult r = g_encode(map, dt, static_cast<cuuint32_t>(rank),
                           const_cast<void*>(base), gdims, gstrides, gbox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -133,7 +130,7 @@ using namespace cmt;
 
 extern "C" {
 
-int cmt_version(void) { return 100; }
+int cmt_version(void) { return 101; }
 
 const char* cmt_last_error_string(void) { return g_err; }
 
@@ -195,8 +192,11 @@ int cmt_gemm_bias_act(const void* A, const void* B, const float* bias, void* C, 
     CMT_CHECK_ARG(M > 0 && N > 0 && K > 0 && batch > 0, "cmt_gemm_bias_act: bad shape M=%d N=%d K=%d batch=%d", M,
                   N, K, batch);
     CMT_CHECK_ARG(lda >= K && ldb >= K && cb > 0, "cmt_gemm_bias_act: bad leading dimensions");
-    CMT_CHECK_ARG(in_dtype == CMT_F32 || in_dtype == CMT_BF16, "cmt_gemm_bias_act: bad in_dtype");
-    CMT_CHECK_ARG(out_dtype == CMT_F32 || out_dtype == CMT_BF16, "cmt_gemm_bias_act: bad out_dtype");
+    CMT_CHECK_ARG(in_dtype == CMT_F32 || in_dtype == CMT_BF16 || in_dtype == CMT_F16, "cmt_gemm_bias_act: bad in_dtype");
+    CMT_CHECK_ARG(out_dtype == CMT_F32 || out_dtype == CMT_BF16 || out_dtype == CMT_F16, "cmt_gemm_bias_act: bad out_dtype");
+    CMT_CHECK_ARG(in_dtype == CMT_F16 ? out_dtype != CMT_BF16 : out_dtype != CMT_F16,
+                  "cmt_gemm_bias_act: fp16 operands take an fp16 or fp32 output, and an fp16 output needs fp16 operands");
+    CMT_CHECK_ARG(in_dtype != CMT_F16 || !(flags & CMT_GEMM_FORCE_SIMT), "cmt_gemm_bias_act: fp16 operands run on the tensor cores only");
     GemmArgs g{};
     g.A = A;
     g.B = B;
@@ -216,15 +216,15 @@ int cmt_gemm_bias_act(const void* A, const void* B, const float* bias, void* C, 
     g.alpha = alpha;
     g.relu = (flags & CMT_GEMM_RELU) ? 1 : 0;
     g.bias_per_row = (flags & CMT_GEMM_BIAS_PER_ROW) ? 1 : 0;
-    g.out_bf16 = out_dtype == CMT_BF16;
+    g.out_16 = out_dtype != CMT_F32;
+    g.f16 = in_dtype == CMT_F16;
     g.transpose_c = (flags & CMT_GEMM_TRANSPOSE_OUT) ? 1 : 0;
     g.norm2_max = norm2_max;
-    CMT_CHECK_ARG(norm2_max == nullptr || (in_dtype == CMT_BF16 && !(flags & CMT_GEMM_FORCE_SIMT)),
-                  "cmt_gemm_bias_act: norm2_max is a bf16 tensor-core path option");
-    CMT_CHECK_ARG(!g.transpose_c || (in_dtype == CMT_BF16 && !(flags & CMT_GEMM_FORCE_SIMT)),
-                  "cmt_gemm_bias_act: CMT_GEMM_TRANSPOSE_OUT is a bf16 tensor-core path option");
+    const bool tc = in_dtype != CMT_F32 && !(flags & CMT_GEMM_FORCE_SIMT);
+    CMT_CHECK_ARG(norm2_max == nullptr || tc, "cmt_gemm_bias_act: norm2_max is a 16-bit tensor-core path option");
+    CMT_CHECK_ARG(!g.transpose_c || tc, "cmt_gemm_bias_act: CMT_GEMM_TRANSPOSE_OUT is a 16-bit tensor-core path option");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (in_dtype == CMT_BF16 && !(flags & CMT_GEMM_FORCE_SIMT)) return launch_tc_gemm(g, batch, s);
+    if (tc) return launch_tc_gemm(g, batch, s);
     return launch_simt_gemm(g, batch, in_dtype, s);
 }
 
@@ -256,7 +256,7 @@ int cmt_gemm_segmented(const void* A, const void* B, const float* bias, void* C,
     g.alpha = alpha;
     g.relu = (flags & CMT_GEMM_RELU) ? 1 : 0;
     g.bias_per_row = (flags & CMT_GEMM_BIAS_PER_ROW) ? 1 : 0;
-    g.out_bf16 = out_dtype == CMT_BF16;
+    g.out_16 = out_dtype == CMT_BF16;
     g.n_seg = n_seg;
     g.seg_k = seg_k;
     g.a_row_off = a_row_off;
@@ -272,16 +272,18 @@ int cmt_gemm_segmented(const void* A, const void* B, const float* bias, void* C,
     return launch_tc_gemm(g, batch, static_cast<cudaStream_t>(stream));
 }
 
-int cmt_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, int W, int guard_rows, int in_dtype, void* stream) {
+int cmt_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, int W, int guard_rows, int in_dtype, void* stream,
+                            int out_dtype) {
     CMT_REQUIRE_DEVICE();
-    return launch_nchw_to_padded_nhwc(x, out, B, C, H, W, guard_rows, in_dtype, static_cast<cudaStream_t>(stream));
+    return launch_nchw_to_padded_nhwc(x, out, B, C, H, W, guard_rows, in_dtype, out_dtype, static_cast<cudaStream_t>(stream));
 }
 
 int cmt_shared_conv_tokens(const void* xp, const void* w, const float* bias, const float* bev_pos, void* xk, void* xv, int B,
                            int Cin, int Cout, int H, int W, int guard_rows, int64_t out_frame_stride, int tok_begin, int tok_end,
-                           void* stream) {
+                           void* stream, int dtype) {
     CMT_REQUIRE_DEVICE();
     CMT_CHECK_ARG(xp && w && bias && bev_pos && xk && xv, "cmt_shared_conv_tokens: null pointer");
+    CMT_CHECK_ARG(dtype == CMT_BF16 || dtype == CMT_F16, "cmt_shared_conv_tokens: bad dtype");
     CMT_CHECK_ARG(B > 0 && Cin > 0 && Cin % 64 == 0 && Cout > 0 && Cout % 32 == 0 && H > 0 && W > 0 && guard_rows >= W + 3,
                   "cmt_shared_conv_tokens: bad shape (Cin %% 64, Cout %% 32, guard_rows >= W + 3)");
     CMT_CHECK_ARG(0 <= tok_begin && tok_begin < tok_end && tok_end <= H * W, "cmt_shared_conv_tokens: bad token range");
@@ -304,7 +306,8 @@ int cmt_shared_conv_tokens(const void* xp, const void* w, const float* bias, con
     g.strideC = 0;
     g.alpha = 1.0f;
     g.relu = 1;
-    g.out_bf16 = 1;
+    g.out_16 = 1;
+    g.f16 = dtype == CMT_F16;
     g.n_seg = 9;
     g.seg_k = Cin;
     g.a_row_off = guard_rows;
@@ -341,8 +344,10 @@ int cmt_cross_attn_fwd(const void* q, const void* k, const void* vt, void* o, fl
     CMT_CHECK_ARG(B > 0 && H > 0 && Nq > 0 && N_kv > 0, "cmt_cross_attn_fwd: bad shape");
     CMT_CHECK_ARG(0 <= kv_begin && kv_begin < kv_end && kv_end <= N_kv,
                   "cmt_cross_attn_fwd: bad token range [%d,%d) of %d", kv_begin, kv_end, N_kv);
-    CMT_CHECK_ARG(dtype == CMT_F32 || dtype == CMT_BF16 || dtype == CMT_BF16_SIMT, "cmt_cross_attn_fwd: bad dtype");
-    CMT_CHECK_ARG(o_dtype == CMT_F32 || o_dtype == CMT_BF16, "cmt_cross_attn_fwd: bad o_dtype");
+    CMT_CHECK_ARG(dtype == CMT_F32 || dtype == CMT_BF16 || dtype == CMT_F16 || dtype == CMT_BF16_SIMT,
+                  "cmt_cross_attn_fwd: bad dtype");
+    CMT_CHECK_ARG(o_dtype == CMT_F32 || o_dtype == CMT_BF16 || o_dtype == CMT_F16, "cmt_cross_attn_fwd: bad o_dtype");
+    CMT_CHECK_ARG(o_dtype != CMT_F16 || dtype == CMT_F16, "cmt_cross_attn_fwd: an fp16 output needs fp16 operands");
     CMT_CHECK_ARG(q_ld >= H * 32 && v_ld >= kv_end, "cmt_cross_attn_fwd: bad leading dimensions");
     AttnArgs a{};
     a.q = q;
@@ -362,13 +367,14 @@ int cmt_cross_attn_fwd(const void* q, const void* k, const void* vt, void* o, fl
     a.v_bstride = v_bstride;
     a.v_hstride = v_hstride;
     a.v_ld = v_ld;
-    a.o_bf16 = o_dtype == CMT_BF16;
+    a.f16 = dtype == CMT_F16;
+    a.o_dtype = o_dtype;
     a.key_keep = key_keep;
     a.q_norm2 = q_norm2_max;
     a.k_norm2 = k_norm2_max;
     a.kn_bstride = kn_bstride;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (dtype == CMT_BF16) return launch_tc_attn(a, workspace, workspace_bytes, s);
+    if (dtype == CMT_BF16 || dtype == CMT_F16) return launch_tc_attn(a, workspace, workspace_bytes, s);
     return launch_simt_attn(a, dtype == CMT_BF16_SIMT ? CMT_BF16 : dtype, s);
 }
 

@@ -4,6 +4,7 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <cstdlib>
 #include <stdint.h>
@@ -53,10 +54,7 @@ struct DeviceOnce {
 
 // Driver entry point for cuTensorMapEncodeTiled, fetched once through the runtime
 // (no link-time dependency on libcuda).
-int encode_tma_bf16(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
-                    const uint64_t* strides_bytes /* rank-1 */, const uint32_t* box,
-                    int swizzle_bytes /* 64 or 128 */);
-// general form: dtype CMT_F32 | CMT_BF16, swizzle_bytes 0 (none) | 32 | 64 | 128
+// dtype CMT_F32 | CMT_BF16 | CMT_F16, strides_bytes: rank - 1 entries, swizzle_bytes 0 (none) | 32 | 64 | 128
 int encode_tma(CUtensorMap* map, const void* base, int dtype, int rank, const uint64_t* dims,
                const uint64_t* strides_bytes, const uint32_t* box, int swizzle_bytes);
 
@@ -71,6 +69,29 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     uint32_t r;
     asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
     return r;
+}
+
+__device__ __forceinline__ uint32_t pack_f16x2(float lo, float hi) {
+    uint32_t r;
+    asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    return r;
+}
+
+// Two values rounded to the 16-bit compute dtype kLp (CMT_F16, else bf16) in one word, `lo` in the low half.
+template <int kLp>
+__device__ __forceinline__ uint32_t pack_lp2(float lo, float hi) {
+    return kLp == CMT_F16 ? pack_f16x2(lo, hi) : pack_bf16x2(lo, hi);
+}
+// One value of the 16-bit dtype kLp (CMT_F16, else bf16): element i of `base`.
+template <int kLp>
+__device__ __forceinline__ void store_lp(void* base, long long i, float v) {
+    if (kLp == CMT_F16) reinterpret_cast<__half*>(base)[i] = __float2half_rn(v);
+    else reinterpret_cast<__nv_bfloat16*>(base)[i] = __float2bfloat16_rn(v);
+}
+template <int kLp>
+__device__ __forceinline__ float load_lp(const void* base, long long i) {
+    if (kLp == CMT_F16) return __half2float(reinterpret_cast<const __half*>(base)[i]);
+    return __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(base)[i]);
 }
 
 __device__ __forceinline__ float ex2_approx(float x) {
@@ -376,9 +397,9 @@ __device__ __forceinline__ uint64_t make_kmajor_desc(uint32_t smem_addr, int swi
     return d;
 }
 
-// Instruction descriptor: kind::f16, A=B=bf16, D=fp32, both operands K-major.
-__host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(N >> 3) << 17) |
+// Instruction descriptor: kind::f16, D=fp32, both operands K-major; A=B=bf16 (a/b format 1), or fp16 (format 0).
+__host__ __device__ constexpr uint32_t make_idesc(int M, int N, bool fp16) {
+    return (1u << 4) | (fp16 ? 0u : (1u << 7) | (1u << 10)) | (static_cast<uint32_t>(N >> 3) << 17) |
            (static_cast<uint32_t>(M >> 4) << 24);
 }
 

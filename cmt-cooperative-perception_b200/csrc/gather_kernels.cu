@@ -44,7 +44,8 @@ __device__ __forceinline__ void unpack_feat2(uint32_t w, float& lo, float& hi) {
     }
 }
 
-template <bool kBf16, int kIn>
+// kOut: dtype of xk / xv, CMT_F32 | CMT_BF16 | CMT_F16.
+template <int kOut, int kIn>
 __global__ void __launch_bounds__(256) gather_tokens_kernel(
     const void* __restrict__ x_bev, const void* __restrict__ x_img,
     const float* __restrict__ bev_pos, const float* __restrict__ rv_pos, void* __restrict__ xk,
@@ -110,9 +111,9 @@ __global__ void __launch_bounds__(256) gather_tokens_kernel(
         for (int c = lane * 2; c < C; c += 64) {
             const float m0 = trow[c], m1 = trow[c + 1];
             const float2 pp = *reinterpret_cast<const float2*>(prow + c);
-            if (kBf16) {
-                reinterpret_cast<uint32_t*>(xk)[(drow + c) >> 1] = pack_bf16x2(m0 + pp.x, m1 + pp.y);
-                reinterpret_cast<uint32_t*>(xv)[(drow + c) >> 1] = pack_bf16x2(m0, m1);
+            if (kOut != CMT_F32) {
+                reinterpret_cast<uint32_t*>(xk)[(drow + c) >> 1] = pack_lp2<kOut>(m0 + pp.x, m1 + pp.y);
+                reinterpret_cast<uint32_t*>(xv)[(drow + c) >> 1] = pack_lp2<kOut>(m0, m1);
             } else {
                 *reinterpret_cast<float2*>(reinterpret_cast<float*>(xk) + drow + c) =
                     make_float2(m0 + pp.x, m1 + pp.y);
@@ -132,7 +133,7 @@ int launch_gather_tokens(const void* x_bev, const void* x_img, const float* bev_
     CMT_CHECK_ARG(n_bev >= 0 && V >= 0 && n_img >= 0, "cmt_gather_tokens: bad token counts");
     CMT_CHECK_ARG(n_bev == 0 || x_bev == nullptr || bev_pos, "cmt_gather_tokens: BEV position encoding missing");
     CMT_CHECK_ARG(V == 0 || n_img == 0 || (x_img && rv_pos), "cmt_gather_tokens: image pointers missing");
-    CMT_CHECK_ARG(out_dtype == CMT_F32 || out_dtype == CMT_BF16, "cmt_gather_tokens: bad output dtype");
+    CMT_CHECK_ARG(out_dtype == CMT_F32 || out_dtype == CMT_BF16 || out_dtype == CMT_F16, "cmt_gather_tokens: bad output dtype");
     CMT_CHECK_ARG(feat_dtype == CMT_F32 || feat_dtype == CMT_BF16 || feat_dtype == CMT_F16, "cmt_gather_tokens: bad feature dtype");
     CMT_CHECK_ARG(B <= 65535, "cmt_gather_tokens: batch too large for one launch");
     const long long n_kv = n_bev + static_cast<long long>(V) * n_img;
@@ -160,26 +161,32 @@ int launch_gather_tokens(const void* x_bev, const void* x_img, const float* bev_
     const size_t smem = static_cast<size_t>(kTileTok) * (C + 1) * sizeof(float);
     CMT_CHECK_ARG(smem <= 48 * 1024, "cmt_gather_tokens: C too large (%d)", C);
     dim3 grid(tiles, B);
-#define CMT_GATHER_LAUNCH(OUT_BF16, IN)                                                                       \
-    gather_tokens_kernel<OUT_BF16, IN><<<grid, 256, smem, stream>>>(x_bev, x_img, bev_pos, rv_pos, xk, xv, C, n_bev, V, \
-                                                                    n_img, tiles_bev, tiles_img, tok_begin, tok_end, rv_tok0, rv_rows)
-    const bool ob = out_dtype == CMT_BF16;
-    if (feat_dtype == CMT_F32) { if (ob) CMT_GATHER_LAUNCH(true, CMT_F32); else CMT_GATHER_LAUNCH(false, CMT_F32); }
-    else if (feat_dtype == CMT_BF16) { if (ob) CMT_GATHER_LAUNCH(true, CMT_BF16); else CMT_GATHER_LAUNCH(false, CMT_BF16); }
-    else { if (ob) CMT_GATHER_LAUNCH(true, CMT_F16); else CMT_GATHER_LAUNCH(false, CMT_F16); }
+#define CMT_GATHER_LAUNCH(OUT, IN)                                                                            \
+    gather_tokens_kernel<OUT, IN><<<grid, 256, smem, stream>>>(x_bev, x_img, bev_pos, rv_pos, xk, xv, C, n_bev, V, \
+                                                               n_img, tiles_bev, tiles_img, tok_begin, tok_end, rv_tok0, rv_rows)
+#define CMT_GATHER_LAUNCH_OUT(IN)                                                                             \
+    do {                                                                                                      \
+        if (out_dtype == CMT_BF16) CMT_GATHER_LAUNCH(CMT_BF16, IN);                                          \
+        else if (out_dtype == CMT_F16) CMT_GATHER_LAUNCH(CMT_F16, IN);                                       \
+        else CMT_GATHER_LAUNCH(CMT_F32, IN);                                                                 \
+    } while (0)
+    if (feat_dtype == CMT_F32) CMT_GATHER_LAUNCH_OUT(CMT_F32);
+    else if (feat_dtype == CMT_BF16) CMT_GATHER_LAUNCH_OUT(CMT_BF16);
+    else CMT_GATHER_LAUNCH_OUT(CMT_F16);
+#undef CMT_GATHER_LAUNCH_OUT
 #undef CMT_GATHER_LAUNCH
     CMT_LAUNCH_CHECK("cmt_gather_tokens");
     return CMT_OK;
 }
 
 // ---------------------------------------------------------------------------
-// NCHW feature map -> zero-padded, channel-last bf16 rows: the A operand of the 3x3 shared_conv implicit GEMM
+// NCHW feature map -> zero-padded, channel-last 16-bit rows (kOut = CMT_BF16 | CMT_F16): the A operand of the 3x3 shared_conv implicit GEMM
 // (cmt_head.py:280-287,481).  Frame b occupies `rows_per_frame = 2 * guard + (H + 2) * (W + 2)` rows of C channels; pixel
 // (y, x) lands in row guard + (y + 1) * (W + 2) + (x + 1).  Only interior rows are written: the border and guard rows
 // are zero from the (one-time) allocation, so a filter tap is a pure row shift of -(W+2)-1 .. +(W+2)+1 with no edge
 // handling.  Block = 32 consecutive pixels x one block of up to 256 channels, same transpose tile as the token gather.
-template <int kIn>
-__global__ void __launch_bounds__(256) nchw_to_padded_nhwc_kernel(const void* __restrict__ x, __nv_bfloat16* __restrict__ out,
+template <int kIn, int kOut>
+__global__ void __launch_bounds__(256) nchw_to_padded_nhwc_kernel(const void* __restrict__ x, uint16_t* __restrict__ out,
                                                                   int C, int H, int W, int guard, long long rows_per_frame) {
     extern __shared__ float tile[];  // [32][257]
     constexpr int ESZ = kIn == CMT_F32 ? 4 : 2;
@@ -214,24 +221,31 @@ __global__ void __launch_bounds__(256) nchw_to_padded_nhwc_kernel(const void* __
         const long long row = static_cast<long long>(b) * rows_per_frame + guard + static_cast<long long>(y + 1) * (W + 2) + (xx + 1);
         uint32_t* dst = reinterpret_cast<uint32_t*>(out + row * C + c0);
         const float* trow = tile + r * pitch;
-        for (int c = lane * 2; c < nc; c += 64) dst[c >> 1] = pack_bf16x2(trow[c], trow[c + 1]);
+        for (int c = lane * 2; c < nc; c += 64) dst[c >> 1] = pack_lp2<kOut>(trow[c], trow[c + 1]);
     }
 }
 
 int launch_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, int W, int guard, int in_dtype,
-                               cudaStream_t stream) {
+                               int out_dtype, cudaStream_t stream) {
     CMT_CHECK_ARG(x && out && B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0 && guard >= W + 3,
                   "cmt_nchw_to_padded_nhwc: bad arguments (guard must be >= W + 3)");
     CMT_CHECK_ARG(in_dtype == CMT_F32 || in_dtype == CMT_BF16 || in_dtype == CMT_F16, "cmt_nchw_to_padded_nhwc: bad dtype");
+    CMT_CHECK_ARG(out_dtype == CMT_BF16 || out_dtype == CMT_F16, "cmt_nchw_to_padded_nhwc: bad output dtype");
     CMT_CHECK_ARG(B <= 65535, "cmt_nchw_to_padded_nhwc: batch too large");
     CMT_CHECK_ARG(in_dtype == CMT_F32 || (reinterpret_cast<uintptr_t>(x) & 3) == 0, "cmt_nchw_to_padded_nhwc: unaligned input");
     const long long rows = 2ll * guard + static_cast<long long>(H + 2) * (W + 2);
     dim3 grid((H * W + kTileTok - 1) / kTileTok, B, (C + 255) / 256);
     const size_t smem = static_cast<size_t>(kTileTok) * 257 * sizeof(float);
-    __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out);
-    if (in_dtype == CMT_F32) nchw_to_padded_nhwc_kernel<CMT_F32><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
-    else if (in_dtype == CMT_BF16) nchw_to_padded_nhwc_kernel<CMT_BF16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
-    else nchw_to_padded_nhwc_kernel<CMT_F16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
+    uint16_t* o = reinterpret_cast<uint16_t*>(out);
+    if (out_dtype == CMT_BF16) {
+        if (in_dtype == CMT_F32) nchw_to_padded_nhwc_kernel<CMT_F32, CMT_BF16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
+        else if (in_dtype == CMT_BF16) nchw_to_padded_nhwc_kernel<CMT_BF16, CMT_BF16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
+        else nchw_to_padded_nhwc_kernel<CMT_F16, CMT_BF16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
+    } else {
+        if (in_dtype == CMT_F32) nchw_to_padded_nhwc_kernel<CMT_F32, CMT_F16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
+        else if (in_dtype == CMT_BF16) nchw_to_padded_nhwc_kernel<CMT_BF16, CMT_F16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
+        else nchw_to_padded_nhwc_kernel<CMT_F16, CMT_F16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
+    }
     CMT_LAUNCH_CHECK("cmt_nchw_to_padded_nhwc");
     return CMT_OK;
 }
@@ -281,8 +295,8 @@ int launch_coop_max(const float* a, const float* b, float* out, long long n, cud
 }
 
 // ---------------------------------------------------------------------------
-// o = sum_g exp(lse_g - lse) * o_g ,  lse = log(sum_g exp(lse_g)).  One thread per (b, n, h, 4 dims).
-template <bool kBf16>
+// o = sum_g exp(lse_g - lse) * o_g ,  lse = log(sum_g exp(lse_g)).  One thread per (b, n, h, 4 dims).  kOut: dtype of o.
+template <int kOut>
 __global__ void __launch_bounds__(256) lse_merge_kernel(const float* __restrict__ o_parts,
                                                         const float* __restrict__ lse_parts,
                                                         void* __restrict__ o,
@@ -312,10 +326,10 @@ __global__ void __launch_bounds__(256) lse_merge_kernel(const float* __restrict_
         }
         const float inv = den > 0.0f ? 1.0f / den : 0.0f;
         acc.x *= inv; acc.y *= inv; acc.z *= inv; acc.w *= inv;
-        if (kBf16) {
+        if (kOut != CMT_F32) {
             uint2 w;
-            w.x = pack_bf16x2(acc.x, acc.y);
-            w.y = pack_bf16x2(acc.z, acc.w);
+            w.x = pack_lp2<kOut>(acc.x, acc.y);
+            w.y = pack_lp2<kOut>(acc.z, acc.w);
             reinterpret_cast<uint2*>(o)[t] = w;
         } else {
             reinterpret_cast<float4*>(o)[t] = acc;
@@ -336,11 +350,14 @@ int launch_lse_merge(const float* o_parts, const float* lse_parts, void* o, floa
     const long long cap = static_cast<long long>(device_sm_count()) * 16;
     if (blocks > cap) blocks = cap;
     if (o_dtype == CMT_BF16)
-        lse_merge_kernel<true><<<static_cast<int>(blocks), 256, 0, stream>>>(o_parts, lse_parts, o,
-                                                                            lse, G, B, H, Nq, o_gstride, lse_gstride);
+        lse_merge_kernel<CMT_BF16><<<static_cast<int>(blocks), 256, 0, stream>>>(o_parts, lse_parts, o,
+                                                                                lse, G, B, H, Nq, o_gstride, lse_gstride);
+    else if (o_dtype == CMT_F16)
+        lse_merge_kernel<CMT_F16><<<static_cast<int>(blocks), 256, 0, stream>>>(o_parts, lse_parts, o,
+                                                                               lse, G, B, H, Nq, o_gstride, lse_gstride);
     else if (o_dtype == CMT_F32)
-        lse_merge_kernel<false><<<static_cast<int>(blocks), 256, 0, stream>>>(o_parts, lse_parts, o,
-                                                                             lse, G, B, H, Nq, o_gstride, lse_gstride);
+        lse_merge_kernel<CMT_F32><<<static_cast<int>(blocks), 256, 0, stream>>>(o_parts, lse_parts, o,
+                                                                               lse, G, B, H, Nq, o_gstride, lse_gstride);
     else
         CMT_CHECK_ARG(false, "cmt_lse_merge: bad dtype");
     CMT_LAUNCH_CHECK("cmt_lse_merge");
@@ -406,8 +423,8 @@ __device__ __forceinline__ void peer_wait(const unsigned int* flag, unsigned int
 }
 
 // kScatter = false (small groups): every rank merges ALL rows from the G records (G - 1 records over NVLink) into its own
-// context buffer; steps 3b / 4 disappear and the exchange costs one handshake instead of two.
-template <bool kBf16, bool kScatter>
+// context buffer; steps 3b / 4 disappear and the exchange costs one handshake instead of two.  kOut: context dtype.
+template <int kOut, bool kScatter>
 __global__ void __launch_bounds__(256) lse_merge_peer_kernel(const PeerMergeParams p) {
     __shared__ unsigned int seq_s;
     __shared__ int last_s;
@@ -459,10 +476,10 @@ __global__ void __launch_bounds__(256) lse_merge_peer_kernel(const PeerMergePara
         }
         const float inv = den > 0.0f ? 1.0f / den : 0.0f;
         acc.x *= inv; acc.y *= inv; acc.z *= inv; acc.w *= inv;
-        if (kBf16) {
+        if (kOut != CMT_F32) {
             uint2 w;
-            w.x = pack_bf16x2(acc.x, acc.y);
-            w.y = pack_bf16x2(acc.z, acc.w);
+            w.x = pack_lp2<kOut>(acc.x, acc.y);
+            w.y = pack_lp2<kOut>(acc.z, acc.w);
             if (!kScatter) {
                 reinterpret_cast<uint2*>(p.ctx[0])[t] = w;
             } else {
@@ -505,7 +522,7 @@ int launch_lse_merge_peer(const void* const* records, void* const* ctx, void* co
     CMT_CHECK_ARG(records && ctx && arrive && state, "cmt_lse_merge_peer: null pointer");
     CMT_CHECK_ARG(G > 0 && G <= MAX_PEERS && rank >= 0 && rank < G, "cmt_lse_merge_peer: 1 <= G <= 8, 0 <= rank < G");
     CMT_CHECK_ARG(B > 0 && H > 0 && Nq > 0, "cmt_lse_merge_peer: bad shape");
-    CMT_CHECK_ARG(o_dtype == CMT_BF16 || o_dtype == CMT_F32, "cmt_lse_merge_peer: bad dtype");
+    CMT_CHECK_ARG(o_dtype == CMT_BF16 || o_dtype == CMT_F16 || o_dtype == CMT_F32, "cmt_lse_merge_peer: bad dtype");
     PeerMergeParams p{};
     for (int g = 0; g < G; ++g) {
         CMT_CHECK_ARG(records[g] && arrive[g] && ctx[g] && (reinterpret_cast<uintptr_t>(records[g]) & 15) == 0 &&
@@ -535,11 +552,14 @@ int launch_lse_merge_peer(const void* const* records, void* const* ctx, void* co
     if (blocks < 1) blocks = 1;   // a rank without rows still takes part in the handshakes
     const int nb = static_cast<int>(blocks);
     if (o_dtype == CMT_BF16) {
-        if (scatter) lse_merge_peer_kernel<true, true><<<nb, 256, 0, stream>>>(p);
-        else lse_merge_peer_kernel<true, false><<<nb, 256, 0, stream>>>(p);
+        if (scatter) lse_merge_peer_kernel<CMT_BF16, true><<<nb, 256, 0, stream>>>(p);
+        else lse_merge_peer_kernel<CMT_BF16, false><<<nb, 256, 0, stream>>>(p);
+    } else if (o_dtype == CMT_F16) {
+        if (scatter) lse_merge_peer_kernel<CMT_F16, true><<<nb, 256, 0, stream>>>(p);
+        else lse_merge_peer_kernel<CMT_F16, false><<<nb, 256, 0, stream>>>(p);
     } else {
-        if (scatter) lse_merge_peer_kernel<false, true><<<nb, 256, 0, stream>>>(p);
-        else lse_merge_peer_kernel<false, false><<<nb, 256, 0, stream>>>(p);
+        if (scatter) lse_merge_peer_kernel<CMT_F32, true><<<nb, 256, 0, stream>>>(p);
+        else lse_merge_peer_kernel<CMT_F32, false><<<nb, 256, 0, stream>>>(p);
     }
     CMT_LAUNCH_CHECK("cmt_lse_merge_peer");
     return CMT_OK;

@@ -1,6 +1,6 @@
 // K2: projection / MLP GEMM on the 5th-gen tensor cores.
 //
-//   C = act((A * B^T + bias) * alpha),  A:[M,K] bf16, B:[N,K] bf16 (both K-major), fp32 accumulate.
+//   C = act((A * B^T + bias) * alpha),  A:[M,K], B:[N,K] both bf16 or both fp16 (K-major), fp32 accumulate.
 //
 // Persistent, warp-specialised kernel, one CTA per SM:
 //   warp 0      TMA producer  : 3-D tensor maps (K, rows, batch), 128B swizzle.  Streaming mode: 4-stage ring of
@@ -10,7 +10,7 @@
 //                               M=128 x N=256 x K=16 per instruction, accumulator in TMEM
 //   warp 2      TMEM allocator (512 columns = two 128x256 fp32 accumulators, ping-pong)
 //   warps 4..11 epilogue      : one loop for every output layout: tcgen05.ld 32x32b -> bias (cached in shared memory,
-//                               or per row) / alpha / ReLU -> bf16|fp32 -> global stores straight from registers (a
+//                               or per row) / alpha / ReLU -> bf16|fp16|fp32 -> global stores straight from registers (a
 //                               thread owns 32 consecutive columns of one row: 64 / 128 contiguous bytes), overlapped
 //                               with the next tile's main loop.  Store form (one instantiation each): 256-bit where the
 //                               layout is 32-byte aligned, masked scalar, transposed for V^T, or the shared_conv token
@@ -67,19 +67,21 @@ enum class Store {
     Vec,          // row-major, 32-byte aligned layout, N % 32 == 0, no column bias too wide for the cache: 256-bit stores
     Masked,       // row-major otherwise: 256-bit stores for the full chunks of an aligned layout, masked scalar stores else;
                   // the only form that reads a column bias too wide for the cache
-    Transposed,   // C^T inside each column block (V^T), bf16
+    Transposed,   // C^T inside each column block (V^T), 16-bit
     Conv,         // shared_conv token pair xv / xk
 };
 
-// 32 consecutive outputs of one row as 256-bit stores (dst 32-byte aligned): bf16, 64 bytes / fp32, 128 bytes
-__device__ __forceinline__ void st_bf16x32(uint8_t* dst, const float (&f)[32]) {
+// 32 consecutive outputs of one row as 256-bit stores (dst 32-byte aligned): 16-bit (kLp = CMT_BF16 | CMT_F16), 64 bytes /
+// fp32, 128 bytes
+template <int kLp>
+__device__ __forceinline__ void st_lp16x32(uint8_t* dst, const float (&f)[32]) {
 #pragma unroll
     for (int i = 0; i < 2; ++i)
         asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst + 32 * i),
-                     "r"(pack_bf16x2(f[16 * i + 0], f[16 * i + 1])), "r"(pack_bf16x2(f[16 * i + 2], f[16 * i + 3])),
-                     "r"(pack_bf16x2(f[16 * i + 4], f[16 * i + 5])), "r"(pack_bf16x2(f[16 * i + 6], f[16 * i + 7])),
-                     "r"(pack_bf16x2(f[16 * i + 8], f[16 * i + 9])), "r"(pack_bf16x2(f[16 * i + 10], f[16 * i + 11])),
-                     "r"(pack_bf16x2(f[16 * i + 12], f[16 * i + 13])), "r"(pack_bf16x2(f[16 * i + 14], f[16 * i + 15]))
+                     "r"(pack_lp2<kLp>(f[16 * i + 0], f[16 * i + 1])), "r"(pack_lp2<kLp>(f[16 * i + 2], f[16 * i + 3])),
+                     "r"(pack_lp2<kLp>(f[16 * i + 4], f[16 * i + 5])), "r"(pack_lp2<kLp>(f[16 * i + 6], f[16 * i + 7])),
+                     "r"(pack_lp2<kLp>(f[16 * i + 8], f[16 * i + 9])), "r"(pack_lp2<kLp>(f[16 * i + 10], f[16 * i + 11])),
+                     "r"(pack_lp2<kLp>(f[16 * i + 12], f[16 * i + 13])), "r"(pack_lp2<kLp>(f[16 * i + 14], f[16 * i + 15]))
                      : "memory");
 }
 
@@ -128,11 +130,14 @@ struct TileWalk {
     }
 };
 
-template <Store S>
+// kF16: fp16 operands and 16-bit outputs (g.f16), bf16 otherwise -- its own instantiations, so the bf16 kernels are
+// exactly what they were before fp16 existed.
+template <Store S, bool kF16>
 __global__ void __launch_bounds__(gemm::THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                const TcGemmParams p) {
     using namespace gemm;
+    constexpr int LP = kF16 ? CMT_F16 : CMT_BF16;
     const GemmArgs& g = p.g;
     pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
@@ -228,7 +233,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
         // ------------------------------ MMA issuer ------------------------------
         {
             const bool leader = elect_one();
-            constexpr uint32_t idesc = make_idesc_bf16(BM, BN);
+            constexpr uint32_t idesc = make_idesc(BM, BN, kF16);
             int stage = 0;
             uint32_t phase = 0;
             int acc = 0;
@@ -277,14 +282,14 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
         // one column, 64 contiguous bytes.
         // shared_conv tokens (cmt_head.py:280-287,481 + cmt_transformer.py:105-110 + petr_transformer.py:296-299 for the
         // BEV tokens: the NCHW fp32 map the reference writes and re-reads never exists): the thread's row is a padded
-        // position, stored as xv = bf16(ReLU(acc + bias)) and xk = bf16(that + pos), 64 contiguous bytes each.
+        // position, stored as xv = lp(ReLU(acc + bias)) and xk = lp(that + pos), 64 contiguous bytes each.
         const int quad = warp & 3;
         const int half = (warp - 4) >> 2;
         constexpr bool conv = S == Store::Conv;   // ReLU(acc + bias) with the bias cached (host checks), no alpha
         const bool col_bias = g.bias != nullptr && !g.bias_per_row;   // from bias_s when bias_cached, else from global
         const bool scale = !conv && g.alpha != 1.0f;
         const bool relu = conv || g.relu != 0;
-        const int esz = g.out_bf16 ? 2 : 4;
+        const int esz = g.out_16 ? 2 : 4;
         const uint32_t bias_addr = smem_u32(bias_s);
         int acc = 0;
         uint32_t acc_phase = 0;
@@ -367,28 +372,33 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
                     const long long blk_off = row_off + nb * g.cb_stride;
                     if (row_ok) {
                         if constexpr (conv) {
-                            st_bf16x32(reinterpret_cast<uint8_t*>(g.conv_xv) + (row_off + n0) * 2, f);
+                            st_lp16x32<LP>(reinterpret_cast<uint8_t*>(g.conv_xv) + (row_off + n0) * 2, f);
                             const float4* pp = reinterpret_cast<const float4*>(g.conv_pos + static_cast<long long>(tok) * g.N + n0);
 #pragma unroll
                             for (int i = 0; i < 8; ++i) {
                                 const float4 q = __ldg(pp + i);
                                 f[4 * i] += q.x; f[4 * i + 1] += q.y; f[4 * i + 2] += q.z; f[4 * i + 3] += q.w;
                             }
-                            st_bf16x32(reinterpret_cast<uint8_t*>(g.conv_xk) + (row_off + n0) * 2, f);
+                            st_lp16x32<LP>(reinterpret_cast<uint8_t*>(g.conv_xk) + (row_off + n0) * 2, f);
                         } else if constexpr (S == Store::Transposed) {
-                            // element (m, n) -> blk_off + (n % cb) * ldc + m  (bf16 only)
+                            // element (m, n) -> blk_off + (n % cb) * ldc + m  (16-bit only)
                             uint16_t* dst = reinterpret_cast<uint16_t*>(g.C) + blk_off + rem * g.ldc;
 #pragma unroll
                             for (int i = 0; i < 16; ++i) {
-                                const uint32_t w2 = pack_bf16x2(f[2 * i], f[2 * i + 1]);
+                                const uint32_t w2 = pack_lp2<LP>(f[2 * i], f[2 * i + 1]);
                                 dst[static_cast<long long>(2 * i) * g.ldc] = static_cast<uint16_t>(w2 & 0xffffu);
                                 dst[static_cast<long long>(2 * i + 1) * g.ldc] = static_cast<uint16_t>(w2 >> 16);
                             }
                         } else if (S == Store::Vec || (p.vec_store && n0 + 32 <= g.N)) {
                             uint8_t* dst = reinterpret_cast<uint8_t*>(g.C) + (blk_off + rem) * esz;
-                            if (g.out_bf16) st_bf16x32(dst, f);
+                            if (g.out_16) st_lp16x32<LP>(dst, f);
                             else st_f32x32(dst, f);
-                        } else if (g.out_bf16) {
+                        } else if (g.out_16 && kF16) {
+                            __half* dst = reinterpret_cast<__half*>(g.C) + blk_off + rem;
+#pragma unroll
+                            for (int i = 0; i < 32; ++i)
+                                if (n0 + i < g.N) dst[i] = __float2half_rn(f[i]);
+                        } else if (g.out_16) {
                             __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(g.C) + blk_off + rem;
 #pragma unroll
                             for (int i = 0; i < 32; ++i)
@@ -434,9 +444,11 @@ int launch_tc_gemm(const GemmArgs& g, int batch, cudaStream_t stream) {
                   "cmt_gemm_bias_act(bf16): column block must be >= N or a multiple of 32");
     CMT_CHECK_ARG(g.strideA % 8 == 0 && g.strideB % 8 == 0, "cmt_gemm_bias_act(bf16): batch strides must be multiples of 8");
 
-    // one instantiation per store form, in the order of Store
+    // one instantiation per store form, in the order of Store: bf16, then fp16
     static void (*const kernels[])(CUtensorMap, CUtensorMap, TcGemmParams) = {
-        tc_gemm_kernel<Store::Vec>, tc_gemm_kernel<Store::Masked>, tc_gemm_kernel<Store::Transposed>, tc_gemm_kernel<Store::Conv>};
+        tc_gemm_kernel<Store::Vec, false>, tc_gemm_kernel<Store::Masked, false>, tc_gemm_kernel<Store::Transposed, false>,
+        tc_gemm_kernel<Store::Conv, false>, tc_gemm_kernel<Store::Vec, true>, tc_gemm_kernel<Store::Masked, true>,
+        tc_gemm_kernel<Store::Transposed, true>, tc_gemm_kernel<Store::Conv, true>};
     static DeviceOnce attr_once;
     int attr_dev;
     if (attr_once.need(&attr_dev)) {
@@ -457,7 +469,7 @@ int launch_tc_gemm(const GemmArgs& g, int batch, cudaStream_t stream) {
         uint64_t strides[2] = {static_cast<uint64_t>(g.lda) * 2,
                                static_cast<uint64_t>(batched ? g.strideA : a_rows * g.lda) * 2};
         uint32_t box[3] = {BK, BM, 1};
-        int rc = encode_tma_bf16(&ta, g.A, 3, dims, strides, box, 128);
+        int rc = encode_tma(&ta, g.A, g.f16 ? CMT_F16 : CMT_BF16, 3, dims, strides, box, 128);
         if (rc) return rc;
     }
     {
@@ -467,11 +479,11 @@ int launch_tc_gemm(const GemmArgs& g, int batch, cudaStream_t stream) {
         uint64_t strides[2] = {static_cast<uint64_t>(g.ldb) * 2,
                                static_cast<uint64_t>(batched ? g.strideB : (long long)g.N * g.ldb) * 2};
         uint32_t box[3] = {BK, BN, 1};
-        int rc = encode_tma_bf16(&tb, g.B, 3, dims, strides, box, 128);
+        int rc = encode_tma(&tb, g.B, g.f16 ? CMT_F16 : CMT_BF16, 3, dims, strides, box, 128);
         if (rc) return rc;
     }
 
-    const int esz = g.out_bf16 ? 2 : 4;
+    const int esz = g.out_16 ? 2 : 4;
     const bool plain = g.cb >= g.N;
     if (g.conv_xv != nullptr)
         CMT_CHECK_ARG(g.conv_xk && g.conv_pos && g.bias && !g.bias_per_row && g.N % 32 == 0 && g.N <= BIAS_CAP - 64 &&
@@ -480,8 +492,8 @@ int launch_tc_gemm(const GemmArgs& g, int batch, cudaStream_t stream) {
                       "cmt_shared_conv_tokens: bias, pos, 32-byte aligned outputs and N %% 32 == 0 required");
     const bool bias_ok = g.bias == nullptr || g.bias_per_row || g.N <= BIAS_CAP - 64;
     if (g.transpose_c)
-        CMT_CHECK_ARG(g.out_bf16 && g.cb % 32 == 0 && g.N % 32 == 0 && bias_ok && !plain,
-                      "cmt_gemm_bias_act(bf16): transposed output needs bf16, cb %% 32 == 0, N %% 32 == 0, N <= %d", BIAS_CAP - 64);
+        CMT_CHECK_ARG(g.out_16 && g.cb % 32 == 0 && g.N % 32 == 0 && bias_ok && !plain,
+                      "cmt_gemm_bias_act(bf16): transposed output needs a 16-bit output, cb %% 32 == 0, N %% 32 == 0, N <= %d", BIAS_CAP - 64);
     const bool aligned = (reinterpret_cast<uintptr_t>(g.C) & 31) == 0 && (g.ldc * esz) % 32 == 0 &&
                          (plain || ((g.cb_stride * esz) % 32 == 0 && g.cb % 32 == 0)) &&
                          (batch == 1 || (g.strideC * esz) % 32 == 0);
@@ -523,7 +535,7 @@ int launch_tc_gemm(const GemmArgs& g, int batch, cudaStream_t stream) {
         grid = static_cast<int>(gm) * p.n_tiles;
     }
     {
-        cudaError_t e = launch_pdl(kernels[static_cast<int>(form)], dim3(grid), dim3(THREADS), SMEM_BYTES, stream, ta, tb, p);
+        cudaError_t e = launch_pdl(kernels[static_cast<int>(form) + (g.f16 ? 4 : 0)], dim3(grid), dim3(THREADS), SMEM_BYTES, stream, ta, tb, p);
         if (e != cudaSuccess) return cuda_fail(e, "cmt_gemm_bias_act(tcgen05) launch");
     }
     CMT_LAUNCH_CHECK("cmt_gemm_bias_act(tcgen05)");

@@ -13,14 +13,16 @@ struct GemmArgs {
     long long lda, ldb, ldc, cb, cb_stride;
     long long strideA, strideB, strideC;
     float alpha;
-    int relu, bias_per_row, out_bf16;
-    // bf16 tensor-core path only: element (m, n) of batch z is stored at z*strideC + (n / cb)*cb_stride + (n % cb)*ldc + m
+    int relu, bias_per_row;
+    int out_16;        // 16-bit output: bf16, or fp16 with f16 (else fp32)
+    int f16;           // tensor-core path: fp16 operands and 16-bit outputs instead of bf16
+    // 16-bit tensor-core path only: element (m, n) of batch z is stored at z*strideC + (n / cb)*cb_stride + (n % cb)*ldc + m
     // (C^T inside each column block, see cmt_gemm_bias_act)
     int transpose_c;
-    // bf16 tensor-core path only: [batch][N/32] atomicMax of the squared norm of every row's 32-column block (attention
+    // 16-bit tensor-core path only: [batch][N/32] atomicMax of the squared norm of every row's 32-column block (attention
     // score bound), or nullptr
     float* norm2_max;
-    // ---- bf16 tensor-core path only: segmented K (n_seg == 0: ordinary GEMM) ----
+    // ---- tensor-core path only: segmented K (n_seg == 0: ordinary GEMM) ----
     // K = n_seg * seg_k columns of B; segment s multiplies B[:, s*seg_k : (s+1)*seg_k] with the A columns
     // [seg_acol[s], seg_acol[s] + seg_k) read at row (m + a_row_off + seg_shift[s]) of the batch's A matrix, which has
     // a_rows rows and a_cols columns (rows outside [0, a_rows) are zero-filled by the TMA unit).
@@ -30,8 +32,8 @@ struct GemmArgs {
     int b_batch_div;   // batch z uses B of batch z / b_batch_div (0 or 1: z)
     // ---- token epilogue of the 3x3 shared_conv (conv_xv != nullptr) ----
     // Output row m is position (y, x) = (m / conv_Wp, m % conv_Wp) of the zero-padded map of frame z; interior positions
-    // become token t = (y - 1) * conv_W + (x - 1) and are stored as xv[z][t - tok_begin] = bf16(v),
-    // xk[z][t - tok_begin] = bf16(v + pos[t]) (v = ReLU(acc + bias)); border rows are dropped.
+    // become token t = (y - 1) * conv_W + (x - 1) and are stored as xv[z][t - tok_begin] = lp(v),
+    // xk[z][t - tok_begin] = lp(v + pos[t]) (v = ReLU(acc + bias), lp = rounding to the operand dtype); border rows are dropped.
     void* conv_xk;
     void* conv_xv;
     const float* conv_pos;
@@ -47,7 +49,8 @@ struct AttnArgs {
     float* lse;
     int B, H, Nq, N_kv, kv_begin, kv_end;
     long long q_ld, k_bstride, k_hstride, v_bstride, v_hstride, v_ld;
-    int o_bf16;
+    int f16;                         // tensor-core path: fp16 q / k / vt instead of bf16
+    int o_dtype;                     // CMT_F32 | CMT_BF16 | CMT_F16
     const unsigned char* key_keep;   // [B, N_kv] 1 = attend, 0 = padded key (attention.py:76-90), or nullptr
     const float* q_norm2;            // [B*H] max |q|^2 per (frame, head), or nullptr (online softmax)
     const float* k_norm2;            // max |k|^2 per (frame, head) at [b * kn_bstride + h]
@@ -70,7 +73,7 @@ int launch_gather_tokens(const void* x_bev, const void* x_img, const float* bev_
                          int n_img, int tok_begin, int tok_end, int rv_tok0, int rv_rows, int feat_dtype, int out_dtype,
                          cudaStream_t stream);
 int launch_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, int W, int guard, int in_dtype,
-                               cudaStream_t stream);
+                               int out_dtype, cudaStream_t stream);
 int launch_coop_max(const float* a, const float* b, float* out, long long n, cudaStream_t stream);
 int launch_lse_merge(const float* o_parts, const float* lse_parts, void* o, float* lse, int G,
                      int B, int H, int Nq, long long o_gstride, long long lse_gstride, int o_dtype, cudaStream_t stream);

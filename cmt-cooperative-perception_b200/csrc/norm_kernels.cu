@@ -3,14 +3,14 @@
 // projects/mmdet3d_plugin/models/utils/petr_transformer.py:347-371).  One warp per 256-wide row:
 //   y   = LN(x + r; gamma, beta)                               fp32
 //   y2  = LN(y; gamma2, beta2)            (optional: the stacked post-normed intermediate)
-//   ylp = cast(y), yadd = cast(y + add)   (optional: bf16|fp32 A operands of the next projections,
+//   ylp = cast(y), yadd = cast(y + add)   (optional: bf16|fp16|fp32 A operands of the next projections,
 //                                          `add` = query_pos)
 // HBM/launch bound; replaces ~6 eager torch launches per norm.
 #include "kernels.cuh"
 
 namespace cmt {
 
-template <int kPerLane, bool kLpBf16>
+template <int kPerLane, int kLp>
 __global__ void __launch_bounds__(256) add_layernorm_kernel(const float* __restrict__ x, const float* __restrict__ r,
                                                             const float* __restrict__ gamma,
                                                             const float* __restrict__ beta, float eps, int M,
@@ -62,11 +62,11 @@ __global__ void __launch_bounds__(256) add_layernorm_kernel(const float* __restr
             *reinterpret_cast<float4*>(y + base + idx) = make_float4(v[4 * g], v[4 * g + 1], v[4 * g + 2], v[4 * g + 3]);
             s2 += (v[4 * g] + v[4 * g + 1]) + (v[4 * g + 2] + v[4 * g + 3]);
             if (ylp != nullptr) {
-                if (kLpBf16) {
+                if (kLp != CMT_F32) {
                     uint2 w;
-                    w.x = pack_bf16x2(v[4 * g], v[4 * g + 1]);
-                    w.y = pack_bf16x2(v[4 * g + 2], v[4 * g + 3]);
-                    *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(ylp) + base + idx) = w;
+                    w.x = pack_lp2<kLp>(v[4 * g], v[4 * g + 1]);
+                    w.y = pack_lp2<kLp>(v[4 * g + 2], v[4 * g + 3]);
+                    *reinterpret_cast<uint2*>(reinterpret_cast<uint16_t*>(ylp) + base + idx) = w;
                 } else {
                     *reinterpret_cast<float4*>(reinterpret_cast<float*>(ylp) + base + idx) =
                         make_float4(v[4 * g], v[4 * g + 1], v[4 * g + 2], v[4 * g + 3]);
@@ -76,11 +76,11 @@ __global__ void __launch_bounds__(256) add_layernorm_kernel(const float* __restr
                 const float4 ad = *reinterpret_cast<const float4*>(add + base + idx);
                 const float a0 = v[4 * g] + ad.x, a1 = v[4 * g + 1] + ad.y, a2 = v[4 * g + 2] + ad.z,
                             a3 = v[4 * g + 3] + ad.w;
-                if (kLpBf16) {
+                if (kLp != CMT_F32) {
                     uint2 w;
-                    w.x = pack_bf16x2(a0, a1);
-                    w.y = pack_bf16x2(a2, a3);
-                    *reinterpret_cast<uint2*>(reinterpret_cast<__nv_bfloat16*>(yadd) + base + idx) = w;
+                    w.x = pack_lp2<kLp>(a0, a1);
+                    w.y = pack_lp2<kLp>(a2, a3);
+                    *reinterpret_cast<uint2*>(reinterpret_cast<uint16_t*>(yadd) + base + idx) = w;
                 } else {
                     *reinterpret_cast<float4*>(reinterpret_cast<float*>(yadd) + base + idx) = make_float4(a0, a1, a2, a3);
                 }
@@ -117,17 +117,20 @@ int launch_add_layernorm(const float* x, const float* r, const float* gamma, con
     CMT_CHECK_ARG(C == 256, "cmt_add_layernorm: embed dim 256 only (got %d)", C);
     CMT_CHECK_ARG(y2 == nullptr || (gamma2 && beta2), "cmt_add_layernorm: second norm needs gamma2/beta2");
     CMT_CHECK_ARG(yadd == nullptr || add != nullptr, "cmt_add_layernorm: yadd needs add");
-    CMT_CHECK_ARG(lp_dtype == CMT_F32 || lp_dtype == CMT_BF16, "cmt_add_layernorm: bad lp dtype");
+    CMT_CHECK_ARG(lp_dtype == CMT_F32 || lp_dtype == CMT_BF16 || lp_dtype == CMT_F16, "cmt_add_layernorm: bad lp dtype");
     const int rows_per_block = 8;
     long long blocks = (M + rows_per_block - 1) / rows_per_block;
     const long long cap = static_cast<long long>(device_sm_count()) * 8;
     if (blocks > cap) blocks = cap;
     if (lp_dtype == CMT_BF16)
-        launch_pdl(add_layernorm_kernel<8, true>, dim3(static_cast<int>(blocks)), dim3(256), 0, stream, x, r, gamma, beta, eps, M, y, gamma2,
-                                                                                   beta2, y2, add, ylp, yadd, x_row_broadcast);
+        launch_pdl(add_layernorm_kernel<8, CMT_BF16>, dim3(static_cast<int>(blocks)), dim3(256), 0, stream, x, r, gamma, beta, eps, M, y,
+                   gamma2, beta2, y2, add, ylp, yadd, x_row_broadcast);
+    else if (lp_dtype == CMT_F16)
+        launch_pdl(add_layernorm_kernel<8, CMT_F16>, dim3(static_cast<int>(blocks)), dim3(256), 0, stream, x, r, gamma, beta, eps, M, y,
+                   gamma2, beta2, y2, add, ylp, yadd, x_row_broadcast);
     else
-        launch_pdl(add_layernorm_kernel<8, false>, dim3(static_cast<int>(blocks)), dim3(256), 0, stream, x, r, gamma, beta, eps, M, y, gamma2,
-                                                                                    beta2, y2, add, ylp, yadd, x_row_broadcast);
+        launch_pdl(add_layernorm_kernel<8, CMT_F32>, dim3(static_cast<int>(blocks)), dim3(256), 0, stream, x, r, gamma, beta, eps, M, y,
+                   gamma2, beta2, y2, add, ylp, yadd, x_row_broadcast);
     CMT_LAUNCH_CHECK("cmt_add_layernorm");
     return CMT_OK;
 }

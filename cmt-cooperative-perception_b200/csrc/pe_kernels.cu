@@ -36,7 +36,8 @@ __device__ __forceinline__ float div_by_const(float a, float b, float inv) {
 // ~9 instructions per output value, so the kernel is bound by the HBM write instead of by issue.
 // kBins = depth bins per thread-item: 16 (D % 16 == 0: 96 bytes of bf16 = three 256-bit stores, every store instruction
 // writes whole 32-byte sectors) or 8 (48 bytes = three 128-bit stores at a 48-byte lane stride: half-filled sectors).
-template <bool kBf16, int kBins>
+// kOut: output dtype, CMT_F32 | CMT_BF16 | CMT_F16 (the 16-bit forms differ only in the rounding).
+template <int kOut, int kBins>
 __global__ void __launch_bounds__(256) ray_pe_kernel(const float* __restrict__ img2lidar,
                                                      void* __restrict__ out, RayPeParams p) {
     extern __shared__ float sm[];
@@ -78,26 +79,26 @@ __global__ void __launch_bounds__(256) ray_pe_kernel(const float* __restrict__ i
             }
         }
         const long long t = row_base + tl;  // in NV-feature units
-        if (kBf16) {
+        if (kOut != CMT_F32) {
             if (kBins == 16) {
                 uint8_t* o = reinterpret_cast<uint8_t*>(out) + t * (NV * 2);
 #pragma unroll
                 for (int q = 0; q < 3; ++q)
                     asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(o + 32 * q),
-                                 "r"(pack_bf16x2(vals[16 * q + 0], vals[16 * q + 1])), "r"(pack_bf16x2(vals[16 * q + 2], vals[16 * q + 3])),
-                                 "r"(pack_bf16x2(vals[16 * q + 4], vals[16 * q + 5])), "r"(pack_bf16x2(vals[16 * q + 6], vals[16 * q + 7])),
-                                 "r"(pack_bf16x2(vals[16 * q + 8], vals[16 * q + 9])), "r"(pack_bf16x2(vals[16 * q + 10], vals[16 * q + 11])),
-                                 "r"(pack_bf16x2(vals[16 * q + 12], vals[16 * q + 13])), "r"(pack_bf16x2(vals[16 * q + 14], vals[16 * q + 15]))
+                                 "r"(pack_lp2<kOut>(vals[16 * q + 0], vals[16 * q + 1])), "r"(pack_lp2<kOut>(vals[16 * q + 2], vals[16 * q + 3])),
+                                 "r"(pack_lp2<kOut>(vals[16 * q + 4], vals[16 * q + 5])), "r"(pack_lp2<kOut>(vals[16 * q + 6], vals[16 * q + 7])),
+                                 "r"(pack_lp2<kOut>(vals[16 * q + 8], vals[16 * q + 9])), "r"(pack_lp2<kOut>(vals[16 * q + 10], vals[16 * q + 11])),
+                                 "r"(pack_lp2<kOut>(vals[16 * q + 12], vals[16 * q + 13])), "r"(pack_lp2<kOut>(vals[16 * q + 14], vals[16 * q + 15]))
                                  : "memory");
             } else {
                 uint4* o = reinterpret_cast<uint4*>(out) + 3 * t;
 #pragma unroll
                 for (int q = 0; q < 3; ++q) {
                     uint4 w;
-                    w.x = pack_bf16x2(vals[8 * q + 0], vals[8 * q + 1]);
-                    w.y = pack_bf16x2(vals[8 * q + 2], vals[8 * q + 3]);
-                    w.z = pack_bf16x2(vals[8 * q + 4], vals[8 * q + 5]);
-                    w.w = pack_bf16x2(vals[8 * q + 6], vals[8 * q + 7]);
+                    w.x = pack_lp2<kOut>(vals[8 * q + 0], vals[8 * q + 1]);
+                    w.y = pack_lp2<kOut>(vals[8 * q + 2], vals[8 * q + 3]);
+                    w.z = pack_lp2<kOut>(vals[8 * q + 4], vals[8 * q + 5]);
+                    w.w = pack_lp2<kOut>(vals[8 * q + 6], vals[8 * q + 7]);
                     o[q] = w;
                 }
             }
@@ -117,7 +118,7 @@ struct RayQueryParams {
     int B, V, Nq, D;
 };
 
-template <bool kBf16>
+template <int kOut>
 __global__ void __launch_bounds__(256) ray_query_pe_kernel(const float* __restrict__ ref,
                                                            const float* __restrict__ l2i,
                                                            const float* __restrict__ i2l,
@@ -168,12 +169,12 @@ __global__ void __launch_bounds__(256) ray_query_pe_kernel(const float* __restri
             acc = acc + r[3];
             vals[e] = (acc - p.pc_min[c]) / p.pc_rng[c];
         }
-        if (kBf16) {
+        if (kOut != CMT_F32) {
             uint4 w;
-            w.x = pack_bf16x2(vals[0], vals[1]);
-            w.y = pack_bf16x2(vals[2], vals[3]);
-            w.z = pack_bf16x2(vals[4], vals[5]);
-            w.w = pack_bf16x2(vals[6], vals[7]);
+            w.x = pack_lp2<kOut>(vals[0], vals[1]);
+            w.y = pack_lp2<kOut>(vals[2], vals[3]);
+            w.z = pack_lp2<kOut>(vals[4], vals[5]);
+            w.w = pack_lp2<kOut>(vals[6], vals[7]);
             reinterpret_cast<uint4*>(out)[t] = w;
         } else {
             float4* o = reinterpret_cast<float4*>(out) + 2 * t;
@@ -183,7 +184,7 @@ __global__ void __launch_bounds__(256) ray_query_pe_kernel(const float* __restri
     }
 }
 
-template <bool kBf16>
+template <int kIn>
 __global__ void __launch_bounds__(256) masked_view_sum_kernel(const void* __restrict__ emb,
                                                               const float* __restrict__ mask,
                                                               const float* __restrict__ base, long long base_bstride,
@@ -200,8 +201,8 @@ __global__ void __launch_bounds__(256) masked_view_sum_kernel(const void* __rest
             const long long row = (static_cast<long long>(b) * V + v) * Nq + n;
             const float m = mask[row];
             float e;
-            if (kBf16)
-                e = __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(emb)[row * C + c]);
+            if (kIn != CMT_F32)
+                e = load_lp<kIn>(emb, row * C + c);
             else
                 e = reinterpret_cast<const float*>(emb)[row * C + c];
             acc += e * m;
@@ -212,7 +213,7 @@ __global__ void __launch_bounds__(256) masked_view_sum_kernel(const void* __rest
     }
 }
 
-template <bool kBf16>
+template <int kOut>
 __global__ void __launch_bounds__(256) pos2embed_kernel(const float* __restrict__ pos,
                                                         void* __restrict__ out, int N,
                                                         int pos_stride, int F) {
@@ -229,8 +230,8 @@ __global__ void __launch_bounds__(256) pos2embed_kernel(const float* __restrict_
         const float dim_t = (2.0f * static_cast<float>(m / 2)) / static_cast<float>(F) + 1.0f;
         const float a = pv / dim_t;
         const float r = (m & 1) ? cosf(a) : sinf(a);
-        if (kBf16)
-            reinterpret_cast<__nv_bfloat16*>(out)[t] = __float2bfloat16_rn(r);
+        if (kOut != CMT_F32)
+            store_lp<kOut>(out, t, r);
         else
             reinterpret_cast<float*>(out)[t] = r;
     }
@@ -250,7 +251,7 @@ int launch_ray_pe(const float* img2lidar, void* out, int n_cam, int H, int W, in
     CMT_CHECK_ARG(img2lidar && out && pc, "cmt_ray_pe: null pointer");
     CMT_CHECK_ARG(n_cam > 0 && H > 0 && W > 0 && D > 0, "cmt_ray_pe: bad shape");
     CMT_CHECK_ARG(D % 8 == 0, "cmt_ray_pe: depth_num must be a multiple of 8 (got D=%d)", D);
-    CMT_CHECK_ARG(out_dtype == CMT_F32 || out_dtype == CMT_BF16, "cmt_ray_pe: bad dtype");
+    CMT_CHECK_ARG(out_dtype == CMT_F32 || out_dtype == CMT_BF16 || out_dtype == CMT_F16, "cmt_ray_pe: bad dtype");
     RayPeParams p{};
     for (int c = 0; c < 3; ++c) {
         p.pc_min[c] = pc[c];
@@ -271,11 +272,15 @@ int launch_ray_pe(const float* img2lidar, void* out, int n_cam, int H, int W, in
     CMT_CHECK_ARG(smem <= 48 * 1024, "cmt_ray_pe: W + D too large");
     const bool wide = D % 16 == 0 && (reinterpret_cast<uintptr_t>(out) & 31) == 0;
     if (out_dtype == CMT_BF16 && wide)
-        ray_pe_kernel<true, 16><<<grid, 256, smem, stream>>>(img2lidar, out, p);
+        ray_pe_kernel<CMT_BF16, 16><<<grid, 256, smem, stream>>>(img2lidar, out, p);
     else if (out_dtype == CMT_BF16)
-        ray_pe_kernel<true, 8><<<grid, 256, smem, stream>>>(img2lidar, out, p);
+        ray_pe_kernel<CMT_BF16, 8><<<grid, 256, smem, stream>>>(img2lidar, out, p);
+    else if (out_dtype == CMT_F16 && wide)
+        ray_pe_kernel<CMT_F16, 16><<<grid, 256, smem, stream>>>(img2lidar, out, p);
+    else if (out_dtype == CMT_F16)
+        ray_pe_kernel<CMT_F16, 8><<<grid, 256, smem, stream>>>(img2lidar, out, p);
     else
-        ray_pe_kernel<false, 8><<<grid, 256, smem, stream>>>(img2lidar, out, p);
+        ray_pe_kernel<CMT_F32, 8><<<grid, 256, smem, stream>>>(img2lidar, out, p);
     CMT_LAUNCH_CHECK("cmt_ray_pe");
     return CMT_OK;
 }
@@ -286,7 +291,7 @@ int launch_ray_query_pe(const float* ref, const float* l2i, const float* i2l, vo
     CMT_CHECK_ARG(ref && l2i && i2l && out && mask && pc, "cmt_ray_query_pe: null pointer");
     CMT_CHECK_ARG(B > 0 && V > 0 && Nq > 0 && D > 0, "cmt_ray_query_pe: bad shape");
     CMT_CHECK_ARG((D * 3) % 8 == 0, "cmt_ray_query_pe: depth_num*3 must be a multiple of 8");
-    CMT_CHECK_ARG(out_dtype == CMT_F32 || out_dtype == CMT_BF16, "cmt_ray_query_pe: bad dtype");
+    CMT_CHECK_ARG(out_dtype == CMT_F32 || out_dtype == CMT_BF16 || out_dtype == CMT_F16, "cmt_ray_query_pe: bad dtype");
     RayQueryParams p{};
     for (int c = 0; c < 3; ++c) {
         p.pc_min[c] = pc[c];
@@ -302,9 +307,11 @@ int launch_ray_query_pe(const float* ref, const float* l2i, const float* i2l, vo
     const long long total = static_cast<long long>(B) * V * Nq * (D * 3 / 8);
     const int grid = grid_for(total, 256);
     if (out_dtype == CMT_BF16)
-        ray_query_pe_kernel<true><<<grid, 256, 0, stream>>>(ref, l2i, i2l, out, mask, p);
+        ray_query_pe_kernel<CMT_BF16><<<grid, 256, 0, stream>>>(ref, l2i, i2l, out, mask, p);
+    else if (out_dtype == CMT_F16)
+        ray_query_pe_kernel<CMT_F16><<<grid, 256, 0, stream>>>(ref, l2i, i2l, out, mask, p);
     else
-        ray_query_pe_kernel<false><<<grid, 256, 0, stream>>>(ref, l2i, i2l, out, mask, p);
+        ray_query_pe_kernel<CMT_F32><<<grid, 256, 0, stream>>>(ref, l2i, i2l, out, mask, p);
     CMT_LAUNCH_CHECK("cmt_ray_query_pe");
     return CMT_OK;
 }
@@ -316,9 +323,11 @@ int launch_masked_view_sum(const void* emb, const float* mask, const float* base
     const long long total = static_cast<long long>(B) * Nq * C;
     const int grid = grid_for(total, 256);
     if (emb_dtype == CMT_BF16)
-        masked_view_sum_kernel<true><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C);
+        masked_view_sum_kernel<CMT_BF16><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C);
+    else if (emb_dtype == CMT_F16)
+        masked_view_sum_kernel<CMT_F16><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C);
     else if (emb_dtype == CMT_F32)
-        masked_view_sum_kernel<false><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C);
+        masked_view_sum_kernel<CMT_F32><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C);
     else
         CMT_CHECK_ARG(false, "cmt_masked_view_sum: bad dtype");
     CMT_LAUNCH_CHECK("cmt_masked_view_sum");
@@ -332,9 +341,11 @@ int launch_pos2embed(const float* pos, void* out, int N, int pos_stride, int F, 
     const long long total = static_cast<long long>(N) * 2 * F;
     const int grid = grid_for(total, 256);
     if (out_dtype == CMT_BF16)
-        pos2embed_kernel<true><<<grid, 256, 0, stream>>>(pos, out, N, pos_stride, F);
+        pos2embed_kernel<CMT_BF16><<<grid, 256, 0, stream>>>(pos, out, N, pos_stride, F);
+    else if (out_dtype == CMT_F16)
+        pos2embed_kernel<CMT_F16><<<grid, 256, 0, stream>>>(pos, out, N, pos_stride, F);
     else if (out_dtype == CMT_F32)
-        pos2embed_kernel<false><<<grid, 256, 0, stream>>>(pos, out, N, pos_stride, F);
+        pos2embed_kernel<CMT_F32><<<grid, 256, 0, stream>>>(pos, out, N, pos_stride, F);
     else
         CMT_CHECK_ARG(false, "cmt_pos2embed: bad dtype");
     CMT_LAUNCH_CHECK("cmt_pos2embed");

@@ -63,7 +63,7 @@ __global__ void __launch_bounds__(256) simt_gemm_kernel(GemmArgs g) {
             if (g.relu) v = fmaxf(v, 0.0f);
             const long long off = z * g.strideC + (n / g.cb) * g.cb_stride +
                                   static_cast<long long>(m) * g.ldc + (n % g.cb);
-            if (g.out_bf16)
+            if (g.out_16)
                 reinterpret_cast<__nv_bfloat16*>(g.C)[off] = __float2bfloat16_rn(v);
             else
                 reinterpret_cast<float*>(g.C)[off] = v;
@@ -148,7 +148,7 @@ __global__ void __launch_bounds__(128) simt_attn_kernel(AttnArgs a) {
 #pragma unroll
     for (int d = 0; d < 32; ++d) {
         const float v = o[d] * inv;
-        if (a.o_bf16)
+        if (a.o_dtype == CMT_BF16)
             reinterpret_cast<__nv_bfloat16*>(a.o)[obase + d] = __float2bfloat16_rn(v);
         else
             reinterpret_cast<float*>(a.o)[obase + d] = v;

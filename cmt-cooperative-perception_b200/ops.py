@@ -69,12 +69,27 @@ class _timed:
 FORCE_ONLINE_SOFTMAX = False
 
 
+# The compute precisions of the modules (`set_precision`): 'bf16' and 'fp16' run the tcgen05 kernels with 16-bit operands,
+# 'fp32' the fp32 CUDA-core verification kernels.  The task heads stay fp32-grade in every precision.
+PRECISIONS = {"bf16": torch.bfloat16, "fp16": torch.float16, "fp32": torch.float32}
+
+
+def compute_dtype(precision: str) -> torch.dtype:
+    """The torch dtype of a precision name; an unknown name raises ValueError."""
+    try:
+        return PRECISIONS[precision]
+    except KeyError:
+        raise ValueError(f"unknown precision {precision!r} (one of {', '.join(PRECISIONS)})") from None
+
+
 def _dt(dtype) -> int:
     if dtype == torch.float32:
         return CMT_F32
     if dtype == torch.bfloat16:
         return CMT_BF16
-    raise TypeError(f"unsupported dtype {dtype} (fp32 or bf16 only)")
+    if dtype == torch.float16:
+        return CMT_F16
+    raise TypeError(f"unsupported dtype {dtype} (fp32, bf16 or fp16 only)")
 
 
 def _ptr(t):
@@ -227,21 +242,24 @@ def conv_guard_rows(W):
     return (W + 3 + 7) // 8 * 8
 
 
-def nchw_to_padded_nhwc(x, out=None):
-    """[B,C,H,W] (fp32|bf16|fp16) -> zero-padded channel-last bf16 rows [B, 2*guard + (H+2)*(W+2), C] (cmt_nchw_to_padded_nhwc).
-    `out` (zero-initialised once, then reusable: only interior rows are written) is allocated when None."""
+def nchw_to_padded_nhwc(x, out=None, dtype=torch.bfloat16):
+    """[B,C,H,W] (fp32|bf16|fp16) -> zero-padded channel-last rows [B, 2*guard + (H+2)*(W+2), C] in `dtype` (bf16 or fp16)
+    (cmt_nchw_to_padded_nhwc).  `out` (zero-initialised once, then reusable: only interior rows are written) is allocated
+    when None."""
     x = _cuda(x, "x")
     if x.dtype not in _FEAT_DTYPES:
         raise TypeError(f"feature maps must be fp32, bf16 or fp16, got {x.dtype}")
     B, C, H, W = x.shape
     guard = conv_guard_rows(W)
     rows = 2 * guard + (H + 2) * (W + 2)
+    if dtype not in (torch.bfloat16, torch.float16):
+        raise TypeError(f"nchw_to_padded_nhwc: output dtype must be bf16 or fp16, got {dtype}")
     if out is None:
-        out = torch.zeros((B, rows, C), dtype=torch.bfloat16, device=x.device)
-    assert out.shape == (B, rows, C) and out.dtype == torch.bfloat16 and out.is_contiguous()
+        out = torch.zeros((B, rows, C), dtype=dtype, device=x.device)
+    assert out.shape == (B, rows, C) and out.dtype == dtype and out.is_contiguous()
     lib = _lib.load()
     with torch.cuda.device(x.device), _timed("nchw_to_padded_nhwc", x):
-        rc = lib.cmt_nchw_to_padded_nhwc(_ptr(x), _ptr(out), B, C, H, W, guard, _FEAT_DTYPES[x.dtype], _stream(x))
+        rc = lib.cmt_nchw_to_padded_nhwc(_ptr(x), _ptr(out), B, C, H, W, guard, _FEAT_DTYPES[x.dtype], _stream(x), _dt(dtype))
     _lib.check(rc, "cmt_nchw_to_padded_nhwc")
     _count()
     return out
@@ -249,14 +267,17 @@ def nchw_to_padded_nhwc(x, out=None):
 
 def shared_conv_tokens(xp, w, bias, bev_pos, xk, xv, H, W, tok_range=None):
     """3x3 conv + folded BN + ReLU as an implicit GEMM writing the BEV token rows of xk / xv (cmt_shared_conv_tokens).
-    xp [B,rows,Cin] from nchw_to_padded_nhwc; w [Cout, 9*Cin] bf16 tap-major with the BN scale folded in; bias [Cout] fp32;
-    bev_pos [H*W,Cout] fp32; xk, xv [B,n_rows,Cout] bf16 whose first (hi-lo) rows receive tokens [lo,hi) (default all)."""
-    xp = _cuda(xp, "xp", torch.bfloat16)
-    w = _cuda(w, "w", torch.bfloat16)
+    xp [B,rows,Cin] from nchw_to_padded_nhwc; w [Cout, 9*Cin] tap-major with the BN scale folded in; bias [Cout] fp32;
+    bev_pos [H*W,Cout] fp32; xk, xv [B,n_rows,Cout] whose first (hi-lo) rows receive tokens [lo,hi) (default all).
+    xp, w, xk and xv share one dtype, bf16 or fp16."""
+    xp = _cuda(xp, "xp")
+    if xp.dtype not in (torch.bfloat16, torch.float16):
+        raise TypeError(f"shared_conv_tokens: operands must be bf16 or fp16, got {xp.dtype}")
+    w = _cuda(w, "w", xp.dtype)
     bias = _cuda(bias, "bias", torch.float32)
     bev_pos = _cuda(bev_pos, "bev_pos", torch.float32)
-    xk = _cuda(xk, "xk", torch.bfloat16)
-    xv = _cuda(xv, "xv", torch.bfloat16)
+    xk = _cuda(xk, "xk", xp.dtype)
+    xv = _cuda(xv, "xv", xp.dtype)
     B, rows, Cin = xp.shape
     Cout = w.shape[0]
     guard = conv_guard_rows(W)
@@ -266,7 +287,7 @@ def shared_conv_tokens(xp, w, bias, bev_pos, xk, xv, H, W, tok_range=None):
     lib = _lib.load()
     with torch.cuda.device(xp.device), _timed("shared_conv", xp):
         rc = lib.cmt_shared_conv_tokens(_ptr(xp), _ptr(w), _ptr(bias), _ptr(bev_pos), _ptr(xk), _ptr(xv), B, Cin, Cout, H, W,
-                                        guard, xk.shape[1] * Cout, lo, hi, _stream(xp))
+                                        guard, xk.shape[1] * Cout, lo, hi, _stream(xp), _dt(xp.dtype))
     _lib.check(rc, "cmt_shared_conv_tokens")
     _count()
 
@@ -297,7 +318,7 @@ def gemm(A, Bm, bias, C, M, N, K, *, lda, ldb, ldc, cb=None, cb_stride=0, batch=
          strideC=0, alpha=1.0, relu=False, bias_per_row=False, force_simt=False, transpose_out=False,
          norm2_max=None, tag=None):
     """Raw cmt_gemm_bias_act: C = act((A B^T + bias) * alpha) with column-block output addressing.
-    norm2_max: optional zero-initialised fp32 [batch, N/32] receiving max |row block|^2 (bf16 path)."""
+    norm2_max: optional zero-initialised fp32 [batch, N/32] receiving max |row block|^2 (16-bit tensor-core path)."""
     A = _cuda(A, "A")
     Bm = _cuda(Bm, "B", A.dtype)
     C = _cuda(C, "C")
@@ -366,7 +387,7 @@ def project_values_t(xv, w, bias, n_layers, H, out=None):
     ld = (N_kv + 7) // 8 * 8
     if out is None:
         out = torch.empty((B, n_layers, H, HEAD_DIM, ld), dtype=xv.dtype, device=xv.device)
-    if xv.dtype == torch.bfloat16:
+    if xv.dtype != torch.float32:
         # tokens on the M side like the K projection (the CTA keeps its slice of W_v resident in shared memory and
         # streams token tiles), each [tokens, 32] head block stored transposed
         gemm(xv, w, bias, out, N_kv, NO, C, lda=C, ldb=C, ldc=ld, cb=HEAD_DIM, cb_stride=HEAD_DIM * ld, batch=B,
@@ -395,7 +416,8 @@ def cross_attn(q, k, vt, layer, *, kv_begin=0, kv_end=None, o_dtype=None, return
     vt [B,L,H,32,ld]; attends tokens [kv_begin,kv_end) of layer `layer`. -> o [B,Nq,H*32] (, lse [B,H,Nq]).
     key_keep: optional [B,N_kv] bool/uint8, True = attend (the key_padding_mask of attention.py:76-90, whose
     unpad_input keeps the True entries).
-    q_norm2 [B,H] / k_norm2 [B,L,H] fp32 (from the projections' norm2_max): enables the static softmax shift."""
+    q_norm2 [B,H] / k_norm2 [B,L,H] fp32 (from the projections' norm2_max): enables the static softmax shift.
+    q, k, vt: bf16 or fp16 (tcgen05 kernel) or fp32 (CUDA-core kernel); o_dtype: fp32 or q's dtype."""
     q = _cuda(q, "q")
     k = _cuda(k, "k", q.dtype)
     vt = _cuda(vt, "vt", q.dtype)
@@ -424,8 +446,11 @@ def cross_attn(q, k, vt, layer, *, kv_begin=0, kv_end=None, o_dtype=None, return
     dt = _dt(q.dtype)
     if simt and dt == CMT_BF16:
         dt = CMT_BF16_SIMT
+    elif simt and dt == CMT_F16:
+        raise TypeError("cross_attn(simt=True): fp16 operands run on the tcgen05 kernel only")
+    tc = dt in (CMT_BF16, CMT_F16)
     ws, ws_bytes = None, 0
-    if dt == CMT_BF16:
+    if tc:
         with torch.cuda.device(q.device):
             ws_bytes = int(lib.cmt_cross_attn_workspace_bytes(B, H, Nq, kv_end - kv_begin))
         ws = _workspace(q.device, ws_bytes)
@@ -435,7 +460,7 @@ def cross_attn(q, k, vt, layer, *, kv_begin=0, kv_end=None, o_dtype=None, return
         key_keep = key_keep.to(torch.uint8).contiguous()
     qn = kn = None
     kn_stride = 0
-    if q_norm2 is not None and k_norm2 is not None and dt == CMT_BF16 and not FORCE_ONLINE_SOFTMAX:
+    if q_norm2 is not None and k_norm2 is not None and tc and not FORCE_ONLINE_SOFTMAX:
         qn = _cuda(q_norm2, "q_norm2", torch.float32)
         k_norm2 = _cuda(k_norm2, "k_norm2", torch.float32)
         assert qn.shape == (B, H) and k_norm2.shape == (B, L, H)
@@ -455,7 +480,7 @@ def cross_attn(q, k, vt, layer, *, kv_begin=0, kv_end=None, o_dtype=None, return
         ev.append((e0, e1))
     _lib.check(rc, "cmt_cross_attn_fwd")
     # tcgen05 path: [mask pack] + [static-shift kernel] + online kernel + merge
-    _count((2 if dt == CMT_BF16 else 1) + (1 if key_keep is not None and dt == CMT_BF16 else 0) + (1 if qn is not None else 0))
+    _count((2 if tc else 1) + (1 if key_keep is not None and tc else 0) + (1 if qn is not None else 0))
     return (o, lse) if return_lse else o
 
 

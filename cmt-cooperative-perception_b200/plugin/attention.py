@@ -1,7 +1,7 @@
 """FlashAttention / FlashMHA with the reference's constructor and forward signatures
 (projects/mmdet3d_plugin/models/utils/attention.py:30-138), backed by libcmtcoop_b200:
 in-projection and out-projection run on the tcgen05 GEMM, the attention core on the tcgen05
-flash kernel (bf16 mode) or on the fp32 CUDA-core kernels (fp32 verification mode).
+flash kernel (bf16 and fp16 modes) or on the fp32 CUDA-core kernels (fp32 verification mode).
 
 State-dict keys are the reference's: in_proj_weight [3E,E], in_proj_bias [3E], out_proj.{weight,bias}.
 """
@@ -15,10 +15,7 @@ import torch.nn as nn
 from .. import ops
 
 _Q_SCALE = ops.LOG2E / math.sqrt(ops.HEAD_DIM)  # Q is pre-multiplied by log2(e)/sqrt(d): softmax is a bare exp2
-
-
-def _compute_dtype(precision):
-    return torch.float32 if precision == "fp32" else torch.bfloat16
+_compute_dtype = ops.compute_dtype
 
 
 class KVCache:
@@ -50,6 +47,12 @@ class FlashAttention(nn.Module):
         self.dropout_p = attention_dropout
         self.fp16_enabled = True
         self.precision = "bf16"
+
+    def set_precision(self, precision):
+        """'bf16' (default) or 'fp16' (tcgen05 kernel; the reference runs flash-attn in fp16), or 'fp32' (CUDA-core)."""
+        _compute_dtype(precision)
+        self.precision = precision
+        return self
 
     def forward(self, q, kv, causal=False, key_padding_mask=None):
         assert q.is_cuda and kv.is_cuda, "FlashAttention runs on the GPU only (no CPU fallback)"
@@ -105,6 +108,13 @@ class FlashMHA(nn.Module):
         self.precision = "bf16"
         self._wcache = None
         self._reset_parameters()
+
+    def set_precision(self, precision):
+        """'bf16' (default), 'fp16' or 'fp32' for the projections and the attention core."""
+        _compute_dtype(precision)
+        self.precision = precision
+        self.inner_attn.precision = precision
+        return self
 
     def _reset_parameters(self):
         nn.init.xavier_uniform_(self.in_proj_weight)

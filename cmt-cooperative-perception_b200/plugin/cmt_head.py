@@ -9,6 +9,7 @@ What runs where (default bf16 inference path):
     operands on the tensor cores, fp32 accumulation / residuals / statistics.  The reference computes the
     decoder in fp32 (nn.MultiheadAttention, nn.Linear); the difference is inside the 1e-2 rel-L2 budget of
     the bf16 mode and `set_precision('fp32')` selects the fp32 CUDA-core kernels (<= 1e-4).
+    `set_precision('fp16')` runs the same tensor-core kernels with fp16 operands (3 more mantissa bits than bf16).
   * the task heads always compute in fp32 (their logits feed the top-k).
 Losses, denoising queries and target assignment are training-only and not part of this package.
 """
@@ -213,8 +214,7 @@ class _ConvModule(nn.Module):
         return self.activate(self.bn(self.conv(x)))
 
 
-def _compute_dtype(precision):
-    return torch.float32 if precision == "fp32" else torch.bfloat16
+_compute_dtype = ops.compute_dtype
 
 
 class _torch_math:
@@ -274,7 +274,7 @@ class _CmtHeadBase(nn.Module):
         self.precision = "bf16"
         # bench.py times "CmtTransformer+PE" from the post-shared_conv BEV map (SURVEY.md 8(d)); set False then
         self.apply_shared_conv = True
-        # bf16 mode: shared_conv runs as a tcgen05 implicit GEMM whose epilogue writes the BEV token rows directly
+        # bf16 / fp16 modes: shared_conv runs as a tcgen05 implicit GEMM whose epilogue writes the BEV token rows directly
         # (cmt_shared_conv_tokens); False keeps torch's Conv2d + BatchNorm2d + ReLU (always used in fp32 mode)
         self.fuse_shared_conv = True
 
@@ -303,8 +303,10 @@ class _CmtHeadBase(nn.Module):
         nn.init.uniform_(self.reference_points.weight.data, 0, 1)
 
     def set_precision(self, precision):
-        """'bf16' (tcgen05 kernels, default) or 'fp32' (CUDA-core verification mode)."""
-        assert precision in ("bf16", "fp32")
+        """'bf16' (tcgen05 kernels, default), 'fp16' (tcgen05 kernels with fp16 operands: 3 more mantissa bits, the
+        attention core at the reference's flash-attn precision) or 'fp32' (CUDA-core verification mode).  The task heads
+        are fp32-grade in every mode."""
+        _compute_dtype(precision)   # rejects an unknown precision
         self.precision = precision
         self.transformer.set_precision(precision)
         self._cache.clear()
@@ -368,16 +370,17 @@ class _CmtHeadBase(nn.Module):
 
     # -- shared_conv (cmt_head.py:280-287, applied :481) -------------------------------------
     def _shared_conv_folded(self):
-        """conv weight with the eval-mode BatchNorm scale folded in, tap-major [Cout, 9*Cin] bf16, and the remaining
-        per-channel bias: BN(conv(x)) = conv(x; w * s) + (beta - mean * s), s = gamma / sqrt(var + eps)."""
+        """conv weight with the eval-mode BatchNorm scale folded in, tap-major [Cout, 9*Cin] in the compute dtype (bf16 or
+        fp16), and the remaining per-channel bias: BN(conv(x)) = conv(x; w * s) + (beta - mean * s), s = gamma / sqrt(var + eps)."""
         conv, bn = self.shared_conv.conv, self.shared_conv.bn
-        key = ("conv", conv.weight._version, conv.weight.data_ptr(), bn.weight._version, bn.bias._version,
+        dt = _compute_dtype(self.precision)
+        key = ("conv", dt, conv.weight._version, conv.weight.data_ptr(), bn.weight._version, bn.bias._version,
                bn.running_mean._version, bn.running_var._version, bn.running_mean.data_ptr())
         hit = self._cache.get("shared_conv")
         if hit is None or hit[0] != key:
             s = bn.weight.detach().float() / torch.sqrt(bn.running_var.detach().float() + bn.eps)
             w = conv.weight.detach().float() * s[:, None, None, None]                  # [Cout, Cin, 3, 3]
-            w = w.permute(0, 2, 3, 1).reshape(w.shape[0], -1).to(torch.bfloat16).contiguous()   # [Cout, (ky, kx, c)]
+            w = w.permute(0, 2, 3, 1).reshape(w.shape[0], -1).to(dt).contiguous()   # [Cout, (ky, kx, c)]
             b = (bn.bias.detach().float() - bn.running_mean.detach().float() * s).contiguous()
             hit = (key, (w, b))
             self._cache["shared_conv"] = hit
@@ -385,11 +388,11 @@ class _CmtHeadBase(nn.Module):
 
     def _apply_shared_conv_to(self, x):
         """The BEV map the transformer consumes: the input itself (bench scope), a BevTokenSource for the fused
-        implicit-GEMM path (bf16 mode), or torch's conv + BN + ReLU in fp32."""
+        implicit-GEMM path (bf16 and fp16 modes), or torch's conv + BN + ReLU in fp32."""
         if not self.apply_shared_conv:
             return x
         conv = self.shared_conv.conv
-        if (self.precision == "bf16" and self.fuse_shared_conv and conv.kernel_size == (3, 3) and conv.in_channels % 64 == 0
+        if (self.precision in ("bf16", "fp16") and self.fuse_shared_conv and conv.kernel_size == (3, 3) and conv.in_channels % 64 == 0
                 and conv.out_channels % 32 == 0):
             from .cmt_transformer import BevTokenSource
             w, b = self._shared_conv_folded()

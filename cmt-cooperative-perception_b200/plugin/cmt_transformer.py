@@ -18,8 +18,7 @@ from .petr_transformer import PETRMultiheadFlashAttention, build_transformer_lay
 from .registry import TRANSFORMER
 
 
-def _compute_dtype(precision):
-    return torch.float32 if precision == "fp32" else torch.bfloat16
+_compute_dtype = ops.compute_dtype
 
 
 class RvPosRows:
@@ -42,7 +41,7 @@ class BevTokenSource:
 
     def __init__(self, x_raw, w, bias):
         self.x = x_raw                      # [B, Cin, H, W] fp32 | bf16 | fp16
-        self.w = w                          # [Cout, 9*Cin] bf16, tap-major, BN scale folded in
+        self.w = w                          # [Cout, 9*Cin] in the compute dtype (bf16 | fp16), tap-major, BN scale folded in
         self.bias = bias                    # [Cout] fp32
         self.shape = (x_raw.shape[0], w.shape[0], x_raw.shape[2], x_raw.shape[3])
         self.device = x_raw.device
@@ -78,7 +77,7 @@ class _CmtTransformerBase(nn.Module):
         self._is_init = True
 
     def set_precision(self, precision):
-        assert precision in ("bf16", "fp32")
+        _compute_dtype(precision)   # rejects an unknown precision
         self.precision = precision
         for m in self.modules():
             if hasattr(m, "precision"):
@@ -146,11 +145,11 @@ class _CmtTransformerBase(nn.Module):
             dev = x_bev.device
             xk = torch.empty((B, hi - lo, C), dtype=dt, device=dev)
             xv = torch.empty((B, hi - lo, C), dtype=dt, device=dev)
-            key = (tuple(x_bev.x.shape), str(dev))
+            key = (tuple(x_bev.x.shape), str(dev), dt)
             if self._xp is None or self._xp[0] != key:   # zero-padded channel-last operand: zeroed once, interior rewritten per call
-                self._xp = (key, ops.nchw_to_padded_nhwc(x_bev.x))
+                self._xp = (key, ops.nchw_to_padded_nhwc(x_bev.x, dtype=dt))
             else:
-                ops.nchw_to_padded_nhwc(x_bev.x, self._xp[1])
+                ops.nchw_to_padded_nhwc(x_bev.x, self._xp[1], dtype=dt)
             if lo < n_bev:
                 ops.shared_conv_tokens(self._xp[1], x_bev.w, x_bev.bias, bev_pos, xk, xv, Hb, Wb, tok_range=(lo, min(hi, n_bev)))
             if x_img is not None and hi > n_bev:
@@ -160,7 +159,7 @@ class _CmtTransformerBase(nn.Module):
             xk, xv = ops.gather_tokens(x_bev, x_img, bev_pos, rv_pos, B, V, out_dtype=dt,
                                        tok_range=None if group is None else (lo, hi), rv_rows=rv_rows)
         wk, bk, wv, bv = self._stacked_kv_weights()
-        kn2 = torch.zeros((B, L, H), dtype=torch.float32, device=xk.device) if dt == torch.bfloat16 else None
+        kn2 = torch.zeros((B, L, H), dtype=torch.float32, device=xk.device) if dt != torch.float32 else None
         k = ops.project_keys(xk, wk, bk, L, H, norm2_max=kn2)
         vt = ops.project_values_t(xv, wv, bv, L, H)
         return KVCache(k, vt, hi - lo, group, k_norm2=kn2, peer=self._peer_exchange if (group is not None and self.kv_split_peer) else None), xv

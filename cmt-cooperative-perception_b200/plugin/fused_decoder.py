@@ -8,12 +8,12 @@ sequence-first and back around every attention, petr_transformer.py:307-319):
 
   per layer (15 launches instead of ~60 eager ones):
     self-attention   Q/K/V^T projections (3 GEMMs) -> flash attention kernel -> out-proj GEMM
-    norm0            fused (x + sa) LayerNorm, also emits bf16(x1 + query_pos) for the next projection
+    norm0            fused (x + sa) LayerNorm, also emits lp(x1 + query_pos) for the next projection (lp: bf16 / fp16)
     cross-attention  Q GEMM -> flash attention over the hoisted K/V cache -> out-proj GEMM
-    norm1            fused (x1 + ca) LayerNorm, also emits bf16(x2) for the FFN
+    norm1            fused (x1 + ca) LayerNorm, also emits lp(x2) for the FFN
     ffn              GEMM+bias+ReLU, GEMM+bias
     norm2 (+post)    fused (x2 + ffn) LayerNorm + the shared post_norm written straight into the stacked
-                     [L,B,Nq,C] output, also emits bf16(x3), bf16(x3 + query_pos) for the next layer
+                     [L,B,Nq,C] output, also emits lp(x3), lp(x3 + query_pos) for the next layer
 """
 from __future__ import annotations
 
@@ -21,7 +21,7 @@ import torch
 import torch.nn as nn
 
 from .. import ops
-from .attention import KVCache, _Q_SCALE, _compute_dtype
+from .attention import KVCache, _Q_SCALE
 
 _STD_ORDER = ("self_attn", "norm", "cross_attn", "norm", "ffn", "norm")
 
@@ -30,7 +30,9 @@ _STD_ORDER = ("self_attn", "norm", "cross_attn", "norm", "ffn", "norm")
 SKIP_ZERO_TARGET_SELF_ATTENTION = True
 
 # diagnostics for bench.py: the operand-norm maxima of the last forward, (q_norm2 [L,B,H], [k_norm2 [B_i,L,H] per cache]) or None.
-# An attention item (layer, frame, head) takes the static-shift kernel iff sqrt(qn * kn) * 1.0079 + 1e-3 <= 60.
+# An attention item (layer, frame, head) takes the static-shift kernel iff sqrt(qn * kn) * 1.0079 + 1e-3 <= limit, with
+# limit STATIC_LIMIT[dtype] (the largest |score| whose weight 2^score is a normal number of the dtype).
+STATIC_LIMIT = {torch.bfloat16: 60.0, torch.float16: 14.0}
 last_norms = None
 
 
@@ -112,7 +114,7 @@ def run(decoder, query_pos: torch.Tensor, cache, precision: str) -> torch.Tensor
 
 def _run(decoder, query_pos, caches, precision):
     cache = caches[0]
-    dt = _compute_dtype(precision)
+    dt = ops.compute_dtype(precision)
     B, Nq, C = query_pos.shape
     L = len(decoder.layers)
     H = decoder.layers[0].attentions[0].attn.num_heads
@@ -129,7 +131,7 @@ def _run(decoder, query_pos, caches, precision):
 
     # max |q|^2 per (layer, frame, head) of the cross-attention queries: with cache.k_norm2 the attention kernel gets a
     # bound on every score and drops the running row maximum (ops.cross_attn)
-    static_shift = all(c.k_norm2 is not None for c in caches) and dt == torch.bfloat16
+    static_shift = all(c.k_norm2 is not None for c in caches) and dt in STATIC_LIMIT
     qn2 = torch.zeros((L, B, H), dtype=torch.float32, device=dev) if static_shift else None
 
     global last_norms

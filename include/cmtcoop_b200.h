@@ -10,7 +10,9 @@
  *     no exception crosses this boundary;
  *   - sm_100a only: on any other device every launch entry returns CMT_ERR_ARCH.
  *     There is no CPU or generic-CUDA fallback.
- *   - dtype codes: CMT_F32 / CMT_BF16.
+ *   - dtype codes: CMT_F32 / CMT_BF16 / CMT_F16.  Three compute precisions: bf16 and fp16 run the tensor-core
+ *     kernels (same rate; fp16 has 3 more mantissa bits, bf16 the fp32 exponent range), fp32 the CUDA-core
+ *     verification kernels.
  */
 #ifndef CMTCOOP_B200_H_
 #define CMTCOOP_B200_H_
@@ -30,14 +32,15 @@ extern "C" {
 
 #define CMT_F32 0
 #define CMT_BF16 1
-#define CMT_F16 2       /* feature maps entering cmt_gather_tokens / cmt_nchw_to_padded_nhwc only */
+#define CMT_F16 2       /* fp16: a compute dtype of every entry below that takes one (never of the task-head chain:
+                           cmt_split3_bf16 / cmt_gemm_segmented / cmt_task_head_tail), and a feature-map dtype */
 #define CMT_BF16_SIMT 3 /* cmt_cross_attn_fwd only: bf16 operands through the fp32 CUDA-core kernel (comparator) */
 
 /* flags of cmt_gemm_bias_act */
 #define CMT_GEMM_RELU 1          /* out = max(out, 0)                                  */
 #define CMT_GEMM_BIAS_PER_ROW 2  /* bias indexed by output row (default: by column)    */
-#define CMT_GEMM_FORCE_SIMT 4    /* fp32 CUDA-core kernel even for bf16 operands       */
-#define CMT_GEMM_TRANSPOSE_OUT 8 /* store C^T inside each column block (bf16 tensor-core path only) */
+#define CMT_GEMM_FORCE_SIMT 4    /* fp32 CUDA-core kernel even for bf16 operands (not fp16) */
+#define CMT_GEMM_TRANSPOSE_OUT 8 /* store C^T inside each column block (16-bit tensor-core path only) */
 
 /* flags of cmt_add_layernorm */
 #define CMT_LN_X_ROW_BROADCAST 1 /* x is ONE row [C] shared by all M rows (decoder layer 0: see cmt_add_layernorm) */
@@ -51,7 +54,7 @@ int cmt_check_device(int dev);
  * Replaces the eager meshgrid/einsum/normalise block of CmtHead._rv_pe
  * (models/dense_heads/cmt_head.py:417-432, same code cmt_head_coop.py:283-298).
  * img2lidar: [n_cam,4,4] fp32 row-major = float32(inv_float64(lidar2img)) (cmt_head.py:428-429).
- * out:       [n_cam,H,W,D*3] (feature index 3*k+c, cmt_head.py:433), fp32 or bf16.
+ * out:       [n_cam,H,W,D*3] (feature index 3*k+c, cmt_head.py:433), fp32, bf16 or fp16.
  * pc_range:  6 host floats.  Token index inside a frame is cam*H*W + i*W + j. */
 int cmt_ray_pe(const float* img2lidar, void* out, int n_cam, int H, int W, int D, float pad_h,
                float pad_w, const float* pc_range_host, int out_dtype, void* stream);
@@ -60,20 +63,21 @@ int cmt_ray_pe(const float* img2lidar, void* out, int n_cam, int H, int W, int D
  * Replaces CmtHead._rv_query_embed up to the rv_embedding MLP (cmt_head.py:439-464).
  * ref:       [B,Nq,3] fp32 in [0,1] (already inverse_sigmoid(...).sigmoid()'ed, :470)
  * lidar2img: [B,V,4,4] fp32, img2lidar: [B,V,4,4] fp32
- * out:       [B,V,Nq,D*3] (fp32|bf16), mask: [B,V,Nq] fp32 (1.0 inside image & z>0). */
+ * out:       [B,V,Nq,D*3] (fp32|bf16|fp16), mask: [B,V,Nq] fp32 (1.0 inside image & z>0). */
 int cmt_ray_query_pe(const float* ref, const float* lidar2img, const float* img2lidar, void* out,
                      float* mask, int B, int V, int Nq, int D, float pad_h, float pad_w,
                      const float* pc_range_host, int out_dtype, void* stream);
 
 /* out[b,n,:] = base[b,n,:] + sum_v mask[b,v,n] * emb[b,v,n,:]  (cmt_head.py:466 and the `bev + rv` of :492).
- * emb fp32|bf16, out fp32; base (nullable) fp32 at base + b*base_bstride + n*C (base_bstride = 0: one [Nq,C]
+ * emb fp32|bf16|fp16, out fp32; base (nullable) fp32 at base + b*base_bstride + n*C (base_bstride = 0: one [Nq,C]
  * embedding shared by every frame -- in eval the BEV query embedding depends on the weights only). */
 int cmt_masked_view_sum(const void* emb, const float* mask, const float* base, int64_t base_bstride, float* out,
                         int B, int V, int Nq, int C, int emb_dtype, void* stream);
 
 /* ---- sine/cosine BEV embedding ------------------------------------------------------
  * pos2embed (cmt_head.py:40-50) including its `dim_t = 2*(i//2)/F + 1` divisor.
- * pos: [N,pos_stride] fp32 (only columns 0 (x) and 1 (y) are read); out: [N,2F] = cat(emb(y), emb(x)). */
+ * pos: [N,pos_stride] fp32 (only columns 0 (x) and 1 (y) are read); out: [N,2F] = cat(emb(y), emb(x)),
+ * fp32|bf16|fp16. */
 int cmt_pos2embed(const float* pos, void* out, int N, int pos_stride, int F, int out_dtype,
                   void* stream);
 
@@ -92,7 +96,7 @@ int cmt_pos2embed(const float* pos, void* out, int N, int pos_stride, int F, int
  * [B, tok_end - tok_begin, C] (0, N_kv = everything; a sub-range = this rank's share of a KV-token
  * split).  rv_rows > 0: rv_pos holds only rows [rv_tok0, rv_tok0 + rv_rows) of every frame's V*n_img image tokens,
  * [B, rv_rows, C] (the rank computed the rv-PE MLP for its own tokens only); rv_rows = 0: all of them.
- * out dtype fp32|bf16. */
+ * out dtype fp32|bf16|fp16. */
 int cmt_gather_tokens(const void* x_bev, const void* x_img, const float* bev_pos,
                       const float* rv_pos, void* xk, void* xv, int B, int C, int n_bev, int V,
                       int n_img, int tok_begin, int tok_end, int rv_tok0, int rv_rows, int feat_dtype, int out_dtype,
@@ -109,14 +113,15 @@ int cmt_gather_tokens(const void* x_bev, const void* x_img, const float* bev_pos
  * [.., H, tokens, 32] layout the attention kernel reads.  With CMT_GEMM_TRANSPOSE_OUT the block is
  * written transposed,
  *     C + z*strideC + (n / cb)*cb_stride + (n % cb)*ldc + m
- * which with cb = 32, ldc = ld gives the token-contiguous V^T layout [.., H, 32, ld] (bf16 operands and
+ * which with cb = 32, ldc = ld gives the token-contiguous V^T layout [.., H, 32, ld] (16-bit operands and
  * output, cb % 32 == 0, N % 32 == 0, N <= 1984).
- * norm2_max (bf16 path, or NULL): [batch][N/32] fp32, zero-initialised by the caller; the epilogue raises
+ * norm2_max (16-bit path, or NULL): [batch][N/32] fp32, zero-initialised by the caller; the epilogue raises
  * entry (z, n/32) to the largest squared norm of a row's 32-column block (one attention head of one
  * query/key).  cmt_cross_attn_fwd turns the two maxima into a bound on every score (see there).
- * in_dtype bf16 -> TMA + tcgen05 kernel (fp32 accumulate in TMEM); in_dtype fp32 -> fp32
- * CUDA-core kernel (verification mode).  Requirements for bf16: K % 8 == 0, lda/ldb % 8 == 0,
- * 16-byte aligned bases, and (cb >= N or cb % 32 == 0). */
+ * in_dtype bf16 or fp16 -> TMA + tcgen05 kernel (fp32 accumulate in TMEM); in_dtype fp32 -> fp32
+ * CUDA-core kernel (verification mode).  out_dtype: fp32 or the 16-bit dtype of the operands (fp32 operands: fp32 or
+ * bf16).  Requirements for 16-bit operands: K % 8 == 0, lda/ldb % 8 == 0, 16-byte aligned bases, and
+ * (cb >= N or cb % 32 == 0). */
 int cmt_gemm_bias_act(const void* A, const void* B, const float* bias, void* C, int M, int N,
                       int K, int64_t lda, int64_t ldb, int64_t ldc, int64_t cb, int64_t cb_stride,
                       int batch, int64_t strideA, int64_t strideB, int64_t strideC, float alpha,
@@ -139,20 +144,21 @@ int cmt_gemm_segmented(const void* A, const void* B, const float* bias, void* C,
  * Replaces ConvModule(conv3x3 no bias, BN2d, ReLU) of CmtHead (models/dense_heads/cmt_head.py:280-287, applied :481,
  * coop: cmt_head_coop.py:343) TOGETHER with the BEV half of the token rearrange / pos add
  * (models/utils/cmt_transformer.py:105-110, petr_transformer.py:296-299): the NCHW fp32 map never exists.
- * Step 1, cmt_nchw_to_padded_nhwc: x [B,C,H,W] (fp32|bf16|fp16) -> out bf16 [B][2*guard_rows + (H+2)*(W+2)][C], pixel
+ * dtype (out_dtype / dtype, the trailing argument of both entries): CMT_BF16 or CMT_F16, the operand and token dtype.
+ * Step 1, cmt_nchw_to_padded_nhwc: x [B,C,H,W] (fp32|bf16|fp16) -> out (dtype) [B][2*guard_rows + (H+2)*(W+2)][C], pixel
  *   (y,x) in row guard_rows + (y+1)*(W+2) + (x+1); only interior rows are written (the caller zero-fills `out` once),
  *   guard_rows >= W + 3.
- * Step 2, cmt_shared_conv_tokens: w bf16 [Cout][9*Cin], tap-major (w[o][(ky*3+kx)*Cin + c] = conv.weight[o][c][ky][kx] *
+ * Step 2, cmt_shared_conv_tokens: w (dtype) [Cout][9*Cin], tap-major (w[o][(ky*3+kx)*Cin + c] = conv.weight[o][c][ky][kx] *
  *   bn_scale[o]), bias fp32 [Cout] = bn.bias - bn.running_mean * bn_scale, bev_pos fp32 [H*W, Cout];
  *   for every frame b and token t = y*W + x in [tok_begin, tok_end):
- *     v = ReLU(conv(x)[b,:,y,x] + bias);  xv[b][t - tok_begin][:] = bf16(v);  xk[b][t - tok_begin][:] = bf16(v + bev_pos[t])
+ *     v = ReLU(conv(x)[b,:,y,x] + bias);  xv[b][t - tok_begin][:] = dtype(v);  xk[b][t - tok_begin][:] = dtype(v + bev_pos[t])
  *   with out_frame_stride elements between frames (N_kv * Cout: the image tokens follow, cmt_gather_tokens with
  *   x_bev = NULL).  Cin % 64 == 0, Cout % 32 == 0, Cout <= 1984. */
 int cmt_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, int W, int guard_rows, int in_dtype,
-                            void* stream);
+                            void* stream, int out_dtype);
 int cmt_shared_conv_tokens(const void* xp, const void* w, const float* bias, const float* bev_pos, void* xk, void* xv,
                            int B, int Cin, int Cout, int H, int W, int guard_rows, int64_t out_frame_stride,
-                           int tok_begin, int tok_end, void* stream);
+                           int tok_begin, int tok_end, void* stream, int dtype);
 
 /* ---- K3: flash cross-attention ------------------------------------------------------
  * Replaces flash_attn_unpadded_kvpacked_func as called by FlashAttention.forward
@@ -167,14 +173,15 @@ int cmt_shared_conv_tokens(const void* xp, const void* w, const float* bias, con
  *      sequence and giving it weight zero are the same softmax.  A query with no attended key gets o = 0.
  * q_norm2_max [B*H], k_norm2_max (entry (b,h) at b*kn_bstride + h), both or neither NULL: upper bounds of
  *      |q|^2 and |k|^2 per (frame, head) as written by cmt_gemm_bias_act(norm2_max).  |q.k| <= |q||k| bounds
- *      every score of the (frame, head); when that bound is <= 60 (log2 units) the bf16 kernel uses it as a
- *      fixed softmax shift and skips the running row maximum and the accumulator rescale (same result: the
- *      softmax is shift-invariant, and all weights stay normal numbers); larger bounds and NULL use the
- *      online softmax.
+ *      every score of the (frame, head); when that bound is <= 60 (bf16) or <= 14 (fp16; log2 units) the
+ *      tensor-core kernel uses it as a fixed softmax shift and skips the running row maximum and the accumulator
+ *      rescale (same result: the softmax is shift-invariant, and all weights stay normal numbers of the dtype);
+ *      larger bounds and NULL use the online softmax.
  * lse: [B,H,Nq] fp32 natural-log sum-exp of the scaled scores over the attended tokens, or NULL
- * dtype bf16 -> tcgen05 kernel, work split over all SMs along the KV axis with partials in
- * `workspace` (cmt_cross_attn_workspace_bytes) merged by a second kernel; dtype fp32 -> fp32
- * CUDA-core kernel.  Head dim is fixed at 32 (256/8, the only value the reference configs use). */
+ * dtype bf16 or fp16 (q, k, vt and the softmax weights P) -> tcgen05 kernel, work split over all SMs along the KV
+ * axis with partials in `workspace` (cmt_cross_attn_workspace_bytes) merged by a second kernel; dtype fp32 -> fp32
+ * CUDA-core kernel.  o_dtype: fp32 or the operand dtype (fp16 only with fp16 operands).  Head dim is fixed at 32
+ * (256/8, the only value the reference configs use). */
 size_t cmt_cross_attn_workspace_bytes(int B, int H, int Nq, int n_kv_tokens);
 int cmt_cross_attn_fwd(const void* q, const void* k, const void* vt, void* o, float* lse, int B,
                        int H, int Nq, int N_kv, int kv_begin, int kv_end, int64_t q_ld,
@@ -185,7 +192,7 @@ int cmt_cross_attn_fwd(const void* q, const void* k, const void* vt, void* o, fl
 
 /* Log-sum-exp merge of G partial attention results (KV-token split across GPUs or streams):
  * part g: o [B,Nq,H*32] fp32 at o_parts + g*o_gstride, lse [B,H,Nq] fp32 (natural log) at lse_parts + g*lse_gstride
- * (strides in elements; 0 = densely stacked [G,...] arrays) -> o [B,Nq,H*32], lse (nullable).  With
+ * (strides in elements; 0 = densely stacked [G,...] arrays) -> o [B,Nq,H*32] (o_dtype fp32|bf16|fp16), lse (nullable).  With
  * o_gstride = lse_gstride = B*Nq*H*32 + B*H*Nq and lse_parts = o_parts + B*Nq*H*32 the parts are the packed
  * (O | LSE) records of ONE all-gather per decoder layer. */
 int cmt_lse_merge(const float* o_parts, const float* lse_parts, void* o, float* lse, int G, int B,
@@ -195,7 +202,7 @@ int cmt_lse_merge(const float* o_parts, const float* lse_parts, void* o, float* 
  * KV-token split.  records[g] / ctx[g] / arrive[g] are HOST arrays of G <= 8 device pointers, all into memory mapped
  * into every rank of the group (the caller maps it, e.g. torch symmetric memory): rank g's packed (O | LSE) record of
  * this exchange -- o [B,Nq,H*32] fp32 followed by lse [B,H,Nq] fp32 --, rank g's context buffer [B,Nq,H*32] (o_dtype)
- * and rank g's block of 16 uint32 counters; `state` points at two uint32 {exchange number, finished blocks} in LOCAL
+ * (fp32|bf16|fp16) and rank g's block of 16 uint32 counters; `state` points at two uint32 {exchange number, finished blocks} in LOCAL
  * memory; counters and state are zero before the first exchange.  The kernel announces the local record to all ranks,
  * waits for theirs, merges this rank's 1/G of the rows straight from the G records (remote ones read through NVLink),
  * stores them into EVERY rank's context buffer, and returns once all ranks' rows have landed in ctx[rank]
@@ -215,7 +222,7 @@ int cmt_lse_merge_peer(const void* const* records, void* const* ctx, void* const
  * next projection needs.  x, r (nullable), add (nullable): [M,C] fp32; C must be 256.
  *   y    = LN(x + r; gamma, beta, eps)            fp32, required
  *   y2   = LN(y; gamma2, beta2, eps)              fp32, optional (NULL)
- *   ylp  = cast(y), yadd = cast(y + add)          lp_dtype (fp32|bf16), each optional (NULL)
+ *   ylp  = cast(y), yadd = cast(y + add)          lp_dtype (fp32|bf16|fp16), each optional (NULL)
  * flags & CMT_LN_X_ROW_BROADCAST: x is a single row [C] used for every output row.  Decoder layer 0 runs on the zero
  * target (cmt_transformer.py:114), so its self-attention attends over values that are all equal to the value bias and
  * returns out_proj(b_v) for every query whatever the weights of the softmax: that one row is the whole `x + attn_out`. */

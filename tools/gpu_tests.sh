@@ -17,3 +17,4 @@ run heads tests/test_gpu_heads.py
 run decoder tests/test_gpu_decoder.py
 run multi tests/test_gpu_multi.py
 run decode tests/test_gpu_bbox_decode.py
+run fp16 tests/test_gpu_fp16.py
