@@ -44,8 +44,8 @@ SIGNATURES = {
     "cmt_coop_max": (_i, [_vp, _vp, _vp, _i64, _vp]),
     "cmt_add_layernorm": (_i, [_vp, _vp, _vp, _vp, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp]),
     "cmt_task_head_tail": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "cmt_split3_bf16": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _i, _i64, _vp]),
-    "cmt_bbox_topk_decode": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "cmt_split3_bf16": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _i, _i64, _vp, _vp]),
+    "cmt_bbox_topk_decode": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i]),
     "cmt_debug_attn_timing": (_i, [_vp]),
 }
 

@@ -130,7 +130,7 @@ using namespace cmt;
 
 extern "C" {
 
-int cmt_version(void) { return 101; }
+int cmt_version(void) { return 102; }
 
 const char* cmt_last_error_string(void) { return g_err; }
 
@@ -390,9 +390,10 @@ int cmt_task_head_tail(const float* h, const float* gamma, const float* beta, co
 }
 
 int cmt_split3_bf16(const float* a, const float* b, void* out, float* merged, int64_t Z, int Nq, int C, int frames,
-                    int64_t layer_stride_rows, void* stream) {
+                    int64_t layer_stride_rows, void* stream, const uint8_t* node_valid) {
     CMT_REQUIRE_DEVICE();
-    return launch_split3(a, b, out, merged, Z, Nq, C, frames, layer_stride_rows, static_cast<cudaStream_t>(stream));
+    return launch_split3(a, b, out, merged, Z, Nq, C, frames, layer_stride_rows, node_valid,
+                         static_cast<cudaStream_t>(stream));
 }
 
 int cmt_debug_attn_timing(void* dev_buf_i64) { return cmt::tc_attn_set_timing_buffer(static_cast<long long*>(dev_buf_i64)); }
@@ -421,12 +422,12 @@ int cmt_add_layernorm(const float* x, const float* r, const float* gamma, const 
 int cmt_bbox_topk_decode(const float* const* task_ptrs_host, const int* task_classes_host, int T, int B, int Nq,
                          int num_classes, int max_num, const float* post_center_range_host, float score_threshold,
                          int use_score_threshold, int bottom_center, float* boxes, float* scores, int64_t* labels,
-                         int32_t* count, int64_t* topk_index, void* stream) {
+                         int32_t* count, int64_t* topk_index, void* stream, const uint8_t* node_valid, int n_nodes) {
     CMT_REQUIRE_DEVICE();
     return launch_bbox_topk_decode(task_ptrs_host, task_classes_host, T, B, Nq, num_classes, max_num, post_center_range_host,
                                    score_threshold, use_score_threshold, bottom_center, boxes, scores,
                                    reinterpret_cast<long long*>(labels), count, reinterpret_cast<long long*>(topk_index),
-                                   static_cast<cudaStream_t>(stream));
+                                   node_valid, n_nodes, static_cast<cudaStream_t>(stream));
 }
 
 int cmt_coop_max(const float* a, const float* b, float* out, int64_t n, void* stream) {

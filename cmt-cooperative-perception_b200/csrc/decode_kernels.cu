@@ -2,6 +2,8 @@
 // (multi_task_bbox_coder.py:46-141, util.py:37-68, z shift of cmt_head.py:912).
 //
 // One 1024-thread CTA per frame:
+//   0. with a node mask, a frame none of whose nodes is present writes the "nothing kept" state (count 0, zero boxes
+//      and scores, label and top-k index -1) and returns;
 //   1. score = 1 / (1 + expf(-logit)) of every (query, class) into shared memory as an order-preserving uint32 key
 //      (NaN -> one key above +inf, as torch ranks it);
 //   2. radix select, four 8-bit digits from the top, finds the K-th largest key; warp-aggregated shared-memory
@@ -42,6 +44,8 @@ struct DecodeParams {
     long long* labels;
     int* count;
     long long* topk_index;
+    const uint8_t* node_valid;   // [n_nodes, B] or nullptr: a frame none of whose nodes delivered keeps nothing
+    int n_nodes;
 };
 
 // torch's CUDA sigmoid for fp32: one / (one + std::exp(-a))
@@ -86,6 +90,23 @@ static __device__ __forceinline__ uint32_t block_scan(uint32_t v, uint32_t* warp
     return r;
 }
 
+// The node-mask check and the empty-frame store, out of line: inlined, they raise the kernel from 37 to 40 registers.
+static __device__ __noinline__ bool frame_present(const DecodeParams& p, int b) {
+    bool any = false;
+    for (int i = 0; i < p.n_nodes; ++i) any |= p.node_valid[static_cast<long long>(i) * gridDim.x + b] != 0;
+    return any;
+}
+static __device__ __noinline__ void write_empty_frame(const DecodeParams& p, int b, int tid) {
+    if (tid < p.K) {
+        const long long o = static_cast<long long>(b) * p.K + tid;
+        for (int j = 0; j < 9; ++j) p.boxes[o * 9 + j] = 0.0f;
+        p.scores[o] = 0.0f;
+        p.labels[o] = -1;
+        p.topk_index[o] = -1;
+    }
+    if (tid == 0) p.count[b] = 0;
+}
+
 __global__ void __launch_bounds__(DEC_THREADS, 1) bbox_topk_decode_kernel(const __grid_constant__ DecodeParams p) {
     extern __shared__ __align__(16) unsigned char dsm[];
     unsigned long long* cand = reinterpret_cast<unsigned long long*>(dsm);         // [P] (key << 32) | ~index
@@ -97,6 +118,12 @@ __global__ void __launch_bounds__(DEC_THREADS, 1) bbox_topk_decode_kernel(const 
     const int tid = threadIdx.x, lane = tid & 31;
     const int b = blockIdx.x;
     const int N = p.N, C = p.C, K = p.K;
+
+    // 0. a frame none of whose nodes delivered
+    if (p.node_valid != nullptr && !frame_present(p, b)) {
+        write_empty_frame(p, b, tid);
+        return;
+    }
 
     // 1. keys
     for (int n = tid; n < N; n += DEC_THREADS) {
@@ -230,9 +257,11 @@ __global__ void __launch_bounds__(DEC_THREADS, 1) bbox_topk_decode_kernel(const 
 int launch_bbox_topk_decode(const float* const* task_ptrs, const int* task_classes, int T, int B, int Nq, int num_classes,
                             int max_num, const float* post_center_range, float score_threshold, int use_score_threshold,
                             int bottom_center, float* boxes, float* scores, long long* labels, int* count,
-                            long long* topk_index, cudaStream_t stream) {
+                            long long* topk_index, const uint8_t* node_valid, int n_nodes, cudaStream_t stream) {
     CMT_CHECK_ARG(task_ptrs && task_classes && post_center_range, "cmt_bbox_topk_decode: null host array");
     CMT_CHECK_ARG(boxes && scores && labels && count && topk_index, "cmt_bbox_topk_decode: null output");
+    CMT_CHECK_ARG(node_valid == nullptr || n_nodes >= 1, "cmt_bbox_topk_decode: node_valid needs n_nodes >= 1 (got %d)",
+                  n_nodes);
     CMT_CHECK_ARG(T >= 1 && T <= CMT_BOX_DECODE_MAX_TASKS, "cmt_bbox_topk_decode: %d tasks (1..%d supported)", T,
                   CMT_BOX_DECODE_MAX_TASKS);
     CMT_CHECK_ARG(B >= 1 && Nq >= 1, "cmt_bbox_topk_decode: bad shape B=%d Nq=%d", B, Nq);
@@ -273,6 +302,8 @@ int launch_bbox_topk_decode(const float* const* task_ptrs, const int* task_class
     p.labels = labels;
     p.count = count;
     p.topk_index = topk_index;
+    p.node_valid = node_valid;
+    p.n_nodes = n_nodes;
     const size_t smem = sizeof(unsigned long long) * p.P + sizeof(uint32_t) * static_cast<size_t>(N);
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(bbox_topk_decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,

@@ -88,12 +88,12 @@ int launch_task_head_tail(const float* h, const float* gamma, const float* beta,
                           const int* dec_comp, const float* dec_scale, const float* dec_offset, const long long* head_off_host,
                           const int* head_cout_host, cudaStream_t stream);
 int launch_split3(const float* a, const float* b, void* out, float* merged, long long Z, int Nq, int C, int frames,
-                  long long layer_stride_rows, cudaStream_t stream);
+                  long long layer_stride_rows, const uint8_t* node_valid, cudaStream_t stream);
 // decode_kernels.cu
 int launch_bbox_topk_decode(const float* const* task_ptrs, const int* task_classes, int T, int B, int Nq, int num_classes,
                             int max_num, const float* post_center_range, float score_threshold, int use_score_threshold,
                             int bottom_center, float* boxes, float* scores, long long* labels, int* count,
-                            long long* topk_index, cudaStream_t stream);
+                            long long* topk_index, const uint8_t* node_valid, int n_nodes, cudaStream_t stream);
 // simt_kernels.cu
 int launch_simt_gemm(const GemmArgs& g, int batch, int in_dtype, cudaStream_t stream);
 int launch_simt_attn(const AttnArgs& a, int dtype, cudaStream_t stream);

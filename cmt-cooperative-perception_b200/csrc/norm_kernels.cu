@@ -144,6 +144,8 @@ int launch_add_layernorm(const float* x, const float* r, const float* gamma, con
 // element-wise max over the two nodes' stacks (cmt_head_coop.py:383-389).
 // in: a (and optionally b) [Z, Nq, 256] fp32; out: [Z, Nq + 2, 768] bf16 = [x1 | x2 | x3] per row, rows 0 and Nq + 1 of
 // every z are zero (the k = 3 convolutions over the query axis read them as padding).  One warp per output row.
+// node_valid (nullable, with b): [2, frames] per-frame presence of the two nodes; a frame takes max(a, b) with both,
+// the present node's rows with one, and zero rows with none.  An absent node's rows are not read.
 __device__ __forceinline__ float nan_to_num_f(float x) {
     if (x != x) return 0.0f;
     if (x == __int_as_float(0x7f800000)) return 3.4028234663852886e38f;
@@ -153,7 +155,8 @@ __device__ __forceinline__ float nan_to_num_f(float x) {
 
 __global__ void __launch_bounds__(256) split3_kernel(const float* __restrict__ a, const float* __restrict__ b,
                                                      __nv_bfloat16* __restrict__ out, float* __restrict__ merged, long long Z, int Nq,
-                                                     int frames, long long layer_stride) {
+                                                     int frames, long long layer_stride,
+                                                     const uint8_t* __restrict__ node_valid) {
     pdl_trigger();
     pdl_wait();
     const int lane = threadIdx.x & 31;
@@ -171,20 +174,23 @@ __global__ void __launch_bounds__(256) split3_kernel(const float* __restrict__ a
         }
         // input row of (layer, frame) = (z / frames, z % frames): layers may be further apart than frames * Nq rows (two
         // nodes' frames stacked in one decoder pass: a = first half of every layer, b = second half)
-        const long long src = ((z / frames) * layer_stride + (z % frames) * Nq + q) * 256 + lane * 8;
+        const long long frame = z % frames;
+        const long long src = ((z / frames) * layer_stride + frame * Nq + q) * 256 + lane * 8;
         const long long dense = (z * Nq + q) * 256 + lane * 8;
-        float v[8];
-        {
+        const bool has_a = node_valid == nullptr || node_valid[frame] != 0;
+        const bool has_b = b != nullptr && (node_valid == nullptr || node_valid[frames + frame] != 0);
+        float v[8] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
+        if (has_a) {
             const float4 p0 = *reinterpret_cast<const float4*>(a + src), p1 = *reinterpret_cast<const float4*>(a + src + 4);
             v[0] = p0.x; v[1] = p0.y; v[2] = p0.z; v[3] = p0.w; v[4] = p1.x; v[5] = p1.y; v[6] = p1.z; v[7] = p1.w;
-        }
 #pragma unroll
-        for (int i = 0; i < 8; ++i) v[i] = nan_to_num_f(v[i]);
-        if (b != nullptr) {
+            for (int i = 0; i < 8; ++i) v[i] = nan_to_num_f(v[i]);
+        }
+        if (has_b) {
             const float4 p0 = *reinterpret_cast<const float4*>(b + src), p1 = *reinterpret_cast<const float4*>(b + src + 4);
             const float w[8] = {p0.x, p0.y, p0.z, p0.w, p1.x, p1.y, p1.z, p1.w};
 #pragma unroll
-            for (int i = 0; i < 8; ++i) v[i] = fmaxf(v[i], nan_to_num_f(w[i]));
+            for (int i = 0; i < 8; ++i) v[i] = has_a ? fmaxf(v[i], nan_to_num_f(w[i])) : nan_to_num_f(w[i]);
         }
         if (merged != nullptr) {
             *reinterpret_cast<float4*>(merged + dense) = make_float4(v[0], v[1], v[2], v[3]);
@@ -210,8 +216,10 @@ __global__ void __launch_bounds__(256) split3_kernel(const float* __restrict__ a
 }
 
 int launch_split3(const float* a, const float* b, void* out, float* merged, long long Z, int Nq, int C, int frames,
-                  long long layer_stride_rows, cudaStream_t stream) {
+                  long long layer_stride_rows, const uint8_t* node_valid, cudaStream_t stream) {
     CMT_CHECK_ARG(a && out && Z > 0 && Nq > 0, "cmt_split3_bf16: bad arguments");
+    CMT_CHECK_ARG(node_valid == nullptr || (b != nullptr && frames > 0),
+                  "cmt_split3_bf16: node_valid needs the second stack b and frames > 0");
     if (frames <= 0) {   // dense input [Z, Nq, C]
         frames = 1;
         layer_stride_rows = Nq;
@@ -224,7 +232,8 @@ int launch_split3(const float* a, const float* b, void* out, float* merged, long
     long long blocks = (rows + 7) / 8;
     const long long cap = static_cast<long long>(device_sm_count()) * 16;
     if (blocks > cap) blocks = cap;
-    launch_pdl(split3_kernel, dim3(static_cast<int>(blocks)), dim3(256), 0, stream, a, b, reinterpret_cast<__nv_bfloat16*>(out), merged, Z, Nq, frames, layer_stride_rows);
+    launch_pdl(split3_kernel, dim3(static_cast<int>(blocks)), dim3(256), 0, stream, a, b, reinterpret_cast<__nv_bfloat16*>(out), merged, Z, Nq, frames, layer_stride_rows,
+               node_valid);
     CMT_LAUNCH_CHECK("cmt_split3_bf16");
     return CMT_OK;
 }

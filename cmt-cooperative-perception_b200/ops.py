@@ -110,6 +110,23 @@ def _cuda(t, name, dtype=None):
     return t
 
 
+def check_node_valid(node_valid, B, device, n_nodes=2):
+    """Host-side checks of a per-frame node mask: a torch.bool tensor [n_nodes, B] on `device` (n_nodes=None: any
+    n_nodes >= 1).  Row n, column b is True when node n delivered frame b.  The values are never read here, so the check
+    costs no device synchronisation.  Returns the mask, contiguous."""
+    if not isinstance(node_valid, torch.Tensor):
+        raise TypeError(f"node_valid must be a torch.bool tensor, got {type(node_valid).__name__}")
+    if node_valid.dtype != torch.bool:
+        raise TypeError(f"node_valid must be torch.bool, got {node_valid.dtype}")
+    rows = n_nodes if n_nodes is not None else (node_valid.shape[0] if node_valid.dim() == 2 else -1)
+    if node_valid.dim() != 2 or rows < 1 or tuple(node_valid.shape) != (rows, B):
+        want = f"[{n_nodes}, {B}]" if n_nodes is not None else f"[n_nodes, {B}]"
+        raise ValueError(f"node_valid must be {want}, got {list(node_valid.shape)}")
+    if node_valid.device != torch.device(device):
+        raise ValueError(f"node_valid must live on {torch.device(device)} (the features' device), got {node_valid.device}")
+    return node_valid.contiguous()
+
+
 def _pc(pc_range):
     return (ctypes.c_float * 6)(*[float(v) for v in pc_range])
 
@@ -585,11 +602,14 @@ def add_layernorm(x, r, gamma, beta, eps=1e-5, *, gamma2=None, beta2=None, y2=No
     return y, y2, ylp, yadd
 
 
-def split3(a, b=None, want_merged=False, stacked_nodes=False):
+def split3(a, b=None, want_merged=False, stacked_nodes=False, node_valid=None):
     """Three-term bf16 split of the stacked decoder outputs with nan_to_num (and the cooperative max over two stacks)
     fused in (cmt_split3_bf16).  a, b: [L,B,Nq,256] fp32 -> [L*B, Nq+2, 768] bf16 (, merged [L,B,Nq,256] fp32).
     stacked_nodes: `a` is [L,2B,Nq,256] holding the first node's frames then the second node's in every layer (one
-    decoder pass over both nodes); the max is taken between frame b and frame B + b."""
+    decoder pass over both nodes); the max is taken between frame b and frame B + b.
+    node_valid: optional torch.bool [2, B] on a's device, row 0 for the first node (`a`, or the first half of the stack)
+    and row 1 for the second; frame b takes the max with both nodes present, the present node's rows with one, and zero
+    rows with none.  An absent node's rows are not read."""
     a = _cuda(a, "a", torch.float32)
     L, B, Nq, C = a.shape
     frames, lstride = 0, 0
@@ -603,11 +623,18 @@ def split3(a, b=None, want_merged=False, stacked_nodes=False):
         b = _cuda(b, "b", torch.float32)
         assert b.shape == a.shape
         bptr = _ptr(b)
+    if node_valid is not None:
+        if bptr is None:
+            raise ValueError("split3: node_valid needs a second node (b or stacked_nodes=True)")
+        node_valid = check_node_valid(node_valid, B, a.device)
+        if not stacked_nodes:   # dense layout, addressed per frame
+            frames, lstride = B, B * Nq
     out = torch.empty((L * B, Nq + 2, 3 * C), dtype=torch.bfloat16, device=a.device)
     merged = torch.empty((L, B, Nq, C), dtype=torch.float32, device=a.device) if want_merged else None
     lib = _lib.load()
     with torch.cuda.device(a.device):
-        rc = lib.cmt_split3_bf16(_ptr(a), bptr, _ptr(out), _ptr(merged), L * B, Nq, C, frames, lstride, _stream(a))
+        rc = lib.cmt_split3_bf16(_ptr(a), bptr, _ptr(out), _ptr(merged), L * B, Nq, C, frames, lstride, _stream(a),
+                                 _ptr(node_valid))
     _lib.check(rc, "cmt_split3_bf16")
     _count()
     return (out, merged) if want_merged else out
@@ -662,13 +689,16 @@ BOX_DECODE_FIELDS = ("cls_logits", "center", "height", "dim", "rot", "vel")
 _BOX_DECODE_WIDTH = {"center": 2, "height": 1, "dim": 3, "rot": 2, "vel": 2}
 
 
-def bbox_topk_decode(tasks, num_classes, max_num, post_center_range, score_threshold=None, bottom_center=False):
+def bbox_topk_decode(tasks, num_classes, max_num, post_center_range, score_threshold=None, bottom_center=False,
+                     node_valid=None):
     """MultiTaskBBoxCoder.decode_single for every frame in one launch (cmt_bbox_topk_decode; multi_task_bbox_coder.py:46-141,
     util.py:37-68, with bottom_center the z shift of cmt_head.py:912).  tasks: one dict per task of its last decoder
     layer's fp32 outputs {cls_logits [B,Nq,C_t], center [B,Nq,2], height [B,Nq,1], dim [B,Nq,3], rot [B,Nq,2],
     vel [B,Nq,2]}.  score_threshold: applied (strict >) only when truthy, like the coder.  Returns the fixed-shape dict
     {boxes [B,K,9] fp32, scores [B,K] fp32, labels [B,K] int64, count [B] int32, topk_index [B,K] int64}: the kept
-    detections of frame b are the first count[b] slots, in score order; the other slots are zero with label -1."""
+    detections of frame b are the first count[b] slots, in score order; the other slots are zero with label -1.
+    node_valid: optional torch.bool [n_nodes, B] on the outputs' device; a frame none of whose nodes is present keeps
+    nothing (count 0, every slot zero with label -1) and its topk_index is -1."""
     if not 1 <= len(tasks) <= 8:
         raise ValueError(f"bbox_topk_decode: {len(tasks)} tasks (1..8 supported)")
     B, Nq = tasks[0]["cls_logits"].shape[:2]
@@ -694,6 +724,8 @@ def bbox_topk_decode(tasks, num_classes, max_num, post_center_range, score_thres
         raise ValueError("post_center_range must have 6 entries")
     K = int(max_num)   # 1 <= K <= min(1024, Nq * num_classes), checked by the library
     dev = keep[0].device
+    if node_valid is not None:
+        node_valid = check_node_valid(node_valid, B, dev, n_nodes=None)
     out = dict(boxes=torch.empty((B, K, 9), dtype=torch.float32, device=dev),
                scores=torch.empty((B, K), dtype=torch.float32, device=dev),
                labels=torch.empty((B, K), dtype=torch.int64, device=dev),
@@ -707,7 +739,8 @@ def bbox_topk_decode(tasks, num_classes, max_num, post_center_range, score_thres
                                       Nq, int(num_classes), K, ctypes.cast(_pc(post_center_range), ctypes.c_void_p),
                                       float(score_threshold or 0.0), 1 if score_threshold else 0, 1 if bottom_center else 0,
                                       *[_ptr(out[n]) for n in ("boxes", "scores", "labels", "count", "topk_index")],
-                                      _stream(keep[0]))
+                                      _stream(keep[0]), _ptr(node_valid),
+                                      0 if node_valid is None else node_valid.shape[0])
     _lib.check(rc, "cmt_bbox_topk_decode")
     _count()
     return out

@@ -68,11 +68,12 @@ class MultiTaskBBoxCoder:
         return [self.decode_single(all_logits[i], all_bbox[i], all_tids[i]) for i in range(all_logits.shape[0])]
 
 
-    def decode_batched(self, preds_dicts, bottom_center=False):
+    def decode_batched(self, preds_dicts, bottom_center=False, node_valid=None):
         """Fixed-shape counterpart of `decode` on CUDA tensors, one launch for the whole batch (ops.bbox_topk_decode).
         Returns {boxes [B,K,9], scores [B,K], labels [B,K], count [B], topk_index [B,K]}: frame b's detections are
         boxes[b, :count[b]] (= decode(...)[b]["bboxes"]), the remaining slots are zero with label -1.  Boxes are before
-        CmtHead.get_bboxes' z shift unless bottom_center (then z -= h / 2 in the kernel)."""
+        CmtHead.get_bboxes' z shift unless bottom_center (then z -= h / 2 in the kernel).  node_valid: optional
+        torch.bool [n_nodes, B] device mask; a frame with no node present gets no detections and topk_index -1."""
         if self.post_center_range is None:
             raise NotImplementedError("Need to reorganize output as a batch, only support "
                                       "post_center_range is not None for now!")
@@ -81,7 +82,7 @@ class MultiTaskBBoxCoder:
         if n_cls != self.num_classes:
             raise ValueError(f"MultiTaskBBoxCoder: num_classes {self.num_classes} != {n_cls} classes of the task heads")
         return ops.bbox_topk_decode(tasks, self.num_classes, self.max_num, self.post_center_range, self.score_threshold,
-                                    bottom_center)
+                                    bottom_center, node_valid=node_valid)
 
 
 def build_bbox_coder(cfg):

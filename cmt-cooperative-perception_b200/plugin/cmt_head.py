@@ -546,10 +546,11 @@ class _CmtHeadBase(nn.Module):
         return outs_dec
 
     # -- task heads + reference-point decode (cmt_head.py:501-547, eval branch) ---------------
-    def _finish(self, outs_dec, reference_points, outs_dec_other=None, stacked_nodes=False):
+    def _finish(self, outs_dec, reference_points, outs_dec_other=None, stacked_nodes=False, node_valid=None):
         """outs_dec: raw stacked decoder outputs [L,B,Nq,C] (nan_to_num not yet applied); outs_dec_other: the second node's
         stack for the cooperative heads -- merged with the element-wise max (cmt_head_coop.py:383-389); stacked_nodes:
-        outs_dec is [L,2B,Nq,C] with the first node's frames then the second node's in every layer."""
+        outs_dec is [L,2B,Nq,C] with the first node's frames then the second node's in every layer; node_valid: the
+        checked [2, B] device mask of the two nodes, applied per frame by the merge (ops.split3)."""
         if stacked_nodes and not all(t.fusable(outs_dec) for t in self.task_heads):
             B2 = outs_dec.shape[1] // 2
             outs_dec, outs_dec_other, stacked_nodes = outs_dec[:, :B2], outs_dec[:, B2:], False
@@ -559,18 +560,23 @@ class _CmtHeadBase(nn.Module):
             L, B, Q, C = outs_dec.shape
             if stacked_nodes:
                 B //= 2
-                xs = ops.split3(outs_dec.contiguous(), stacked_nodes=True)
+                xs = ops.split3(outs_dec.contiguous(), stacked_nodes=True, node_valid=node_valid)
             else:
-                xs = ops.split3(outs_dec.contiguous(), None if outs_dec_other is None else outs_dec_other.contiguous())
+                xs = ops.split3(outs_dec.contiguous(), None if outs_dec_other is None else outs_dec_other.contiguous(),
+                                node_valid=node_valid)
             hit = self._cache.get("ref")
             if hit is not None and hit[1]["ref"] is reference_points:
                 ref_logit = hit[1]["ref_logit"]
             else:
                 ref_logit = inverse_sigmoid(reference_points.clone()).reshape(-1, 3).contiguous()
             return [t.forward_split(xs, B, Q, ref_logit, self.pc_range) for t in self.task_heads]
-        outs_dec = torch.nan_to_num(outs_dec)
-        if outs_dec_other is not None:
-            outs_dec = ops.coop_max(outs_dec.contiguous(), torch.nan_to_num(outs_dec_other).contiguous())
+        if node_valid is not None:
+            _, outs_dec = ops.split3(outs_dec.contiguous(), outs_dec_other.contiguous(), want_merged=True,
+                                     node_valid=node_valid)
+        else:
+            outs_dec = torch.nan_to_num(outs_dec)
+            if outs_dec_other is not None:
+                outs_dec = ops.coop_max(outs_dec.contiguous(), torch.nan_to_num(outs_dec_other).contiguous())
         # torch path (non-standard head shapes): strict fp32 (no TF32), these outputs feed the top-k
         with _torch_math("fp32"):
             return self._finish_impl(outs_dec, reference_points)
@@ -606,12 +612,13 @@ class _CmtHeadBase(nn.Module):
             ret_list.append([bboxes, preds["scores"], preds["labels"]])
         return ret_list
 
-    def get_bboxes_batched(self, preds_dicts, img_metas):
+    def get_bboxes_batched(self, preds_dicts, img_metas, node_valid=None):
         """Fixed-shape counterpart of `get_bboxes` for CUDA tensors: every frame decoded in one launch with the z shift
         applied, no host synchronisation (can be captured in a CUDA graph).  Returns the device-tensor dict
         {boxes [B,K,9], scores [B,K], labels [B,K], count [B], topk_index [B,K]} of `bbox_coder.decode_batched`;
-        detector_glue.batched_to_results turns it into per-frame result dicts."""
-        return self.bbox_coder.decode_batched(preds_dicts, bottom_center=True)
+        detector_glue.batched_to_results turns it into per-frame result dicts.  node_valid: the cooperative heads'
+        [2, B] node mask; frames with no node present get no detections."""
+        return self.bbox_coder.decode_batched(preds_dicts, bottom_center=True, node_valid=node_valid)
 
 
 @HEADS.register_module()

@@ -48,11 +48,22 @@ class CmtHeadCoop(_CmtHeadBase):
             return out_v
         return ops.coop_max(out_v.contiguous(), out_i.contiguous())  # max(stack([veh, infra]), 0)
 
-    def forward_single(self, x_vehicle, x_infrastructure, x_img_vehicle, x_img_infrastructure, img_metas):
-        reference_points = self.reference_points.weight
-        reference_points, attn_mask, mask_dict = self.prepare_for_dn(len(img_metas), reference_points, img_metas)
+    def forward_single(self, x_vehicle, x_infrastructure, x_img_vehicle, x_img_infrastructure, img_metas, node_valid=None):
+        """node_valid: optional torch.bool [2, B] on the features' device, row 0 the vehicle and row 1 the infrastructure:
+        False where that node did not deliver the frame.  Such a frame's features of that node may hold anything (NaN
+        included) and change no output bit: the frame's merged decoder output is the other node's (nan_to_num'ed), or
+        zero rows when neither node delivered it.  The absent node's rows still go through the decoder (same GPU time).
+        A node missing for the whole batch is passed as None instead, without a mask."""
         has_v = x_vehicle is not None or x_img_vehicle is not None
         has_i = x_infrastructure is not None or x_img_infrastructure is not None
+        if node_valid is not None:
+            if not (has_v and has_i):
+                raise ValueError("node_valid needs the features of both nodes; pass a node missing from the whole batch "
+                                 "as None, without a mask")
+            dev = (x_vehicle if x_vehicle is not None else x_img_vehicle).device
+            node_valid = ops.check_node_valid(node_valid, len(img_metas), dev)
+        reference_points = self.reference_points.weight
+        reference_points, attn_mask, mask_dict = self.prepare_for_dn(len(img_metas), reference_points, img_metas)
         if (has_v and has_i and attn_mask is None and self.batch_nodes and not self.training
                 and self.transformer.kv_split_group is None):
             # Both nodes in ONE decoder pass: the reference runs the same decoder (shared weights, same reference points)
@@ -67,7 +78,7 @@ class CmtHeadCoop(_CmtHeadBase):
                                             reference_points)
                 outs = self.transformer.decode_nodes([c_v, c_i], torch.cat([q_v, q_i], 0))
             if outs is not None:
-                return self._finish(outs, reference_points, stacked_nodes=True)
+                return self._finish(outs, reference_points, stacked_nodes=True, node_valid=node_valid)
         out_v = out_i = None
         if x_vehicle is not None or x_img_vehicle is not None:
             out_v = self._outs_dec_raw(x_vehicle, x_img_vehicle, get_vehicle_image_metas(img_metas),
@@ -78,13 +89,14 @@ class CmtHeadCoop(_CmtHeadBase):
         if out_v is None or out_i is None:
             return self._finish(out_v if out_i is None else out_i, reference_points)
         # max(stack([veh, infra]), 0) (cmt_head_coop.py:383-389) is folded into the task heads' first kernel
-        return self._finish(out_v, reference_points, outs_dec_other=out_i)
+        return self._finish(out_v, reference_points, outs_dec_other=out_i, node_valid=node_valid)
 
     def forward(self, vehicle_pts_feats, infrastructure_pts_feats, vehicle_img_feats=None,
-                infrastructure_img_feats=None, img_metas=None):
+                infrastructure_img_feats=None, img_metas=None, node_valid=None):
+        """node_valid: the per-frame node mask of forward_single, shared by every feature level."""
         img_metas = [img_metas for _ in range(len(vehicle_pts_feats))]
         return multi_apply(self.forward_single, vehicle_pts_feats, infrastructure_pts_feats, vehicle_img_feats,
-                           infrastructure_img_feats, img_metas)
+                           infrastructure_img_feats, img_metas, node_valid=node_valid)
 
 
 @HEADS.register_module()
@@ -92,9 +104,9 @@ class CmtImageHeadCoop(CmtHeadCoop):
     """cmt_head_coop.py:812-911 (camera only)."""
     _has_bev = False
 
-    def forward_single(self, x_vehicle, x_infrastructure, x_img_vehicle, x_img_infrastructure, img_metas):
+    def forward_single(self, x_vehicle, x_infrastructure, x_img_vehicle, x_img_infrastructure, img_metas, node_valid=None):
         assert x_vehicle is None and x_infrastructure is None
-        return super().forward_single(None, None, x_img_vehicle, x_img_infrastructure, img_metas)
+        return super().forward_single(None, None, x_img_vehicle, x_img_infrastructure, img_metas, node_valid)
 
 
 @HEADS.register_module()
@@ -103,6 +115,6 @@ class CmtLidarHeadCoop(CmtHeadCoop):
     simply two decoder passes followed by the pairwise max."""
     _has_img = False
 
-    def forward_single(self, x_vehicle, x_infrastructure, x_img_vehicle, x_img_infrastructure, img_metas):
+    def forward_single(self, x_vehicle, x_infrastructure, x_img_vehicle, x_img_infrastructure, img_metas, node_valid=None):
         assert x_img_vehicle is None and x_img_infrastructure is None
-        return super().forward_single(x_vehicle, x_infrastructure, None, None, img_metas)
+        return super().forward_single(x_vehicle, x_infrastructure, None, None, img_metas, node_valid)

@@ -59,8 +59,10 @@ def simple_test_pts(head, x, x_img, img_metas, rescale=False):
 
 
 def coop_simple_test_pts(head, vehicle_pts_feats, infrastructure_pts_feats, vehicle_img_feats, infrastructure_img_feats,
-                         img_metas, rescale=False):
-    """CmtCoopDetector.coop_simple_test_pts (detectors/cmt_coop.py:549-569)."""
+                         img_metas, rescale=False, node_valid=None):
+    """CmtCoopDetector.coop_simple_test_pts (detectors/cmt_coop.py:549-569).  node_valid: optional torch.bool [2, B]
+    device mask of the nodes that delivered each frame (CmtHeadCoop.forward_single); a frame with neither node gets an
+    empty result."""
     if vehicle_pts_feats is None:
         vehicle_pts_feats = [None]
     if infrastructure_pts_feats is None:
@@ -69,8 +71,12 @@ def coop_simple_test_pts(head, vehicle_pts_feats, infrastructure_pts_feats, vehi
         vehicle_img_feats = [None]
     if infrastructure_img_feats is None:
         infrastructure_img_feats = [None]
-    outs = head(vehicle_pts_feats, infrastructure_pts_feats, vehicle_img_feats, infrastructure_img_feats, img_metas)
+    outs = head(vehicle_pts_feats, infrastructure_pts_feats, vehicle_img_feats, infrastructure_img_feats, img_metas,
+                node_valid=node_valid)
     bbox_list = head.get_bboxes(outs, img_metas, rescale=rescale)
+    if node_valid is not None:   # get_bboxes has synchronised already: reading the mask on the host costs nothing more
+        present = node_valid.any(0).tolist()
+        bbox_list = [item if present[i] else [t[:0] for t in item] for i, item in enumerate(bbox_list)]
     return [bbox3d2result(bboxes, scores, labels) for bboxes, scores, labels in bbox_list]
 
 
@@ -87,11 +93,12 @@ def simple_test(head, pts_feats, img_feats, img_metas, rescale=False):
 
 
 def coop_simple_test(head, vehicle_pts_feats, infrastructure_pts_feats, vehicle_img_feats, infrastructure_img_feats,
-                     img_metas, rescale=False):
-    """The part of CmtCoopDetector.simple_test after the two extract_*_feat calls (detectors/cmt_coop.py:571-594)."""
+                     img_metas, rescale=False, node_valid=None):
+    """The part of CmtCoopDetector.simple_test after the two extract_*_feat calls (detectors/cmt_coop.py:571-594).
+    node_valid: as in coop_simple_test_pts."""
     bbox_list = [dict() for _ in range(len(img_metas))]
     bbox_pts = coop_simple_test_pts(head, vehicle_pts_feats, infrastructure_pts_feats, vehicle_img_feats,
-                                    infrastructure_img_feats, img_metas, rescale=rescale)
+                                    infrastructure_img_feats, img_metas, rescale=rescale, node_valid=node_valid)
     for result_dict, pts_bbox in zip(bbox_list, bbox_pts):
         result_dict["pts_bbox"] = pts_bbox
     return bbox_list

@@ -58,13 +58,32 @@ class numa_local_to_gpu:
         return False
 
 
+def _head_forward(head, coop, inputs, metas, decode_boxes):
+    """head.forward_single on an inputs dict (feature tensors, plus "node_valid" for the cooperative heads), followed
+    by the batched box decode with decode_boxes."""
+    g = inputs.get
+    node_valid = g("node_valid")
+    if coop:
+        rets = head.forward_single(g("vehicle_pts_feats"), g("infrastructure_pts_feats"), g("vehicle_img_feats"),
+                                   g("infrastructure_img_feats"), metas, node_valid=node_valid)
+    else:
+        if node_valid is not None:
+            raise ValueError("node_valid is an input of the cooperative heads only")
+        rets = head.forward_single(g("pts_feats"), g("img_feats"), metas)
+    if decode_boxes:
+        return rets, head.get_bboxes_batched([[r] for r in rets], metas, node_valid=node_valid)
+    return rets
+
+
 class PipelinedRunner:
     def __init__(self, head, img_metas, example_inputs: dict, device, use_cuda_graph: bool = False,
                  keep_results: bool = True, partial_upload=None, outputs: str = "heads"):
         """example_inputs: {name: pinned CPU tensor} with the feature tensors `forward_single` takes
         (pts_feats / img_feats, or the four vehicle_/infrastructure_ entries for the coop heads); fp32, bf16 or
         fp16 -- the gather kernel rounds every feature to the compute dtype on arrival, so 16-bit features halve
-        the PCIe traffic without changing a single output bit in bf16 mode.
+        the PCIe traffic without changing a single output bit in bf16 mode.  A cooperative head may also take
+        "node_valid", a pinned torch.bool [2, B] mask of the nodes that delivered each frame (forward_single); it is
+        copied in with every batch like the features and, with outputs="boxes", also reaches the decode.
         use_cuda_graph: replay one captured forward per device input slot instead of launching eagerly.
         keep_results: `run` returns every batch's outputs as ordinary CPU tensors (copied out of the two pinned
         staging buffers before those are reused); False keeps only the staging buffers (results of the last two
@@ -114,15 +133,7 @@ class PipelinedRunner:
                                           decode_boxes=outputs == "boxes") for slot in range(2)]
 
     def _forward(self, feats):
-        g = feats.get
-        if self.coop:
-            rets = self.head.forward_single(g("vehicle_pts_feats"), g("infrastructure_pts_feats"),
-                                            g("vehicle_img_feats"), g("infrastructure_img_feats"), self.metas)
-        else:
-            rets = self.head.forward_single(g("pts_feats"), g("img_feats"), self.metas)
-        if self.outputs == "boxes":
-            return rets, self.head.get_bboxes_batched([[r] for r in rets], self.metas)
-        return rets
+        return _head_forward(self.head, self.coop, feats, self.metas, self.outputs == "boxes")
 
     def _payload(self, staging):
         """What a batch hands out: the per-task list of head outputs, or the box dict."""
@@ -284,6 +295,9 @@ class GraphedForward:
     With decode_boxes=True the graph also holds `head.get_bboxes_batched` of the outputs, and a call returns
     (head outputs, boxes dict), both static outputs of the graph.
 
+    For a cooperative head the inputs may include "node_valid" (torch.bool [2, B], forward_single): like the features it
+    lives in a static buffer that each call overwrites, so a new mask is one small copy and never a re-capture.
+
     The graph bakes in device addresses, so the inputs live in static buffers (`g.static_inputs`) and the outputs are
     overwritten by the next replay.  The calibration matrices enter the forward as device tensors uploaded once per
     distinct `img_metas` (CmtHead._matrices); a call with different calibration re-captures.
@@ -303,15 +317,7 @@ class GraphedForward:
         self._capture(img_metas, warmup)
 
     def _forward(self, metas):
-        g = self.static_inputs.get
-        if self.coop:
-            rets = self.head.forward_single(g("vehicle_pts_feats"), g("infrastructure_pts_feats"),
-                                            g("vehicle_img_feats"), g("infrastructure_img_feats"), metas)
-        else:
-            rets = self.head.forward_single(g("pts_feats"), g("img_feats"), metas)
-        if self.decode_boxes:
-            return rets, self.head.get_bboxes_batched([[r] for r in rets], metas)
-        return rets
+        return _head_forward(self.head, self.coop, self.static_inputs, metas, self.decode_boxes)
 
     @torch.no_grad()
     def _capture(self, img_metas, warmup):

@@ -242,6 +242,11 @@ int cmt_add_layernorm(const float* x, const float* r, const float* gamma, const 
  *    frames > 0: the inputs are strided -- row q of z = (layer, frame) sits at row layer*layer_stride_rows + frame*Nq + q
  *    (both nodes' frames stacked in one decoder pass: a = the stack, b = a + frames*Nq*256, layer_stride_rows =
  *    2*frames*Nq); frames = 0: dense [Z, Nq, 256].
+ *    node_valid (nullable DEVICE array, since version 102): uint8 [2, frames], entry [n][f] != 0 when node n (0: the node
+ *    in `a`, 1: the node in `b`) delivered frame f.  Needs b and frames > 0 (for the dense layout pass frames = B and
+ *    layer_stride_rows = B*Nq).  Frame f then takes max(nan_to_num(a), nan_to_num(b)) with both nodes, nan_to_num of the
+ *    present node's rows with one, and zero rows with none; `merged` follows the same rule, and an absent node's rows
+ *    are not read (they may hold anything).  NULL: every node is present.
  * 2. cmt_gemm_segmented with 6 segments per tap (x1w1, x1w2, x2w1, x1w3, x2w2, x3w1; the weights split the same way):
  *    the first grouped convolution as a tensor-core GEMM that reproduces the fp32 product to ~2^-22.
  * 3. cmt_task_head_tail: group-LN + ReLU + second convolution (+ optional reference-point decode):
@@ -257,7 +262,7 @@ int cmt_add_layernorm(const float* x, const float* r, const float* gamma, const 
  *   head_off_host / head_cout_host (nullable HOST arrays of NH entries, NH <= 8): instead of the padded layout, head i is
  *          written as its own contiguous [L, M, cout[i]] tensor starting at out + off[i] (elements). */
 int cmt_split3_bf16(const float* a, const float* b, void* out, float* merged, int64_t Z, int Nq, int C, int frames,
-                    int64_t layer_stride_rows, void* stream);
+                    int64_t layer_stride_rows, void* stream, const uint8_t* node_valid);
 int cmt_task_head_tail(const float* h, const float* gamma, const float* beta, const float* w2,
                        const float* b2, float* out, int L, int M, int NH, int HC, int CMAX, float eps,
                        int ksize, int Nq, const float* ref_logit, const int* dec_comp, const float* dec_scale,
@@ -285,6 +290,9 @@ int cmt_coop_max(const float* a, const float* b, float* out, int64_t n, void* st
  *   Outputs (caller-owned, fixed shape): boxes [B,K,9] fp32, scores [B,K] fp32, labels [B,K] int64 -- the kept slots
  *     first, in score order, then zeros with label -1;  count [B] int32 kept slots;  topk_index [B,K] int64 every
  *     selected flat index before the mask.
+ *   node_valid (nullable DEVICE array, since version 102): uint8 [n_nodes, B]; frame b is decoded when any entry
+ *     [n][b] != 0.  Otherwise its head outputs are not read and the frame gets count 0, zero boxes and scores, and
+ *     labels and topk_index -1 in every slot.  NULL: every frame is decoded (n_nodes is then ignored).
  *   Limits (CMT_ERR_BAD_ARG otherwise): 1 <= K <= min(CMT_BOX_DECODE_MAX_K, Nq*num_classes), and
  *     Nq*num_classes <= CMT_BOX_DECODE_MAX_CANDIDATES (one CTA per frame keeps every score in shared memory; nuScenes
  *     is 900 x 10 = 9000). */
@@ -294,7 +302,7 @@ int cmt_coop_max(const float* a, const float* b, float* out, int64_t n, void* st
 int cmt_bbox_topk_decode(const float* const* task_ptrs_host, const int* task_classes_host, int T, int B, int Nq,
                          int num_classes, int max_num, const float* post_center_range_host, float score_threshold,
                          int use_score_threshold, int bottom_center, float* boxes, float* scores, int64_t* labels,
-                         int32_t* count, int64_t* topk_index, void* stream);
+                         int32_t* count, int64_t* topk_index, void* stream, const uint8_t* node_valid, int n_nodes);
 
 /* ---- diagnostics -----------------------------------------------------------------------
  * Cycle accounting of the tcgen05 attention kernel on the CURRENT device.  dev_buf: device buffer of

@@ -18,3 +18,4 @@ run decoder tests/test_gpu_decoder.py
 run multi tests/test_gpu_multi.py
 run decode tests/test_gpu_bbox_decode.py
 run fp16 tests/test_gpu_fp16.py
+run node_mask tests/test_gpu_coop_node_mask.py
