@@ -155,6 +155,10 @@ __global__ void __launch_bounds__(256) ray_query_pe_kernel(const float* __restri
         const bool inside = (px < p.pad_w) && (px >= 0.0f) && (py < p.pad_h) && (py >= 0.0f) && zpos;
         if (g == 0) mask[pt] = inside ? 1.0f : 0.0f;
         const float* M = i2l + (static_cast<long long>(b) * p.V + v) * 16;
+        // A point outside the view enters the view sum as emb * 0 (cmt_head.py:466) whatever its features, so they are
+        // written as zeros.  Their true values are unbounded: near the camera plane (s[2] -> 0) px and py reach ~1e8
+        // and the lifted coordinates overflow fp16 to inf, which the rv-PE MLP turns into NaN and the view sum into
+        // NaN * 0.
         float vals[8];
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
@@ -167,7 +171,7 @@ __global__ void __launch_bounds__(256) ray_query_pe_kernel(const float* __restri
             acc = fmaf(py * d, r[1], acc);
             acc = fmaf(pz * d, r[2], acc);
             acc = acc + r[3];
-            vals[e] = (acc - p.pc_min[c]) / p.pc_rng[c];
+            vals[e] = inside ? (acc - p.pc_min[c]) / p.pc_rng[c] : 0.0f;
         }
         if (kOut != CMT_F32) {
             uint4 w;

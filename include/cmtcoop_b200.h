@@ -63,7 +63,9 @@ int cmt_ray_pe(const float* img2lidar, void* out, int n_cam, int H, int W, int D
  * Replaces CmtHead._rv_query_embed up to the rv_embedding MLP (cmt_head.py:439-464).
  * ref:       [B,Nq,3] fp32 in [0,1] (already inverse_sigmoid(...).sigmoid()'ed, :470)
  * lidar2img: [B,V,4,4] fp32, img2lidar: [B,V,4,4] fp32
- * out:       [B,V,Nq,D*3] (fp32|bf16|fp16), mask: [B,V,Nq] fp32 (1.0 inside image & z>0). */
+ * out:       [B,V,Nq,D*3] (fp32|bf16|fp16), mask: [B,V,Nq] fp32 (1.0 inside image & z>0).
+ *            Where mask is 0 the features are written as 0: the view sum ignores them, and their true values
+ *            overflow fp16 for points near the camera plane. */
 int cmt_ray_query_pe(const float* ref, const float* lidar2img, const float* img2lidar, void* out,
                      float* mask, int B, int V, int Nq, int D, float pad_h, float pad_w,
                      const float* pc_range_host, int out_dtype, void* stream);

@@ -277,6 +277,38 @@ def test_ray_query_pe_pos2embed_and_view_sum_fp16():
     assert torch.equal(ops.masked_view_sum(emb, m16, base=base), ops.masked_view_sum(emb.float(), m16, base=base))
 
 
+def test_ray_query_pe_fp16_points_on_the_camera_plane():
+    """Reference points on camera 0's plane (z = 0) project to |px| ~ 1e8: their lifted coordinates are far beyond fp16's
+    range.  They are outside the view, so their features are written as zeros in every dtype; the rv-PE MLP and the view
+    sum then stay finite in fp16, and the in-view points of camera 1 keep the oracle's features."""
+    B, Nq = 1, 200
+    rng = np.random.RandomState(9)
+    plane = np.diag([800.0, 800.0, 1.0, 1.0])                     # s = (800 x, 800 y, z): z = 0 is the camera plane
+    l2i = np.stack([plane, synth.camera_matrices(1, rng, 160.0, 96.0)[0]])[None]
+    l32, i32 = torch.from_numpy(l2i).float(), torch.from_numpy(np.linalg.inv(l2i)).float()
+    ref = torch.from_numpy(rng.uniform(0, 1, (B, Nq, 3)).astype(np.float32))
+    ref[..., 2] = 0.625                                            # z = 0.625 * 8 - 5 = 0 exactly
+    want, wmask = O.rv_query_feats(ref, l32, i32, 64, 96.0, 160.0, NUSC)
+    assert not bool(wmask[0, 0].any()) and float(want[0, 0].abs().max()) > 65504.0   # the overflow this guards against
+    feats = {dt: ops.ray_query_pe(ref.to(DEV), l32.to(DEV), i32.to(DEV), 64, 96.0, 160.0, NUSC, out_dtype=dt)
+             for dt in (torch.float32, torch.bfloat16, torch.float16)}
+    f32, m32 = feats[torch.float32]
+    assert torch.equal(m32.cpu() > 0.5, wmask)
+    for dt, (f, m) in feats.items():
+        assert torch.equal(m, m32) and bool(torch.isfinite(f).all()), dt
+        assert float(f[m == 0].abs().max()) == 0.0, dt
+    sel = wmask.unsqueeze(-1).expand_as(want)
+    assert int(wmask.sum()) > 0 and _rel(f32.cpu()[sel], want[sel]) < 1e-5
+    f16 = feats[torch.float16][0]
+    assert torch.equal(f16, f32.half())
+    g = torch.Generator().manual_seed(2)
+    w0 = (torch.randn(1024, 192, generator=g) / math.sqrt(192)).half().to(DEV)
+    w1 = (torch.randn(256, 1024, generator=g) / 32).half().to(DEV)
+    h = ops.linear(f16, w0, torch.zeros(1024, device=DEV), relu=True)
+    emb = ops.linear(h, w1, torch.zeros(256, device=DEV), out_dtype=torch.float32)
+    assert bool(torch.isfinite(ops.masked_view_sum(emb, m32)).all())
+
+
 @pytest.mark.parametrize("fdt", [torch.float32, torch.float16])
 def test_gather_tokens_fp16(fdt):
     B, C, V = 2, 256, 3
