@@ -27,14 +27,15 @@ SIGNATURES = {
     "cmt_check_device": (_i, [_i]),
     "cmt_ray_pe": (_i, [_vp, _vp, _i, _i, _i, _i, _f, _f, _vp, _i, _vp]),
     "cmt_ray_query_pe": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _f, _vp, _i, _vp]),
-    "cmt_masked_view_sum": (_i, [_vp, _vp, _vp, _i64, _vp, _i, _i, _i, _i, _i, _vp]),
+    "cmt_masked_view_sum": (_i, [_vp, _vp, _vp, _i64, _vp, _i, _i, _i, _i, _i, _vp, _vp]),
     "cmt_pos2embed": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
-    "cmt_gather_tokens": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
+    "cmt_gather_tokens": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
+    "cmt_sensor_key_keep": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
     "cmt_gemm_bias_act": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i64, _i64, _i64, _i64, _i64, _i,
                                _i64, _i64, _i64, _f, _i, _i, _i, _vp, _vp]),
     "cmt_gemm_segmented": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _i, _i64, _i, _i64, _i64, _i64, _i, _i64, _i64, _i,
                                 _i64, _f, _i, _i, _vp]),
-    "cmt_nchw_to_padded_nhwc": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i]),
+    "cmt_nchw_to_padded_nhwc": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i, _vp]),
     "cmt_shared_conv_tokens": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i64, _i, _i, _vp, _i]),
     "cmt_cross_attn_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "cmt_cross_attn_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i64, _i64, _i64,

@@ -130,7 +130,7 @@ using namespace cmt;
 
 extern "C" {
 
-int cmt_version(void) { return 102; }
+int cmt_version(void) { return 103; }
 
 const char* cmt_last_error_string(void) { return g_err; }
 
@@ -165,9 +165,10 @@ int cmt_ray_query_pe(const float* ref, const float* lidar2img, const float* img2
 }
 
 int cmt_masked_view_sum(const void* emb, const float* mask, const float* base, int64_t base_bstride, float* out, int B, int V,
-                        int Nq, int C, int emb_dtype, void* stream) {
+                        int Nq, int C, int emb_dtype, void* stream, const uint8_t* view_valid) {
     CMT_REQUIRE_DEVICE();
-    return launch_masked_view_sum(emb, mask, base, base_bstride, out, B, V, Nq, C, emb_dtype, static_cast<cudaStream_t>(stream));
+    return launch_masked_view_sum(emb, mask, base, base_bstride, out, B, V, Nq, C, emb_dtype, view_valid,
+                                  static_cast<cudaStream_t>(stream));
 }
 
 int cmt_pos2embed(const float* pos, void* out, int N, int pos_stride, int F, int out_dtype, void* stream) {
@@ -177,10 +178,15 @@ int cmt_pos2embed(const float* pos, void* out, int N, int pos_stride, int F, int
 
 int cmt_gather_tokens(const void* x_bev, const void* x_img, const float* bev_pos, const float* rv_pos,
                       void* xk, void* xv, int B, int C, int n_bev, int V, int n_img, int tok_begin, int tok_end,
-                      int rv_tok0, int rv_rows, int feat_dtype, int out_dtype, void* stream) {
+                      int rv_tok0, int rv_rows, int feat_dtype, int out_dtype, void* stream, const uint8_t* sensor_valid) {
     CMT_REQUIRE_DEVICE();
     return launch_gather_tokens(x_bev, x_img, bev_pos, rv_pos, xk, xv, B, C, n_bev, V, n_img, tok_begin, tok_end,
-                                rv_tok0, rv_rows, feat_dtype, out_dtype, static_cast<cudaStream_t>(stream));
+                                rv_tok0, rv_rows, feat_dtype, out_dtype, sensor_valid, static_cast<cudaStream_t>(stream));
+}
+
+int cmt_sensor_key_keep(const uint8_t* sensor_valid, uint8_t* key_keep, int B, int n_bev, int V, int n_img, void* stream) {
+    CMT_REQUIRE_DEVICE();
+    return launch_sensor_key_keep(sensor_valid, key_keep, B, n_bev, V, n_img, static_cast<cudaStream_t>(stream));
 }
 
 int cmt_gemm_bias_act(const void* A, const void* B, const float* bias, void* C, int M, int N, int K,
@@ -273,9 +279,10 @@ int cmt_gemm_segmented(const void* A, const void* B, const float* bias, void* C,
 }
 
 int cmt_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, int W, int guard_rows, int in_dtype, void* stream,
-                            int out_dtype) {
+                            int out_dtype, const uint8_t* frame_valid) {
     CMT_REQUIRE_DEVICE();
-    return launch_nchw_to_padded_nhwc(x, out, B, C, H, W, guard_rows, in_dtype, out_dtype, static_cast<cudaStream_t>(stream));
+    return launch_nchw_to_padded_nhwc(x, out, B, C, H, W, guard_rows, in_dtype, out_dtype, frame_valid,
+                                      static_cast<cudaStream_t>(stream));
 }
 
 int cmt_shared_conv_tokens(const void* xp, const void* w, const float* bias, const float* bev_pos, void* xk, void* xv, int B,

@@ -25,6 +25,14 @@ constexpr int kTileTok = 32;
 //
 // [tok_begin, tok_end): only these tokens of the concatenated BEV ++ image axis are produced (KV-token split across
 // GPUs: a rank gathers, projects and attends its own range only); row 0 of xk / xv is token tok_begin.
+//
+// sensor_valid (nullable): [S, B] bytes, row 0 the BEV map when n_bev > 0, then one row per camera.  The tokens of an
+// absent (sensor, frame) are written as zero rows of xk AND xv: neither its features nor its position encoding is
+// read (they may hold NaN), so every K / V row stays finite and the attention's key mask only has to drop them.
+__device__ __forceinline__ bool sensor_present(const uint8_t* sensor_valid, int row, int b, int B) {
+    return sensor_valid == nullptr || sensor_valid[static_cast<long long>(row) * B + b] != 0;
+}
+
 template <int kIn>
 __device__ __forceinline__ float load_feat(const void* p, long long i) {
     if (kIn == CMT_F32) return __ldg(reinterpret_cast<const float*>(p) + i);
@@ -50,7 +58,7 @@ __global__ void __launch_bounds__(256) gather_tokens_kernel(
     const void* __restrict__ x_bev, const void* __restrict__ x_img,
     const float* __restrict__ bev_pos, const float* __restrict__ rv_pos, void* __restrict__ xk,
     void* __restrict__ xv, int C, int n_bev, int V, int n_img, int tiles_bev, int tiles_img, int tok_begin,
-    int tok_end, int rv_tok0, int rv_rows) {
+    int tok_end, int rv_tok0, int rv_rows, const uint8_t* __restrict__ sensor_valid) {
     extern __shared__ float tile[];  // [kTileTok][C + 1]
     constexpr int ESZ = kIn == CMT_F32 ? 4 : 2;
     const int b = blockIdx.y;
@@ -60,12 +68,14 @@ __global__ void __launch_bounds__(256) gather_tokens_kernel(
     const float* pos;           // [n_src, C] token-major (already offset to this source's first token)
     int n_src, t0;
     long long dst_tok0;         // first destination token of this source inside the frame
+    bool present;               // block-uniform
     if (tix < tiles_bev) {
         src = reinterpret_cast<const unsigned char*>(x_bev) + static_cast<long long>(b) * C * n_bev * ESZ;
         pos = bev_pos;
         n_src = n_bev;
         t0 = tix * kTileTok;
         dst_tok0 = 0;
+        present = sensor_present(sensor_valid, 0, b, gridDim.y);
     } else {
         tix -= tiles_bev;
         const int v = tix / tiles_img;
@@ -77,6 +87,7 @@ __global__ void __launch_bounds__(256) gather_tokens_kernel(
         n_src = n_img;
         t0 = (tix % tiles_img) * kTileTok;
         dst_tok0 = n_bev + static_cast<long long>(v) * n_img;
+        present = sensor_present(sensor_valid, (n_bev > 0 ? 1 : 0) + v, b, gridDim.y);
     }
     // tiles entirely outside this rank's token range have nothing to do (block-uniform)
     if (dst_tok0 + t0 >= tok_end || dst_tok0 + t0 + kTileTok <= tok_begin) return;
@@ -87,14 +98,14 @@ __global__ void __launch_bounds__(256) gather_tokens_kernel(
         const int tok = t0 + 2 * l16;
         for (int c = 2 * warp + half; c < C; c += 16) {
             float lo = 0.0f, hi = 0.0f;
-            if (tok < n_src)   // n_src even and tok even: both tokens are in range
+            if (tok < n_src && present)   // n_src even and tok even: both tokens are in range
                 unpack_feat2<kIn>(__ldg(reinterpret_cast<const uint32_t*>(src + (static_cast<long long>(c) * n_src + tok) * 2)), lo, hi);
             tile[(2 * l16) * pitch + c] = lo;
             tile[(2 * l16 + 1) * pitch + c] = hi;
         }
     } else {
         const int tok = t0 + lane;
-        const bool tok_ok = tok < n_src;
+        const bool tok_ok = tok < n_src && present;
         for (int c = warp; c < C; c += 8)
             tile[lane * pitch + c] = tok_ok ? load_feat<kIn>(src, static_cast<long long>(c) * n_src + tok) : 0.0f;
     }
@@ -110,7 +121,7 @@ __global__ void __launch_bounds__(256) gather_tokens_kernel(
         const float* trow = tile + r * pitch;
         for (int c = lane * 2; c < C; c += 64) {
             const float m0 = trow[c], m1 = trow[c + 1];
-            const float2 pp = *reinterpret_cast<const float2*>(prow + c);
+            const float2 pp = present ? *reinterpret_cast<const float2*>(prow + c) : make_float2(0.0f, 0.0f);
             if (kOut != CMT_F32) {
                 reinterpret_cast<uint32_t*>(xk)[(drow + c) >> 1] = pack_lp2<kOut>(m0 + pp.x, m1 + pp.y);
                 reinterpret_cast<uint32_t*>(xv)[(drow + c) >> 1] = pack_lp2<kOut>(m0, m1);
@@ -127,7 +138,7 @@ __global__ void __launch_bounds__(256) gather_tokens_kernel(
 int launch_gather_tokens(const void* x_bev, const void* x_img, const float* bev_pos,
                          const float* rv_pos, void* xk, void* xv, int B, int C, int n_bev, int V,
                          int n_img, int tok_begin, int tok_end, int rv_tok0, int rv_rows, int feat_dtype, int out_dtype,
-                         cudaStream_t stream) {
+                         const uint8_t* sensor_valid, cudaStream_t stream) {
     CMT_CHECK_ARG(xk && xv, "cmt_gather_tokens: null output");
     CMT_CHECK_ARG(B > 0 && C > 0 && (C % 2) == 0, "cmt_gather_tokens: bad B/C");
     CMT_CHECK_ARG(n_bev >= 0 && V >= 0 && n_img >= 0, "cmt_gather_tokens: bad token counts");
@@ -163,7 +174,8 @@ int launch_gather_tokens(const void* x_bev, const void* x_img, const float* bev_
     dim3 grid(tiles, B);
 #define CMT_GATHER_LAUNCH(OUT, IN)                                                                            \
     gather_tokens_kernel<OUT, IN><<<grid, 256, smem, stream>>>(x_bev, x_img, bev_pos, rv_pos, xk, xv, C, n_bev, V, \
-                                                               n_img, tiles_bev, tiles_img, tok_begin, tok_end, rv_tok0, rv_rows)
+                                                               n_img, tiles_bev, tiles_img, tok_begin, tok_end, rv_tok0, rv_rows, \
+                                                               sensor_valid)
 #define CMT_GATHER_LAUNCH_OUT(IN)                                                                             \
     do {                                                                                                      \
         if (out_dtype == CMT_BF16) CMT_GATHER_LAUNCH(CMT_BF16, IN);                                          \
@@ -185,9 +197,12 @@ int launch_gather_tokens(const void* x_bev, const void* x_img, const float* bev_
 // (y, x) lands in row guard + (y + 1) * (W + 2) + (x + 1).  Only interior rows are written: the border and guard rows
 // are zero from the (one-time) allocation, so a filter tap is a pure row shift of -(W+2)-1 .. +(W+2)+1 with no edge
 // handling.  Block = 32 consecutive pixels x one block of up to 256 channels, same transpose tile as the token gather.
+// frame_valid (nullable): [B] bytes; the interior rows of a frame whose map is absent are written as zeros (its input,
+// which may hold NaN, is not read), so the implicit GEMM produces finite BEV rows for it.
 template <int kIn, int kOut>
 __global__ void __launch_bounds__(256) nchw_to_padded_nhwc_kernel(const void* __restrict__ x, uint16_t* __restrict__ out,
-                                                                  int C, int H, int W, int guard, long long rows_per_frame) {
+                                                                  int C, int H, int W, int guard, long long rows_per_frame,
+                                                                  const uint8_t* __restrict__ frame_valid) {
     extern __shared__ float tile[];  // [32][257]
     constexpr int ESZ = kIn == CMT_F32 ? 4 : 2;
     constexpr int CB = 256, pitch = CB + 1;
@@ -196,20 +211,21 @@ __global__ void __launch_bounds__(256) nchw_to_padded_nhwc_kernel(const void* __
     const int n_src = H * W;
     const int t0 = blockIdx.x * kTileTok;
     const unsigned char* src = reinterpret_cast<const unsigned char*>(x) + (static_cast<long long>(b) * C + c0) * n_src * ESZ;
+    const bool present = frame_valid == nullptr || frame_valid[b] != 0;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (kIn != CMT_F32 && (n_src & 1) == 0) {
         const int half = lane >> 4, l16 = lane & 15;
         const int tok = t0 + 2 * l16;
         for (int c = 2 * warp + half; c < nc; c += 16) {
             float lo = 0.0f, hi = 0.0f;
-            if (tok < n_src)
+            if (tok < n_src && present)
                 unpack_feat2<kIn>(__ldg(reinterpret_cast<const uint32_t*>(src + (static_cast<long long>(c) * n_src + tok) * 2)), lo, hi);
             tile[(2 * l16) * pitch + c] = lo;
             tile[(2 * l16 + 1) * pitch + c] = hi;
         }
     } else {
         const int tok = t0 + lane;
-        const bool tok_ok = tok < n_src;
+        const bool tok_ok = tok < n_src && present;
         for (int c = warp; c < nc; c += 8)
             tile[lane * pitch + c] = tok_ok ? load_feat<kIn>(src, static_cast<long long>(c) * n_src + tok) : 0.0f;
     }
@@ -226,7 +242,7 @@ __global__ void __launch_bounds__(256) nchw_to_padded_nhwc_kernel(const void* __
 }
 
 int launch_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, int W, int guard, int in_dtype,
-                               int out_dtype, cudaStream_t stream) {
+                               int out_dtype, const uint8_t* frame_valid, cudaStream_t stream) {
     CMT_CHECK_ARG(x && out && B > 0 && C > 0 && C % 2 == 0 && H > 0 && W > 0 && guard >= W + 3,
                   "cmt_nchw_to_padded_nhwc: bad arguments (guard must be >= W + 3)");
     CMT_CHECK_ARG(in_dtype == CMT_F32 || in_dtype == CMT_BF16 || in_dtype == CMT_F16, "cmt_nchw_to_padded_nhwc: bad dtype");
@@ -237,16 +253,52 @@ int launch_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, in
     dim3 grid((H * W + kTileTok - 1) / kTileTok, B, (C + 255) / 256);
     const size_t smem = static_cast<size_t>(kTileTok) * 257 * sizeof(float);
     uint16_t* o = reinterpret_cast<uint16_t*>(out);
+#define CMT_LAYOUT_LAUNCH(IN, OUT) \
+    nchw_to_padded_nhwc_kernel<IN, OUT><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows, frame_valid)
     if (out_dtype == CMT_BF16) {
-        if (in_dtype == CMT_F32) nchw_to_padded_nhwc_kernel<CMT_F32, CMT_BF16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
-        else if (in_dtype == CMT_BF16) nchw_to_padded_nhwc_kernel<CMT_BF16, CMT_BF16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
-        else nchw_to_padded_nhwc_kernel<CMT_F16, CMT_BF16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
+        if (in_dtype == CMT_F32) CMT_LAYOUT_LAUNCH(CMT_F32, CMT_BF16);
+        else if (in_dtype == CMT_BF16) CMT_LAYOUT_LAUNCH(CMT_BF16, CMT_BF16);
+        else CMT_LAYOUT_LAUNCH(CMT_F16, CMT_BF16);
     } else {
-        if (in_dtype == CMT_F32) nchw_to_padded_nhwc_kernel<CMT_F32, CMT_F16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
-        else if (in_dtype == CMT_BF16) nchw_to_padded_nhwc_kernel<CMT_BF16, CMT_F16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
-        else nchw_to_padded_nhwc_kernel<CMT_F16, CMT_F16><<<grid, 256, smem, stream>>>(x, o, C, H, W, guard, rows);
+        if (in_dtype == CMT_F32) CMT_LAYOUT_LAUNCH(CMT_F32, CMT_F16);
+        else if (in_dtype == CMT_BF16) CMT_LAYOUT_LAUNCH(CMT_BF16, CMT_F16);
+        else CMT_LAYOUT_LAUNCH(CMT_F16, CMT_F16);
     }
+#undef CMT_LAYOUT_LAUNCH
     CMT_LAUNCH_CHECK("cmt_nchw_to_padded_nhwc");
+    return CMT_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Key-keep bytes of the cross-attention from the per-frame sensor mask: keep[b][t] = sensor_valid[s(t)][b] for the
+// concatenated BEV ++ image token axis, s = 0 for the n_bev BEV tokens (when n_bev > 0), then one row per camera of
+// n_img tokens.  One thread per byte (a few hundred KB per batch).
+__global__ void __launch_bounds__(256) sensor_key_keep_kernel(const uint8_t* __restrict__ sensor_valid,
+                                                              uint8_t* __restrict__ keep, int B, int n_bev, int n_img,
+                                                              long long n_kv) {
+    const long long total = n_kv * B;
+    const int cam0 = n_bev > 0 ? 1 : 0;
+    for (long long t = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; t < total;
+         t += static_cast<long long>(gridDim.x) * blockDim.x) {
+        const int b = static_cast<int>(t / n_kv);
+        const long long tok = t - static_cast<long long>(b) * n_kv;
+        const int row = tok < n_bev ? 0 : cam0 + static_cast<int>((tok - n_bev) / n_img);
+        keep[t] = sensor_valid[static_cast<long long>(row) * B + b] != 0 ? 1 : 0;
+    }
+}
+
+int launch_sensor_key_keep(const uint8_t* sensor_valid, uint8_t* keep, int B, int n_bev, int V, int n_img,
+                           cudaStream_t stream) {
+    CMT_CHECK_ARG(sensor_valid && keep, "cmt_sensor_key_keep: null pointer");
+    CMT_CHECK_ARG(B > 0 && n_bev >= 0 && V >= 0 && n_img >= 0, "cmt_sensor_key_keep: bad shape");
+    const long long n_kv = n_bev + static_cast<long long>(V) * n_img;
+    CMT_CHECK_ARG(n_kv > 0, "cmt_sensor_key_keep: no tokens");
+    const long long total = n_kv * B;
+    long long blocks = (total + 255) / 256;
+    const long long cap = static_cast<long long>(device_sm_count()) * 16;
+    if (blocks > cap) blocks = cap;
+    sensor_key_keep_kernel<<<static_cast<int>(blocks), 256, 0, stream>>>(sensor_valid, keep, B, n_bev, n_img, n_kv);
+    CMT_LAUNCH_CHECK("cmt_sensor_key_keep");
     return CMT_OK;
 }
 

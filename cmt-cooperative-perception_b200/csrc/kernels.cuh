@@ -64,16 +64,18 @@ int launch_ray_query_pe(const float* ref, const float* l2i, const float* i2l, vo
                         float* mask, int B, int V, int Nq, int D, float pad_h, float pad_w,
                         const float* pc, int out_dtype, cudaStream_t stream);
 int launch_masked_view_sum(const void* emb, const float* mask, const float* base, long long base_bstride, float* out, int B,
-                           int V, int Nq, int C, int emb_dtype, cudaStream_t stream);
+                           int V, int Nq, int C, int emb_dtype, const uint8_t* view_valid, cudaStream_t stream);
 int launch_pos2embed(const float* pos, void* out, int N, int pos_stride, int F, int out_dtype,
                      cudaStream_t stream);
 // gather_kernels.cu
 int launch_gather_tokens(const void* x_bev, const void* x_img, const float* bev_pos,
                          const float* rv_pos, void* xk, void* xv, int B, int C, int n_bev, int V,
                          int n_img, int tok_begin, int tok_end, int rv_tok0, int rv_rows, int feat_dtype, int out_dtype,
-                         cudaStream_t stream);
+                         const uint8_t* sensor_valid, cudaStream_t stream);
 int launch_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, int W, int guard, int in_dtype,
-                               int out_dtype, cudaStream_t stream);
+                               int out_dtype, const uint8_t* frame_valid, cudaStream_t stream);
+int launch_sensor_key_keep(const uint8_t* sensor_valid, uint8_t* keep, int B, int n_bev, int V, int n_img,
+                           cudaStream_t stream);
 int launch_coop_max(const float* a, const float* b, float* out, long long n, cudaStream_t stream);
 int launch_lse_merge(const float* o_parts, const float* lse_parts, void* o, float* lse, int G,
                      int B, int H, int Nq, long long o_gstride, long long lse_gstride, int o_dtype, cudaStream_t stream);

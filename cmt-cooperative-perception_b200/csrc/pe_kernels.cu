@@ -193,7 +193,7 @@ __global__ void __launch_bounds__(256) masked_view_sum_kernel(const void* __rest
                                                               const float* __restrict__ mask,
                                                               const float* __restrict__ base, long long base_bstride,
                                                               float* __restrict__ out, int B, int V,
-                                                              int Nq, int C) {
+                                                              int Nq, int C, const uint8_t* __restrict__ view_valid) {
     const long long total = static_cast<long long>(B) * Nq * C;
     for (long long t = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; t < total;
          t += static_cast<long long>(gridDim.x) * blockDim.x) {
@@ -202,6 +202,8 @@ __global__ void __launch_bounds__(256) masked_view_sum_kernel(const void* __rest
         const int b = static_cast<int>(t / (static_cast<long long>(C) * Nq));
         float acc = 0.0f;
         for (int v = 0; v < V; ++v) {
+            // an absent camera is skipped, not weighted by zero: its embedding may be NaN (garbage calibration)
+            if (view_valid != nullptr && view_valid[static_cast<long long>(v) * B + b] == 0) continue;
             const long long row = (static_cast<long long>(b) * V + v) * Nq + n;
             const float m = mask[row];
             float e;
@@ -321,17 +323,17 @@ int launch_ray_query_pe(const float* ref, const float* l2i, const float* i2l, vo
 }
 
 int launch_masked_view_sum(const void* emb, const float* mask, const float* base, long long base_bstride, float* out, int B,
-                           int V, int Nq, int C, int emb_dtype, cudaStream_t stream) {
+                           int V, int Nq, int C, int emb_dtype, const uint8_t* view_valid, cudaStream_t stream) {
     CMT_CHECK_ARG(emb && mask && out, "cmt_masked_view_sum: null pointer");
     CMT_CHECK_ARG(B > 0 && V > 0 && Nq > 0 && C > 0, "cmt_masked_view_sum: bad shape");
     const long long total = static_cast<long long>(B) * Nq * C;
     const int grid = grid_for(total, 256);
     if (emb_dtype == CMT_BF16)
-        masked_view_sum_kernel<CMT_BF16><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C);
+        masked_view_sum_kernel<CMT_BF16><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C, view_valid);
     else if (emb_dtype == CMT_F16)
-        masked_view_sum_kernel<CMT_F16><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C);
+        masked_view_sum_kernel<CMT_F16><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C, view_valid);
     else if (emb_dtype == CMT_F32)
-        masked_view_sum_kernel<CMT_F32><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C);
+        masked_view_sum_kernel<CMT_F32><<<grid, 256, 0, stream>>>(emb, mask, base, base_bstride, out, B, V, Nq, C, view_valid);
     else
         CMT_CHECK_ARG(false, "cmt_masked_view_sum: bad dtype");
     CMT_LAUNCH_CHECK("cmt_masked_view_sum");

@@ -110,21 +110,27 @@ def _cuda(t, name, dtype=None):
     return t
 
 
-def check_node_valid(node_valid, B, device, n_nodes=2):
+def check_node_valid(node_valid, B, device, n_nodes=2, name="node_valid"):
     """Host-side checks of a per-frame node mask: a torch.bool tensor [n_nodes, B] on `device` (n_nodes=None: any
     n_nodes >= 1).  Row n, column b is True when node n delivered frame b.  The values are never read here, so the check
-    costs no device synchronisation.  Returns the mask, contiguous."""
+    costs no device synchronisation.  Returns the mask, contiguous.  `name` is the argument named in the errors (the
+    single-node heads' per-sensor mask, `sensor_valid`, has the same layout)."""
     if not isinstance(node_valid, torch.Tensor):
-        raise TypeError(f"node_valid must be a torch.bool tensor, got {type(node_valid).__name__}")
+        raise TypeError(f"{name} must be a torch.bool tensor, got {type(node_valid).__name__}")
     if node_valid.dtype != torch.bool:
-        raise TypeError(f"node_valid must be torch.bool, got {node_valid.dtype}")
+        raise TypeError(f"{name} must be torch.bool, got {node_valid.dtype}")
     rows = n_nodes if n_nodes is not None else (node_valid.shape[0] if node_valid.dim() == 2 else -1)
     if node_valid.dim() != 2 or rows < 1 or tuple(node_valid.shape) != (rows, B):
         want = f"[{n_nodes}, {B}]" if n_nodes is not None else f"[n_nodes, {B}]"
-        raise ValueError(f"node_valid must be {want}, got {list(node_valid.shape)}")
+        raise ValueError(f"{name} must be {want}, got {list(node_valid.shape)}")
     if node_valid.device != torch.device(device):
-        raise ValueError(f"node_valid must live on {torch.device(device)} (the features' device), got {node_valid.device}")
+        raise ValueError(f"{name} must live on {torch.device(device)} (the features' device), got {node_valid.device}")
     return node_valid.contiguous()
+
+
+def _mask_bytes(mask, B, device, rows, name):
+    """A checked bool mask [rows, B] as the uint8 device array the kernels read (a view: bool is one 0/1 byte)."""
+    return check_node_valid(mask, B, device, n_nodes=rows, name=name).view(torch.uint8)
 
 
 def _pc(pc_range):
@@ -165,9 +171,11 @@ def ray_query_pe(ref, lidar2img, img2lidar, depth_num, pad_h, pad_w, pc_range, o
     return out, mask
 
 
-def masked_view_sum(emb, mask, base=None):
+def masked_view_sum(emb, mask, base=None, view_valid=None):
     """base + (emb * mask[..., None]).sum(1)  (cmt_head.py:466, :492). emb [B,V,Nq,C] -> [B,Nq,C] fp32.
-    base: optional fp32 [B,Nq,C] or [Nq,C] (shared by every frame) added after the view sum."""
+    base: optional fp32 [B,Nq,C] or [Nq,C] (shared by every frame) added after the view sum.
+    view_valid: optional torch.bool [V, B] on emb's device; a view that is False for frame b is left out of its sum (its
+    embedding, NaN included, is not read), the others are summed in the same order."""
     emb = _cuda(emb, "emb")
     mask = _cuda(mask, "mask", torch.float32)
     B, V, Nq, C = emb.shape
@@ -177,10 +185,12 @@ def masked_view_sum(emb, mask, base=None):
         base = _cuda(base, "base", torch.float32)
         assert base.shape in ((B, Nq, C), (Nq, C))
         bstride = Nq * C if base.dim() == 3 else 0
+    if view_valid is not None:
+        view_valid = _mask_bytes(view_valid, B, emb.device, V, "view_valid")
     lib = _lib.load()
     with torch.cuda.device(emb.device):
         rc = lib.cmt_masked_view_sum(_ptr(emb), _ptr(mask), _ptr(base), bstride, _ptr(out), B, V, Nq, C, _dt(emb.dtype),
-                                     _stream(emb))
+                                     _stream(emb), _ptr(view_valid))
     _lib.check(rc, "cmt_masked_view_sum")
     _count()
     return out
@@ -205,11 +215,14 @@ _FEAT_DTYPES = {torch.float32: CMT_F32, torch.bfloat16: CMT_BF16, torch.float16:
 
 
 def gather_tokens(x_bev, x_img, bev_pos, rv_pos, B, V, out_dtype=torch.bfloat16, tok_range=None, n_bev_reserved=0,
-                  out=None, rv_rows=None):
+                  out=None, rv_rows=None, sensor_valid=None):
     """K4 (cmt_transformer.py:105-110 + petr_transformer.py:296-299).
     x_bev [B,C,Hb,Wb] | None, x_img [B*V,C,h,w] | None (fp32, bf16 or fp16 -- both the same dtype),
     bev_pos [N_bev,C], rv_pos [B*V*h*w, C] (any leading shape) fp32 -> xk = mem+pos, xv = mem, both
-    [B,N_kv,C]; with tok_range=(lo, hi) only those tokens of the concatenated axis: [B,hi-lo,C]."""
+    [B,N_kv,C]; with tok_range=(lo, hi) only those tokens of the concatenated axis: [B,hi-lo,C].
+    sensor_valid: optional torch.bool [S, B] on the features' device, one row per sensor in token order (the BEV map
+    first when there are BEV tokens, then the V cameras); the tokens of an absent (sensor, frame) become zero rows of
+    xk and xv, whatever its features and position encoding hold."""
     ref = x_bev if x_bev is not None else x_img
     dev = ref.device
     C = ref.shape[1]
@@ -234,6 +247,8 @@ def gather_tokens(x_bev, x_img, bev_pos, rv_pos, B, V, out_dtype=torch.bfloat16,
     if x_bev is None:
         n_bev = n_bev_reserved
     N_kv = n_bev + V * n_img
+    if sensor_valid is not None:
+        sensor_valid = _mask_bytes(sensor_valid, B, dev, (1 if n_bev > 0 else 0) + V, "sensor_valid")
     lo, hi = (0, N_kv) if tok_range is None else tok_range
     if out is not None:
         xk, xv = out
@@ -248,10 +263,27 @@ def gather_tokens(x_bev, x_img, bev_pos, rv_pos, B, V, out_dtype=torch.bfloat16,
         rc = lib.cmt_gather_tokens(_ptr(x_bev), _ptr(x_img), _ptr(bev_pos), _ptr(rv_pos), _ptr(xk), _ptr(xv),
                                    B, C, n_bev, V, n_img, lo, hi, 0 if rv_rows is None else rv_rows[0],
                                    0 if rv_rows is None else rv_rows[1] - rv_rows[0], _FEAT_DTYPES[fdt], _dt(out_dtype),
-                                   _stream(ref))
+                                   _stream(ref), _ptr(sensor_valid))
     _lib.check(rc, "cmt_gather_tokens")
     _count()
     return xk, xv
+
+
+def sensor_key_keep(sensor_valid, B, n_bev, V, n_img):
+    """The cross-attention's key mask from a per-sensor mask (cmt_sensor_key_keep): sensor_valid torch.bool [S, B]
+    (S = (n_bev > 0) + V, as in gather_tokens) -> torch.bool [B, n_bev + V*n_img], True where the token's sensor
+    delivered the frame (cross_attn's key_keep)."""
+    S = (1 if n_bev > 0 else 0) + V
+    if not isinstance(sensor_valid, torch.Tensor) or not sensor_valid.is_cuda:
+        raise _lib.CmtLibraryError("sensor_valid must be a CUDA tensor: libcmtcoop_b200 has no CPU fallback")
+    mask = _mask_bytes(sensor_valid, B, sensor_valid.device, S, "sensor_valid")
+    keep = torch.empty((B, n_bev + V * n_img), dtype=torch.bool, device=mask.device)
+    lib = _lib.load()
+    with torch.cuda.device(mask.device):
+        rc = lib.cmt_sensor_key_keep(_ptr(mask), _ptr(keep), B, n_bev, V, n_img, _stream(mask))
+    _lib.check(rc, "cmt_sensor_key_keep")
+    _count()
+    return keep
 
 
 def conv_guard_rows(W):
@@ -259,10 +291,11 @@ def conv_guard_rows(W):
     return (W + 3 + 7) // 8 * 8
 
 
-def nchw_to_padded_nhwc(x, out=None, dtype=torch.bfloat16):
+def nchw_to_padded_nhwc(x, out=None, dtype=torch.bfloat16, frame_valid=None):
     """[B,C,H,W] (fp32|bf16|fp16) -> zero-padded channel-last rows [B, 2*guard + (H+2)*(W+2), C] in `dtype` (bf16 or fp16)
     (cmt_nchw_to_padded_nhwc).  `out` (zero-initialised once, then reusable: only interior rows are written) is allocated
-    when None."""
+    when None.  frame_valid: optional torch.bool [B] on x's device; the interior rows of a False frame are written as
+    zeros (its input is not read)."""
     x = _cuda(x, "x")
     if x.dtype not in _FEAT_DTYPES:
         raise TypeError(f"feature maps must be fp32, bf16 or fp16, got {x.dtype}")
@@ -274,9 +307,12 @@ def nchw_to_padded_nhwc(x, out=None, dtype=torch.bfloat16):
     if out is None:
         out = torch.zeros((B, rows, C), dtype=dtype, device=x.device)
     assert out.shape == (B, rows, C) and out.dtype == dtype and out.is_contiguous()
+    if frame_valid is not None:
+        frame_valid = _mask_bytes(frame_valid.reshape(1, -1), B, x.device, 1, "frame_valid")
     lib = _lib.load()
     with torch.cuda.device(x.device), _timed("nchw_to_padded_nhwc", x):
-        rc = lib.cmt_nchw_to_padded_nhwc(_ptr(x), _ptr(out), B, C, H, W, guard, _FEAT_DTYPES[x.dtype], _stream(x), _dt(dtype))
+        rc = lib.cmt_nchw_to_padded_nhwc(_ptr(x), _ptr(out), B, C, H, W, guard, _FEAT_DTYPES[x.dtype], _stream(x), _dt(dtype),
+                                         _ptr(frame_valid))
     _lib.check(rc, "cmt_nchw_to_padded_nhwc")
     _count()
     return out
@@ -432,7 +468,7 @@ def cross_attn(q, k, vt, layer, *, kv_begin=0, kv_end=None, o_dtype=None, return
     """K3 (attention.py:46-92). q [B,Nq,H*32] pre-scaled by log2(e)/sqrt(32); k [B,L,H,N_kv,32];
     vt [B,L,H,32,ld]; attends tokens [kv_begin,kv_end) of layer `layer`. -> o [B,Nq,H*32] (, lse [B,H,Nq]).
     key_keep: optional [B,N_kv] bool/uint8, True = attend (the key_padding_mask of attention.py:76-90, whose
-    unpad_input keeps the True entries).
+    unpad_input keeps the True entries); a contiguous bool mask is read in place (no conversion launch).
     q_norm2 [B,H] / k_norm2 [B,L,H] fp32 (from the projections' norm2_max): enables the static softmax shift.
     q, k, vt: bf16 or fp16 (tcgen05 kernel) or fp32 (CUDA-core kernel); o_dtype: fp32 or q's dtype."""
     q = _cuda(q, "q")
@@ -474,7 +510,7 @@ def cross_attn(q, k, vt, layer, *, kv_begin=0, kv_end=None, o_dtype=None, return
     if key_keep is not None:
         key_keep = _cuda(key_keep, "key_keep")
         assert key_keep.shape == (B, N_kv), f"key_keep must be [B, N_kv] = {(B, N_kv)}, got {tuple(key_keep.shape)}"
-        key_keep = key_keep.to(torch.uint8).contiguous()
+        key_keep = key_keep.contiguous().view(torch.uint8) if key_keep.dtype == torch.bool else key_keep.to(torch.uint8).contiguous()
     qn = kn = None
     kn_stride = 0
     if q_norm2 is not None and k_norm2 is not None and tc and not FORCE_ONLINE_SOFTMAX:

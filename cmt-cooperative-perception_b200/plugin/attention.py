@@ -27,13 +27,16 @@ class KVCache:
     k:  [B, L, H, N_kv, 32]      vt: [B, L, H, 32, ld]
     k_norm2: [B, L, H] fp32 max_token |k|^2 (written by the K projection's epilogue), or None: with the matching
     query maxima it lets the attention kernel use a static softmax shift (ops.cross_attn).
+    key_keep: [B, N_kv] bool, False for the tokens of a sensor that did not deliver the frame (ops.sensor_key_keep), or
+    None: every cross-attention of every layer attends the True tokens only.
     """
 
-    def __init__(self, k, vt, n_kv, group=None, k_norm2=None, peer=None):
+    def __init__(self, k, vt, n_kv, group=None, k_norm2=None, peer=None, key_keep=None):
         self.peer = peer      # callable (B, Nq, H, device) -> parallel.PeerExchange: the layer's exchange + merge as one kernel over peer memory; None: NCCL all-gather
         self.k = k
         self.vt = vt
         self.k_norm2 = k_norm2
+        self.key_keep = key_keep
         self.n_kv = n_kv      # tokens held by THIS rank (all of them unless KV-split)
         self.group = group    # torch.distributed group when the token axis is split across ranks
 

@@ -462,8 +462,9 @@ class _CmtHeadBase(nn.Module):
         dt = _compute_dtype(self.precision)
         return self._mlp("bev_embedding", pos2embed(ref_points, num_pos_feats=self.hidden_dim, out_dtype=dt))
 
-    def _rv_query_embed(self, ref_points, img_metas, mats=None, base=None):
-        """cmt_head.py:439-467 (+ `base`, the BEV query embedding, added after the view sum: :492)."""
+    def _rv_query_embed(self, ref_points, img_metas, mats=None, base=None, view_valid=None):
+        """cmt_head.py:439-467 (+ `base`, the BEV query embedding, added after the view sum: :492).  view_valid: the
+        camera rows [V, B] of the sensor mask; an absent camera is left out of the view sum."""
         pad_h, pad_w, _ = img_metas[0]["pad_shape"][0]
         if mats is None:
             mats = self._matrices(img_metas, ref_points.device)
@@ -471,38 +472,51 @@ class _CmtHeadBase(nn.Module):
         feats, mask = ops.ray_query_pe(ref_points.contiguous(), mats[0], mats[1], self.depth_num, pad_h, pad_w,
                                        self.pc_range, out_dtype=dt)
         emb = self._mlp("rv_embedding", feats)
-        return ops.masked_view_sum(emb, mask, base=base)
+        return ops.masked_view_sum(emb, mask, base=base, view_valid=view_valid)
 
-    def query_embed(self, ref_points, img_metas, mats=None):
+    def query_embed(self, ref_points, img_metas, mats=None, view_valid=None):
         """cmt_head.py:469-473 -> (bev_query_embeds, rv_query_embeds)."""
         ref_points = inverse_sigmoid(ref_points.clone()).sigmoid()
         bev = self._bev_query_embed(ref_points, img_metas)
-        rv = self._rv_query_embed(ref_points, img_metas, mats) if self._has_img else None
+        rv = self._rv_query_embed(ref_points, img_metas, mats, view_valid=view_valid) if self._has_img else None
         return bev, rv
 
-    def _query_embeds(self, reference_points, img_metas, mats):
-        """bev + rv query embedding [B,Nq,C] (cmt_head.py:491-492) with the weight-only parts taken from the cache."""
+    def _query_embeds(self, reference_points, img_metas, mats, view_valid=None):
+        """bev + rv query embedding [B,Nq,C] (cmt_head.py:491-492) with the weight-only parts taken from the cache.
+        view_valid: the camera rows of the sensor mask (_rv_query_embed)."""
         B = reference_points.shape[0]
         d = None
         hit = self._cache.get("ref")
         if hit is not None and hit[1]["ref"] is reference_points:
             d = hit[1]
         if d is None or "bev_query" not in d:   # reference points not from prepare_for_dn: the general path
-            bev, rv = self.query_embed(reference_points, img_metas, mats)
+            bev, rv = self.query_embed(reference_points, img_metas, mats, view_valid)
             return bev if rv is None else bev + rv
         if not self._has_img:
             return d["bev_query"].unsqueeze(0).expand(B, -1, -1)
-        return self._rv_query_embed(d["ref_clamped"], img_metas, mats, base=d["bev_query"])
+        return self._rv_query_embed(d["ref_clamped"], img_metas, mats, base=d["bev_query"], view_valid=view_valid)
 
     # -- one node: shared_conv -> PEs -> transformer -> nan_to_num ---------------------------
     def get_outs_dec(self, x, x_img, img_metas, reference_points, attn_mask):
         """cmt_head_coop.py:341-360 (== cmt_head.py:481-499): stacked decoder outputs of one node, nan_to_num'ed."""
         return torch.nan_to_num(self._outs_dec_raw(x, x_img, img_metas, reference_points, attn_mask))
 
-    def _outs_dec_raw(self, x, x_img, img_metas, reference_points, attn_mask):
+    def _outs_dec_raw(self, x, x_img, img_metas, reference_points, attn_mask, sensor_valid=None):
         # without the nan_to_num: the fused task-head path applies it inside cmt_split3_bf16
         with _torch_math(self.precision):
-            return self._get_outs_dec(x, x_img, img_metas, reference_points, attn_mask)
+            return self._get_outs_dec(x, x_img, img_metas, reference_points, attn_mask, sensor_valid)
+
+    def _check_sensor_valid(self, sensor_valid, x, x_img, img_metas):
+        """Host-side checks of the single-node heads' per-frame sensor mask (torch.bool [S, B] on the features' device,
+        one row per sensor in token order: the LiDAR first when the head has BEV tokens, then the cameras in the order of
+        the img_feats views).  Returns it contiguous; the values are never read on the host."""
+        B = len(img_metas)
+        S = (1 if self._has_bev else 0) + (x_img.shape[0] // B if self._has_img else 0)
+        dev = (x if x is not None else x_img).device
+        sensor_valid = ops.check_node_valid(sensor_valid, B, dev, n_nodes=S, name="sensor_valid")
+        if self.transformer.kv_split_group is not None:
+            raise NotImplementedError("sensor_valid together with the multi-GPU KV-token split")
+        return sensor_valid
 
     def _node_cache(self, x, x_img, img_metas, reference_points):
         """Everything of one node up to the decoder: (query_embeds [B,Nq,C], KVCache) -- position encodings, token gather /
@@ -522,27 +536,33 @@ class _CmtHeadBase(nn.Module):
         cache, _ = tr.build_kv_cache(xb, x_img.contiguous() if self._has_img else None, bev_pos, rv_pos, B, V)
         return query_embeds, cache
 
-    def _get_outs_dec(self, x, x_img, img_metas, reference_points, attn_mask):
+    def _get_outs_dec(self, x, x_img, img_metas, reference_points, attn_mask, sensor_valid=None):
+        """sensor_valid: the checked [S, B] sensor mask (_check_sensor_valid) or None."""
         if self.training:
             raise NotImplementedError("libcmtcoop_b200 is forward/inference only (call .eval())")
         dev = (x if x is not None else x_img).device
         if dev.type != "cuda":
             raise RuntimeError("CmtHead needs CUDA tensors: libcmtcoop_b200 has no CPU fallback")
         mats = self._matrices(img_metas, dev) if self._has_img else None
-        query_embeds = self._query_embeds(reference_points, img_metas, mats)
+        view_valid = None
+        if sensor_valid is not None and self._has_img:
+            view_valid = sensor_valid[1:] if self._has_bev else sensor_valid
+        query_embeds = self._query_embeds(reference_points, img_metas, mats, view_valid)
         if self._has_bev and self._has_img:
             n_bev = x.shape[2] * x.shape[3]
             x = self._apply_shared_conv_to(x)
             rv_pos = self._rv_pe(x_img, img_metas, mats, n_bev=n_bev)
             outs_dec, _ = self.transformer(x, x_img, query_embeds, self._bev_pos_embed(dev), rv_pos,
-                                           attn_masks=attn_mask)
+                                           attn_masks=attn_mask, sensor_valid=sensor_valid)
         elif self._has_bev:
             x = self._apply_shared_conv_to(x)
             mask = None
-            outs_dec, _ = self.transformer(x, mask, query_embeds, self._bev_pos_embed(dev), attn_masks=attn_mask)
+            outs_dec, _ = self.transformer(x, mask, query_embeds, self._bev_pos_embed(dev), attn_masks=attn_mask,
+                                           sensor_valid=sensor_valid)
         else:
             rv_pos = self._rv_pe(x_img, img_metas, mats)
-            outs_dec, _ = self.transformer(x_img, query_embeds, rv_pos, attn_masks=attn_mask, bs=len(img_metas))
+            outs_dec, _ = self.transformer(x_img, query_embeds, rv_pos, attn_masks=attn_mask, bs=len(img_metas),
+                                           sensor_valid=sensor_valid)
         return outs_dec
 
     # -- task heads + reference-point decode (cmt_head.py:501-547, eval branch) ---------------
@@ -617,7 +637,8 @@ class _CmtHeadBase(nn.Module):
         applied, no host synchronisation (can be captured in a CUDA graph).  Returns the device-tensor dict
         {boxes [B,K,9], scores [B,K], labels [B,K], count [B], topk_index [B,K]} of `bbox_coder.decode_batched`;
         detector_glue.batched_to_results turns it into per-frame result dicts.  node_valid: the cooperative heads'
-        [2, B] node mask; frames with no node present get no detections."""
+        [2, B] node mask, or the single-node heads' [S, B] sensor mask; frames with no node / sensor present get no
+        detections."""
         return self.bbox_coder.decode_batched(preds_dicts, bottom_center=True, node_valid=node_valid)
 
 
@@ -625,15 +646,26 @@ class _CmtHeadBase(nn.Module):
 class CmtHead(_CmtHeadBase):
     """cmt_head.py:206-919 (multimodal: BEV + camera tokens)."""
 
-    def forward_single(self, x, x_img, img_metas):
+    def forward_single(self, x, x_img, img_metas, sensor_valid=None):
+        """sensor_valid: optional torch.bool [S, B] on the features' device, one row per sensor in token order -- row 0
+        the LiDAR (heads with BEV tokens), then the cameras in the order of the img_feats views and lidar2img -- False
+        where that sensor did not deliver the frame.  Each frame is then computed from its present sensors only, as the
+        reference would compute it on that frame alone with the absent views removed (x = None without the LiDAR).  An
+        absent sensor's features may hold anything (NaN included) and change no output bit; its lidar2img is not read
+        into any output but must stay invertible.  A frame with no sensor gets a zero cross-attention context and finite
+        outputs (get_bboxes_batched keeps nothing for it).  Absent sensors still cost their GPU time.  None: every
+        sensor is present (unchanged path)."""
+        if sensor_valid is not None:
+            sensor_valid = self._check_sensor_valid(sensor_valid, x, x_img, img_metas)
         reference_points = self.reference_points.weight
         reference_points, attn_mask, mask_dict = self.prepare_for_dn(x.shape[0], reference_points, img_metas)
-        outs_dec = self._outs_dec_raw(x, x_img, img_metas, reference_points, attn_mask)
+        outs_dec = self._outs_dec_raw(x, x_img, img_metas, reference_points, attn_mask, sensor_valid)
         return self._finish(outs_dec, reference_points)
 
-    def forward(self, pts_feats, img_feats=None, img_metas=None):
+    def forward(self, pts_feats, img_feats=None, img_metas=None, sensor_valid=None):
+        """sensor_valid: the per-frame sensor mask of forward_single, shared by every feature level."""
         img_metas = [img_metas for _ in range(len(pts_feats))]
-        return multi_apply(self.forward_single, pts_feats, img_feats, img_metas)
+        return multi_apply(self.forward_single, pts_feats, img_feats, img_metas, sensor_valid=sensor_valid)
 
 
 @HEADS.register_module()
@@ -641,11 +673,14 @@ class CmtImageHead(CmtHead):
     """cmt_head.py:922-999 (camera only; shared_conv is None)."""
     _has_bev = False
 
-    def forward_single(self, x, x_img, img_metas):
+    def forward_single(self, x, x_img, img_metas, sensor_valid=None):
+        """sensor_valid: as CmtHead.forward_single, one row per camera ([V, B])."""
         assert x is None
+        if sensor_valid is not None:
+            sensor_valid = self._check_sensor_valid(sensor_valid, None, x_img, img_metas)
         reference_points = self.reference_points.weight
         reference_points, attn_mask, mask_dict = self.prepare_for_dn(len(img_metas), reference_points, img_metas)
-        outs_dec = self._outs_dec_raw(None, x_img, img_metas, reference_points, attn_mask)
+        outs_dec = self._outs_dec_raw(None, x_img, img_metas, reference_points, attn_mask, sensor_valid)
         return self._finish(outs_dec, reference_points)
 
 
@@ -654,9 +689,12 @@ class CmtLidarHead(CmtHead):
     """cmt_head.py:1002-1085 (LiDAR only; rv_embedding is None)."""
     _has_img = False
 
-    def forward_single(self, x, x_img, img_metas):
+    def forward_single(self, x, x_img, img_metas, sensor_valid=None):
+        """sensor_valid: as CmtHead.forward_single, the LiDAR row only ([1, B])."""
         assert x_img is None
+        if sensor_valid is not None:
+            sensor_valid = self._check_sensor_valid(sensor_valid, x, None, img_metas)
         reference_points = self.reference_points.weight
         reference_points, attn_mask, mask_dict = self.prepare_for_dn(x.shape[0], reference_points, img_metas)
-        outs_dec = self._outs_dec_raw(x, None, img_metas, reference_points, attn_mask)
+        outs_dec = self._outs_dec_raw(x, None, img_metas, reference_points, attn_mask, sensor_valid)
         return self._finish(outs_dec, reference_points)

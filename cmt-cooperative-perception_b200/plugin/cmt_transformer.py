@@ -120,9 +120,15 @@ class _CmtTransformerBase(nn.Module):
         from .. import parallel
         return parallel.kv_split_range(n_kv, dist.get_rank(self.kv_split_group), dist.get_world_size(self.kv_split_group))
 
-    def build_kv_cache(self, x_bev, x_img, bev_pos, rv_pos, B, V):
+    def build_kv_cache(self, x_bev, x_img, bev_pos, rv_pos, B, V, sensor_valid=None):
         """gather (K4) + all-layer K / V^T projection (K2).  Returns (KVCache, xv [B,n_tok,C]) where n_tok is
-        this rank's share of the token axis (all tokens without the KV-token split)."""
+        this rank's share of the token axis (all tokens without the KV-token split).
+        sensor_valid: optional torch.bool [S, B] device mask, one row per sensor in token order (the BEV map first when
+        there is one, then the V cameras).  An absent sensor's tokens become zero rows of xk / xv (the fused shared_conv
+        path: zero input rows, hence finite conv rows) and the cache carries the [B, N_kv] key mask that drops them from
+        every cross-attention."""
+        if sensor_valid is not None and self.kv_split_group is not None:
+            raise NotImplementedError("sensor_valid together with the multi-GPU KV-token split")
         dt = _compute_dtype(self.precision)
         rv_rows = None
         n_img_tok = V * x_img.shape[2] * x_img.shape[3] if x_img is not None else 0
@@ -146,23 +152,29 @@ class _CmtTransformerBase(nn.Module):
             xk = torch.empty((B, hi - lo, C), dtype=dt, device=dev)
             xv = torch.empty((B, hi - lo, C), dtype=dt, device=dev)
             key = (tuple(x_bev.x.shape), str(dev), dt)
+            lidar_valid = None if sensor_valid is None else sensor_valid[0]
             if self._xp is None or self._xp[0] != key:   # zero-padded channel-last operand: zeroed once, interior rewritten per call
-                self._xp = (key, ops.nchw_to_padded_nhwc(x_bev.x, dtype=dt))
+                self._xp = (key, ops.nchw_to_padded_nhwc(x_bev.x, dtype=dt, frame_valid=lidar_valid))
             else:
-                ops.nchw_to_padded_nhwc(x_bev.x, self._xp[1], dtype=dt)
+                ops.nchw_to_padded_nhwc(x_bev.x, self._xp[1], dtype=dt, frame_valid=lidar_valid)
             if lo < n_bev:
                 ops.shared_conv_tokens(self._xp[1], x_bev.w, x_bev.bias, bev_pos, xk, xv, Hb, Wb, tok_range=(lo, min(hi, n_bev)))
             if x_img is not None and hi > n_bev:
                 ops.gather_tokens(None, x_img, None, rv_pos, B, V, out_dtype=dt, tok_range=(lo, hi), n_bev_reserved=n_bev,
-                                  out=(xk, xv), rv_rows=rv_rows)
+                                  out=(xk, xv), rv_rows=rv_rows, sensor_valid=sensor_valid)
         else:
             xk, xv = ops.gather_tokens(x_bev, x_img, bev_pos, rv_pos, B, V, out_dtype=dt,
-                                       tok_range=None if group is None else (lo, hi), rv_rows=rv_rows)
+                                       tok_range=None if group is None else (lo, hi), rv_rows=rv_rows,
+                                       sensor_valid=sensor_valid)
+        key_keep = None
+        if sensor_valid is not None:
+            key_keep = ops.sensor_key_keep(sensor_valid, B, n_kv - n_img_tok, V, n_img_tok // V if V else 0)
         wk, bk, wv, bv = self._stacked_kv_weights()
         kn2 = torch.zeros((B, L, H), dtype=torch.float32, device=xk.device) if dt != torch.float32 else None
         k = ops.project_keys(xk, wk, bk, L, H, norm2_max=kn2)
         vt = ops.project_values_t(xv, wv, bv, L, H)
-        return KVCache(k, vt, hi - lo, group, k_norm2=kn2, peer=self._peer_exchange if (group is not None and self.kv_split_peer) else None), xv
+        return KVCache(k, vt, hi - lo, group, k_norm2=kn2, peer=self._peer_exchange if (group is not None and self.kv_split_peer) else None,
+                       key_keep=key_keep), xv
 
     def enable_kv_split(self, group=None, peer_memory=False):
         """Split the K/V token axis across the ranks of `group` (default: the WORLD group); every rank
@@ -212,11 +224,12 @@ class _CmtTransformerBase(nn.Module):
 class CmtTransformer(_CmtTransformerBase):
     """cmt_transformer.py:48-127: BEV + image tokens."""
 
-    def forward(self, x, x_img, query_embed, bev_pos_embed, rv_pos_embed, attn_masks=None, reg_branch=None):
+    def forward(self, x, x_img, query_embed, bev_pos_embed, rv_pos_embed, attn_masks=None, reg_branch=None,
+                sensor_valid=None):
         bs = x.shape[0]
         V = x_img.shape[0] // bs
         cache, xv = self.build_kv_cache(x.contiguous(), x_img.contiguous(), bev_pos_embed.contiguous(),
-                                        rv_pos_embed.contiguous(), bs, V)
+                                        rv_pos_embed.contiguous(), bs, V, sensor_valid)
         out_dec = self._decode(cache, query_embed, attn_masks, reg_branch)
         return out_dec, (None if xv is None else xv.transpose(0, 1))  # memory as [N_kv,B,C] (compute dtype)
 
@@ -226,9 +239,9 @@ class CmtLidarTransformer(_CmtTransformerBase):
     """cmt_transformer.py:130-204: BEV tokens only. `mask` is accepted and ignored like the reference's
     all-zero key_padding_mask."""
 
-    def forward(self, x, mask, query_embed, pos_embed, attn_masks=None, reg_branch=None):
+    def forward(self, x, mask, query_embed, pos_embed, attn_masks=None, reg_branch=None, sensor_valid=None):
         bs = x.shape[0]
-        cache, xv = self.build_kv_cache(x.contiguous(), None, pos_embed.contiguous(), None, bs, 0)
+        cache, xv = self.build_kv_cache(x.contiguous(), None, pos_embed.contiguous(), None, bs, 0, sensor_valid)
         out_dec = self._decode(cache, query_embed, attn_masks, reg_branch)
         return out_dec, (None if xv is None else xv.transpose(0, 1))
 
@@ -237,8 +250,8 @@ class CmtLidarTransformer(_CmtTransformerBase):
 class CmtImageTransformer(_CmtTransformerBase):
     """cmt_transformer.py:207-282: image tokens only."""
 
-    def forward(self, x_img, query_embed, rv_pos_embed, attn_masks=None, reg_branch=None, bs=2):
+    def forward(self, x_img, query_embed, rv_pos_embed, attn_masks=None, reg_branch=None, bs=2, sensor_valid=None):
         V = x_img.shape[0] // bs
-        cache, xv = self.build_kv_cache(None, x_img.contiguous(), None, rv_pos_embed.contiguous(), bs, V)
+        cache, xv = self.build_kv_cache(None, x_img.contiguous(), None, rv_pos_embed.contiguous(), bs, V, sensor_valid)
         out_dec = self._decode(cache, query_embed, attn_masks, reg_branch)
         return out_dec, (None if xv is None else xv.transpose(0, 1))

@@ -50,11 +50,21 @@ def batched_to_results(batched, img_metas):
     return results
 
 
-def simple_test_pts(head, x, x_img, img_metas, rescale=False):
+def _drop_absent_frames(bbox_list, valid):
+    """Empty results for the frames none of whose nodes / sensors is present (valid: a [rows, B] device mask).  Called
+    after get_bboxes, which has synchronised already: reading the mask on the host costs nothing more."""
+    present = valid.any(0).tolist()
+    return [item if present[i] else [t[:0] for t in item] for i, item in enumerate(bbox_list)]
+
+
+def simple_test_pts(head, x, x_img, img_metas, rescale=False, sensor_valid=None):
     """CmtDetector.simple_test_pts (detectors/cmt.py:221-231). x / x_img: lists of feature levels as the detector's
-    extract_feat returns them (`[None]` for a missing modality)."""
-    outs = head(x, x_img, img_metas)
+    extract_feat returns them (`[None]` for a missing modality).  sensor_valid: optional torch.bool [S, B] device mask
+    of the sensors that delivered each frame (CmtHead.forward_single); a frame with no sensor gets an empty result."""
+    outs = head(x, x_img, img_metas, sensor_valid=sensor_valid)
     bbox_list = head.get_bboxes(outs, img_metas, rescale=rescale)
+    if sensor_valid is not None:
+        bbox_list = _drop_absent_frames(bbox_list, sensor_valid)
     return [bbox3d2result(bboxes, scores, labels) for bboxes, scores, labels in bbox_list]
 
 
@@ -74,20 +84,21 @@ def coop_simple_test_pts(head, vehicle_pts_feats, infrastructure_pts_feats, vehi
     outs = head(vehicle_pts_feats, infrastructure_pts_feats, vehicle_img_feats, infrastructure_img_feats, img_metas,
                 node_valid=node_valid)
     bbox_list = head.get_bboxes(outs, img_metas, rescale=rescale)
-    if node_valid is not None:   # get_bboxes has synchronised already: reading the mask on the host costs nothing more
-        present = node_valid.any(0).tolist()
-        bbox_list = [item if present[i] else [t[:0] for t in item] for i, item in enumerate(bbox_list)]
+    if node_valid is not None:
+        bbox_list = _drop_absent_frames(bbox_list, node_valid)
     return [bbox3d2result(bboxes, scores, labels) for bboxes, scores, labels in bbox_list]
 
 
-def simple_test(head, pts_feats, img_feats, img_metas, rescale=False):
-    """The part of CmtDetector.simple_test after extract_feat (detectors/cmt.py:233-252): per-frame result dicts."""
+def simple_test(head, pts_feats, img_feats, img_metas, rescale=False, sensor_valid=None):
+    """The part of CmtDetector.simple_test after extract_feat (detectors/cmt.py:233-252): per-frame result dicts.
+    sensor_valid: as in simple_test_pts."""
     if pts_feats is None:
         pts_feats = [None]
     if img_feats is None:
         img_feats = [None]
     bbox_list = [dict() for _ in range(len(img_metas))]
-    for result_dict, pts_bbox in zip(bbox_list, simple_test_pts(head, pts_feats, img_feats, img_metas, rescale=rescale)):
+    for result_dict, pts_bbox in zip(bbox_list, simple_test_pts(head, pts_feats, img_feats, img_metas, rescale=rescale,
+                                                                sensor_valid=sensor_valid)):
         result_dict["pts_bbox"] = pts_bbox
     return bbox_list
 

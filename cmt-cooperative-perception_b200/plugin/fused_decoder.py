@@ -167,13 +167,15 @@ def _run(decoder, query_pos, caches, precision):
             f0 = 0
             for c in caches:
                 nb = c.k.shape[0]
-                ops.cross_attn(qc[f0:f0 + nb], c.k, c.vt, li, out=ctx[f0:f0 + nb],
+                ops.cross_attn(qc[f0:f0 + nb], c.k, c.vt, li, out=ctx[f0:f0 + nb], key_keep=c.key_keep,
                                q_norm2=qn2[li][f0:f0 + nb] if static_shift else None, k_norm2=c.k_norm2 if static_shift else None)
                 f0 += nb
             assert f0 == B
         elif cache.group is None:
-            ctx = ops.cross_attn(qc, cache.k, cache.vt, li, q_norm2=qn2[li] if static_shift else None,
-                                 k_norm2=cache.k_norm2 if static_shift else None)
+            # key_keep (sensor mask): the masked rows are finite (zero or ReLU(bias) features), so the operand-norm
+            # bounds that include them still bound every attended score
+            ctx = ops.cross_attn(qc, cache.k, cache.vt, li, key_keep=cache.key_keep,
+                                 q_norm2=qn2[li] if static_shift else None, k_norm2=cache.k_norm2 if static_shift else None)
         else:
             ctx = mha._merge_kv_split(qc, cache, li, q_norm2=qn2[li] if static_shift else None)
         ca = ops.linear(ctx, cw["wo"], cw["bo"], out_dtype=torch.float32)

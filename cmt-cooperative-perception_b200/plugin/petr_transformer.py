@@ -124,7 +124,9 @@ class PETRMultiheadFlashAttention(nn.Module):
                 key = key + key_pos
             out = self.attn(q=q, k=key.transpose(0, 1), v=value.transpose(0, 1), key_padding_mask=None)[0]
         else:
-            out = self.attn(q=q, k=None, v=None, key_padding_mask=None, kv_cache=kv_cache, layer_index=layer_index)[0]
+            # the sensor mask of the cache (None unless a sensor is missing for some frames) is the key_padding_mask
+            out = self.attn(q=q, k=None, v=None, key_padding_mask=kv_cache.key_keep, kv_cache=kv_cache,
+                            layer_index=layer_index)[0]
         out = out.transpose(0, 1)
         return identity + self.dropout_layer(self.proj_drop(out))
 

@@ -59,19 +59,22 @@ class numa_local_to_gpu:
 
 
 def _head_forward(head, coop, inputs, metas, decode_boxes):
-    """head.forward_single on an inputs dict (feature tensors, plus "node_valid" for the cooperative heads), followed
-    by the batched box decode with decode_boxes."""
+    """head.forward_single on an inputs dict (feature tensors, plus "node_valid" for the cooperative heads or
+    "sensor_valid" for the single-node heads), followed by the batched box decode with decode_boxes."""
     g = inputs.get
-    node_valid = g("node_valid")
     if coop:
+        if g("sensor_valid") is not None:
+            raise ValueError("sensor_valid is an input of the single-node heads only (the cooperative heads take node_valid)")
+        mask = g("node_valid")
         rets = head.forward_single(g("vehicle_pts_feats"), g("infrastructure_pts_feats"), g("vehicle_img_feats"),
-                                   g("infrastructure_img_feats"), metas, node_valid=node_valid)
+                                   g("infrastructure_img_feats"), metas, node_valid=mask)
     else:
-        if node_valid is not None:
+        if g("node_valid") is not None:
             raise ValueError("node_valid is an input of the cooperative heads only")
-        rets = head.forward_single(g("pts_feats"), g("img_feats"), metas)
+        mask = g("sensor_valid")
+        rets = head.forward_single(g("pts_feats"), g("img_feats"), metas, sensor_valid=mask)
     if decode_boxes:
-        return rets, head.get_bboxes_batched([[r] for r in rets], metas, node_valid=node_valid)
+        return rets, head.get_bboxes_batched([[r] for r in rets], metas, node_valid=mask)
     return rets
 
 
@@ -82,7 +85,8 @@ class PipelinedRunner:
         (pts_feats / img_feats, or the four vehicle_/infrastructure_ entries for the coop heads); fp32, bf16 or
         fp16 -- the gather kernel rounds every feature to the compute dtype on arrival, so 16-bit features halve
         the PCIe traffic without changing a single output bit in bf16 mode.  A cooperative head may also take
-        "node_valid", a pinned torch.bool [2, B] mask of the nodes that delivered each frame (forward_single); it is
+        "node_valid", a pinned torch.bool [2, B] mask of the nodes that delivered each frame, and a single-node head
+        "sensor_valid", a pinned torch.bool [S, B] mask of the sensors that delivered each frame (forward_single); it is
         copied in with every batch like the features and, with outputs="boxes", also reaches the decode.
         use_cuda_graph: replay one captured forward per device input slot instead of launching eagerly.
         keep_results: `run` returns every batch's outputs as ordinary CPU tensors (copied out of the two pinned
@@ -295,8 +299,9 @@ class GraphedForward:
     With decode_boxes=True the graph also holds `head.get_bboxes_batched` of the outputs, and a call returns
     (head outputs, boxes dict), both static outputs of the graph.
 
-    For a cooperative head the inputs may include "node_valid" (torch.bool [2, B], forward_single): like the features it
-    lives in a static buffer that each call overwrites, so a new mask is one small copy and never a re-capture.
+    For a cooperative head the inputs may include "node_valid" (torch.bool [2, B]), for a single-node head
+    "sensor_valid" (torch.bool [S, B]; forward_single): like the features it lives in a static buffer that each call
+    overwrites, so a new mask is one small copy and never a re-capture.
 
     The graph bakes in device addresses, so the inputs live in static buffers (`g.static_inputs`) and the outputs are
     overwritten by the next replay.  The calibration matrices enter the forward as device tensors uploaded once per

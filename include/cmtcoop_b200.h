@@ -72,9 +72,12 @@ int cmt_ray_query_pe(const float* ref, const float* lidar2img, const float* img2
 
 /* out[b,n,:] = base[b,n,:] + sum_v mask[b,v,n] * emb[b,v,n,:]  (cmt_head.py:466 and the `bev + rv` of :492).
  * emb fp32|bf16|fp16, out fp32; base (nullable) fp32 at base + b*base_bstride + n*C (base_bstride = 0: one [Nq,C]
- * embedding shared by every frame -- in eval the BEV query embedding depends on the weights only). */
+ * embedding shared by every frame -- in eval the BEV query embedding depends on the weights only).
+ * view_valid (nullable DEVICE array, since version 103): uint8 [V, B], entry [v][b] != 0 when camera v delivered frame b.
+ * An absent view is left out of the sum (its emb and mask are not read, so NaN there changes nothing); the present
+ * views are summed in the same order as without the mask.  NULL: every view is present. */
 int cmt_masked_view_sum(const void* emb, const float* mask, const float* base, int64_t base_bstride, float* out,
-                        int B, int V, int Nq, int C, int emb_dtype, void* stream);
+                        int B, int V, int Nq, int C, int emb_dtype, void* stream, const uint8_t* view_valid);
 
 /* ---- sine/cosine BEV embedding ------------------------------------------------------
  * pos2embed (cmt_head.py:40-50) including its `dim_t = 2*(i//2)/F + 1` divisor.
@@ -98,11 +101,20 @@ int cmt_pos2embed(const float* pos, void* out, int N, int pos_stride, int F, int
  * [B, tok_end - tok_begin, C] (0, N_kv = everything; a sub-range = this rank's share of a KV-token
  * split).  rv_rows > 0: rv_pos holds only rows [rv_tok0, rv_tok0 + rv_rows) of every frame's V*n_img image tokens,
  * [B, rv_rows, C] (the rank computed the rv-PE MLP for its own tokens only); rv_rows = 0: all of them.
- * out dtype fp32|bf16|fp16. */
+ * out dtype fp32|bf16|fp16.
+ * sensor_valid (nullable DEVICE array, since version 103): uint8 [S, B], one row per sensor in token order -- row 0 the
+ * BEV map when n_bev > 0, then the V cameras -- entry [s][b] != 0 when sensor s delivered frame b.  Every token of an
+ * absent (sensor, frame) is written as a zero row of xk and of xv; its features and position encoding are not read
+ * (they may hold anything, NaN included).  NULL: every sensor is present. */
 int cmt_gather_tokens(const void* x_bev, const void* x_img, const float* bev_pos,
                       const float* rv_pos, void* xk, void* xv, int B, int C, int n_bev, int V,
                       int n_img, int tok_begin, int tok_end, int rv_tok0, int rv_rows, int feat_dtype, int out_dtype,
-                      void* stream);
+                      void* stream, const uint8_t* sensor_valid);
+
+/* Key-keep bytes of cmt_cross_attn_fwd from the sensor mask of cmt_gather_tokens (since version 103):
+ * key_keep [B, n_bev + V*n_img] uint8 (DEVICE), entry [b][t] = 1 when the sensor of token t delivered frame b, else 0
+ * (sensor_valid [S, B] as there, S = (n_bev > 0) + V). */
+int cmt_sensor_key_keep(const uint8_t* sensor_valid, uint8_t* key_keep, int B, int n_bev, int V, int n_img, void* stream);
 
 /* ---- K2: projection / MLP GEMM ------------------------------------------------------
  * C = act((A * B^T + bias) * alpha); A:[M,K] (lda), B:[N,K] (ldb), both row-major, K contiguous.
@@ -155,9 +167,12 @@ int cmt_gemm_segmented(const void* A, const void* B, const float* bias, void* C,
  *   for every frame b and token t = y*W + x in [tok_begin, tok_end):
  *     v = ReLU(conv(x)[b,:,y,x] + bias);  xv[b][t - tok_begin][:] = dtype(v);  xk[b][t - tok_begin][:] = dtype(v + bev_pos[t])
  *   with out_frame_stride elements between frames (N_kv * Cout: the image tokens follow, cmt_gather_tokens with
- *   x_bev = NULL).  Cin % 64 == 0, Cout % 32 == 0, Cout <= 1984. */
+ *   x_bev = NULL).  Cin % 64 == 0, Cout % 32 == 0, Cout <= 1984.
+ * frame_valid (cmt_nchw_to_padded_nhwc, nullable DEVICE array, since version 103): uint8 [B]; the interior rows of a
+ *   frame b with frame_valid[b] == 0 are written as zeros and its input is not read, so step 2 produces finite rows
+ *   ReLU(bias) (+ bev_pos) for it.  NULL: every frame is present. */
 int cmt_nchw_to_padded_nhwc(const void* x, void* out, int B, int C, int H, int W, int guard_rows, int in_dtype,
-                            void* stream, int out_dtype);
+                            void* stream, int out_dtype, const uint8_t* frame_valid);
 int cmt_shared_conv_tokens(const void* xp, const void* w, const float* bias, const float* bev_pos, void* xk, void* xv,
                            int B, int Cin, int Cout, int H, int W, int guard_rows, int64_t out_frame_stride,
                            int tok_begin, int tok_end, void* stream, int dtype);

@@ -20,3 +20,4 @@ run multi tests/test_gpu_multi.py
 run decode tests/test_gpu_bbox_decode.py
 run fp16 tests/test_gpu_fp16.py
 run node_mask tests/test_gpu_coop_node_mask.py
+run sensor_mask tests/test_gpu_sensor_mask.py
