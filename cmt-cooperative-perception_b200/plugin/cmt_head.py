@@ -387,17 +387,15 @@ class _CmtHeadBase(nn.Module):
         return hit[1]
 
     def _apply_shared_conv_to(self, x):
-        """The BEV map the transformer consumes: the input itself (bench scope), a BevTokenSource for the fused
-        implicit-GEMM path (bf16 and fp16 modes), or torch's conv + BN + ReLU in fp32."""
+        """(BEV map, folded shared_conv) for build_kv_cache: (x, None) for the input itself (bench scope), (x, (w, bias))
+        for the fused implicit-GEMM path (bf16 and fp16 modes), or (torch's conv + BN + ReLU of x, None) in fp32."""
         if not self.apply_shared_conv:
-            return x
+            return x, None
         conv = self.shared_conv.conv
         if (self.precision in ("bf16", "fp16") and self.fuse_shared_conv and conv.kernel_size == (3, 3) and conv.in_channels % 64 == 0
                 and conv.out_channels % 32 == 0):
-            from .cmt_transformer import BevTokenSource
-            w, b = self._shared_conv_folded()
-            return BevTokenSource(x, w, b)
-        return self.shared_conv(x.float())
+            return x, self._shared_conv_folded()
+        return self.shared_conv(x.float()), None
 
     # -- position encodings -----------------------------------------------------------------
     def _matrices(self, img_metas, device):
@@ -426,8 +424,10 @@ class _CmtHeadBase(nn.Module):
         return hit
 
     def _rv_pe(self, img_feats, img_metas, mats=None, n_bev=0):
-        """cmt_head.py:417-433 -> [B*V,H,W,C] fp32.  Under the KV-token split a rank needs the encodings of its own image
-        tokens only: the MLP (22 GF per frame) then runs on that row range and an RvPosRows is returned."""
+        """cmt_head.py:417-433 -> ([B*V,H,W,C] fp32, None).  Under the KV-token split a rank needs the encodings of its own
+        image tokens only: the MLP (22 GF per frame) then runs on that row range [a, b) of every frame's V*H*W image
+        tokens, and ([B, b-a, C], (a, b)) is returned (build_kv_cache's rv_rows), or (None, (0, 0)) when the rank's share
+        holds no image token."""
         BN, C, H, W = img_feats.shape
         pad_h, pad_w, _ = img_metas[0]["pad_shape"][0]
         if mats is None:
@@ -438,13 +438,12 @@ class _CmtHeadBase(nn.Module):
         n_img = (BN // B) * H * W
         lo, hi = self.transformer.kv_token_range(n_bev + n_img)
         if (lo, hi) != (0, n_bev + n_img):
-            from .cmt_transformer import RvPosRows
             a, b = max(lo - n_bev, 0), max(hi - n_bev, 0)
             if b <= a:
-                return RvPosRows(coords.new_zeros((B, 0, self.hidden_dim), dtype=torch.float32), 0, 0)
+                return None, (0, 0)
             rows = coords.view(B, n_img, -1)[:, a:b].contiguous()
-            return RvPosRows(self._mlp("rv_embedding", rows, tag="rv_pe_mlp"), a, b)
-        return self._mlp("rv_embedding", coords, tag="rv_pe_mlp")
+            return self._mlp("rv_embedding", rows, tag="rv_pe_mlp"), (a, b)
+        return self._mlp("rv_embedding", coords, tag="rv_pe_mlp"), None
 
     def _bev_pos_embed(self, device):
         """bev_embedding(pos2embed(coords_bev)) (cmt_head.py:489): input independent -> cached per weights."""
@@ -499,12 +498,10 @@ class _CmtHeadBase(nn.Module):
     # -- one node: shared_conv -> PEs -> transformer -> nan_to_num ---------------------------
     def get_outs_dec(self, x, x_img, img_metas, reference_points, attn_mask):
         """cmt_head_coop.py:341-360 (== cmt_head.py:481-499): stacked decoder outputs of one node, nan_to_num'ed."""
-        return torch.nan_to_num(self._outs_dec_raw(x, x_img, img_metas, reference_points, attn_mask))
-
-    def _outs_dec_raw(self, x, x_img, img_metas, reference_points, attn_mask, sensor_valid=None):
-        # without the nan_to_num: the fused task-head path applies it inside cmt_split3_bf16
         with _torch_math(self.precision):
-            return self._get_outs_dec(x, x_img, img_metas, reference_points, attn_mask, sensor_valid)
+            query_embeds, cache = self._node_cache(x, x_img, img_metas, reference_points)
+            outs_dec = self.transformer.decode([cache], query_embeds, attn_mask)
+        return torch.nan_to_num(outs_dec)
 
     def _check_sensor_valid(self, sensor_valid, x, x_img, img_metas):
         """Host-side checks of the single-node heads' per-frame sensor mask (torch.bool [S, B] on the features' device,
@@ -518,52 +515,28 @@ class _CmtHeadBase(nn.Module):
             raise NotImplementedError("sensor_valid together with the multi-GPU KV-token split")
         return sensor_valid
 
-    def _node_cache(self, x, x_img, img_metas, reference_points):
-        """Everything of one node up to the decoder: (query_embeds [B,Nq,C], KVCache) -- position encodings, token gather /
-        shared_conv, all-layer K / V^T projection.  Used by the cooperative heads to decode both nodes in one pass."""
+    def _node_cache(self, x, x_img, img_metas, reference_points, sensor_valid=None):
+        """Everything of one node up to the decoder: (query_embeds [B,Nq,C], KVCache) -- query embedding, position
+        encodings, token gather / shared_conv, all-layer K / V^T projection.  sensor_valid: the checked [S, B] sensor mask
+        (_check_sensor_valid) or None; its camera rows leave absent views out of the query embedding."""
         dev = (x if x is not None else x_img).device
         if dev.type != "cuda":
             raise RuntimeError("CmtHead needs CUDA tensors: libcmtcoop_b200 has no CPU fallback")
         B = len(img_metas)
         mats = self._matrices(img_metas, dev) if self._has_img else None
-        query_embeds = self._query_embeds(reference_points, img_metas, mats)
-        tr = self.transformer
-        bev_pos = self._bev_pos_embed(dev).contiguous() if self._has_bev else None
-        n_bev = x.shape[2] * x.shape[3] if self._has_bev else 0
-        rv_pos = self._rv_pe(x_img, img_metas, mats, n_bev=n_bev).contiguous() if self._has_img else None
-        xb = self._apply_shared_conv_to(x).contiguous() if self._has_bev else None
-        V = (x_img.shape[0] // B) if self._has_img else 0
-        cache, _ = tr.build_kv_cache(xb, x_img.contiguous() if self._has_img else None, bev_pos, rv_pos, B, V)
-        return query_embeds, cache
-
-    def _get_outs_dec(self, x, x_img, img_metas, reference_points, attn_mask, sensor_valid=None):
-        """sensor_valid: the checked [S, B] sensor mask (_check_sensor_valid) or None."""
-        if self.training:
-            raise NotImplementedError("libcmtcoop_b200 is forward/inference only (call .eval())")
-        dev = (x if x is not None else x_img).device
-        if dev.type != "cuda":
-            raise RuntimeError("CmtHead needs CUDA tensors: libcmtcoop_b200 has no CPU fallback")
-        mats = self._matrices(img_metas, dev) if self._has_img else None
         view_valid = None
         if sensor_valid is not None and self._has_img:
             view_valid = sensor_valid[1:] if self._has_bev else sensor_valid
         query_embeds = self._query_embeds(reference_points, img_metas, mats, view_valid)
-        if self._has_bev and self._has_img:
-            n_bev = x.shape[2] * x.shape[3]
-            x = self._apply_shared_conv_to(x)
-            rv_pos = self._rv_pe(x_img, img_metas, mats, n_bev=n_bev)
-            outs_dec, _ = self.transformer(x, x_img, query_embeds, self._bev_pos_embed(dev), rv_pos,
-                                           attn_masks=attn_mask, sensor_valid=sensor_valid)
-        elif self._has_bev:
-            x = self._apply_shared_conv_to(x)
-            mask = None
-            outs_dec, _ = self.transformer(x, mask, query_embeds, self._bev_pos_embed(dev), attn_masks=attn_mask,
-                                           sensor_valid=sensor_valid)
-        else:
-            rv_pos = self._rv_pe(x_img, img_metas, mats)
-            outs_dec, _ = self.transformer(x_img, query_embeds, rv_pos, attn_masks=attn_mask, bs=len(img_metas),
-                                           sensor_valid=sensor_valid)
-        return outs_dec
+        x_bev, conv = self._apply_shared_conv_to(x) if self._has_bev else (None, None)
+        n_bev = x.shape[2] * x.shape[3] if self._has_bev else 0
+        rv_pos, rv_rows = self._rv_pe(x_img, img_metas, mats, n_bev=n_bev) if self._has_img else (None, None)
+        bev_pos = self._bev_pos_embed(dev) if self._has_bev else None
+        V = (x_img.shape[0] // B) if self._has_img else 0
+        cache, _ = self.transformer.build_kv_cache(None if x_bev is None else x_bev.contiguous(),
+                                                   None if x_img is None else x_img.contiguous(), bev_pos, rv_pos, B, V,
+                                                   conv=conv, rv_rows=rv_rows, sensor_valid=sensor_valid)
+        return query_embeds, cache
 
     # -- task heads + reference-point decode (cmt_head.py:501-547, eval branch) ---------------
     def _finish(self, outs_dec, reference_points, outs_dec_other=None, stacked_nodes=False, node_valid=None):
@@ -654,12 +627,18 @@ class CmtHead(_CmtHeadBase):
         absent sensor's features may hold anything (NaN included) and change no output bit; its lidar2img is not read
         into any output but must stay invertible.  A frame with no sensor gets a zero cross-attention context and finite
         outputs (get_bboxes_batched keeps nothing for it).  Absent sensors still cost their GPU time.  None: every
-        sensor is present (unchanged path)."""
+        sensor is present (unchanged path).  CmtImageHead takes one row per camera ([V, B]), CmtLidarHead the LiDAR row
+        only ([1, B])."""
+        assert self._has_bev or x is None
+        assert self._has_img or x_img is None
         if sensor_valid is not None:
             sensor_valid = self._check_sensor_valid(sensor_valid, x, x_img, img_metas)
         reference_points = self.reference_points.weight
-        reference_points, attn_mask, mask_dict = self.prepare_for_dn(x.shape[0], reference_points, img_metas)
-        outs_dec = self._outs_dec_raw(x, x_img, img_metas, reference_points, attn_mask, sensor_valid)
+        reference_points, attn_mask, mask_dict = self.prepare_for_dn(len(img_metas), reference_points, img_metas)
+        with _torch_math(self.precision):
+            query_embeds, cache = self._node_cache(x, x_img, img_metas, reference_points, sensor_valid)
+            # without the nan_to_num of get_outs_dec: the fused task-head path applies it inside cmt_split3_bf16
+            outs_dec = self.transformer.decode([cache], query_embeds, attn_mask)
         return self._finish(outs_dec, reference_points)
 
     def forward(self, pts_feats, img_feats=None, img_metas=None, sensor_valid=None):
@@ -673,28 +652,8 @@ class CmtImageHead(CmtHead):
     """cmt_head.py:922-999 (camera only; shared_conv is None)."""
     _has_bev = False
 
-    def forward_single(self, x, x_img, img_metas, sensor_valid=None):
-        """sensor_valid: as CmtHead.forward_single, one row per camera ([V, B])."""
-        assert x is None
-        if sensor_valid is not None:
-            sensor_valid = self._check_sensor_valid(sensor_valid, None, x_img, img_metas)
-        reference_points = self.reference_points.weight
-        reference_points, attn_mask, mask_dict = self.prepare_for_dn(len(img_metas), reference_points, img_metas)
-        outs_dec = self._outs_dec_raw(None, x_img, img_metas, reference_points, attn_mask, sensor_valid)
-        return self._finish(outs_dec, reference_points)
-
 
 @HEADS.register_module()
 class CmtLidarHead(CmtHead):
     """cmt_head.py:1002-1085 (LiDAR only; rv_embedding is None)."""
     _has_img = False
-
-    def forward_single(self, x, x_img, img_metas, sensor_valid=None):
-        """sensor_valid: as CmtHead.forward_single, the LiDAR row only ([1, B])."""
-        assert x_img is None
-        if sensor_valid is not None:
-            sensor_valid = self._check_sensor_valid(sensor_valid, x, None, img_metas)
-        reference_points = self.reference_points.weight
-        reference_points, attn_mask, mask_dict = self.prepare_for_dn(x.shape[0], reference_points, img_metas)
-        outs_dec = self._outs_dec_raw(x, None, img_metas, reference_points, attn_mask, sensor_valid)
-        return self._finish(outs_dec, reference_points)

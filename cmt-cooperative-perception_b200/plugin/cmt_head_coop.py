@@ -11,7 +11,7 @@ from __future__ import annotations
 import torch
 
 from .. import ops
-from .cmt_head import _CmtHeadBase, multi_apply
+from .cmt_head import _CmtHeadBase, _torch_math, multi_apply
 from .registry import HEADS
 
 
@@ -41,13 +41,6 @@ class CmtHeadCoop(_CmtHeadBase):
 
     batch_nodes = True   # decode both nodes' frames in one pass (False: two sequential decoder passes like the reference)
 
-    def _merge(self, out_v, out_i):
-        if out_v is None:
-            return out_i
-        if out_i is None:
-            return out_v
-        return ops.coop_max(out_v.contiguous(), out_i.contiguous())  # max(stack([veh, infra]), 0)
-
     def forward_single(self, x_vehicle, x_infrastructure, x_img_vehicle, x_img_infrastructure, img_metas, node_valid=None):
         """node_valid: optional torch.bool [2, B] on the features' device, row 0 the vehicle and row 1 the infrastructure:
         False where that node did not deliver the frame.  Such a frame's features of that node may hold anything (NaN
@@ -64,32 +57,28 @@ class CmtHeadCoop(_CmtHeadBase):
             node_valid = ops.check_node_valid(node_valid, len(img_metas), dev)
         reference_points = self.reference_points.weight
         reference_points, attn_mask, mask_dict = self.prepare_for_dn(len(img_metas), reference_points, img_metas)
-        if (has_v and has_i and attn_mask is None and self.batch_nodes and not self.training
-                and self.transformer.kv_split_group is None):
-            # Both nodes in ONE decoder pass: the reference runs the same decoder (shared weights, same reference points)
-            # once per node (cmt_head_coop.py:368-389, :946-1017); frames are independent, so stacking the two nodes'
-            # frames changes no arithmetic -- every small op of the decoder runs once over 2B frames, the cross-attention
-            # is launched per node (their token counts differ), and the V2I max + nan_to_num ride in the task heads'
-            # first kernel.
-            from .cmt_head import _torch_math
-            with _torch_math(self.precision):
-                q_v, c_v = self._node_cache(x_vehicle, x_img_vehicle, get_vehicle_image_metas(img_metas), reference_points)
-                q_i, c_i = self._node_cache(x_infrastructure, x_img_infrastructure, get_infrastructure_image_metas(img_metas),
-                                            reference_points)
-                outs = self.transformer.decode_nodes([c_v, c_i], torch.cat([q_v, q_i], 0))
-            if outs is not None:
-                return self._finish(outs, reference_points, stacked_nodes=True, node_valid=node_valid)
-        out_v = out_i = None
-        if x_vehicle is not None or x_img_vehicle is not None:
-            out_v = self._outs_dec_raw(x_vehicle, x_img_vehicle, get_vehicle_image_metas(img_metas),
-                                       reference_points, attn_mask)
-        if x_infrastructure is not None or x_img_infrastructure is not None:
-            out_i = self._outs_dec_raw(x_infrastructure, x_img_infrastructure,
-                                       get_infrastructure_image_metas(img_metas), reference_points, attn_mask)
-        if out_v is None or out_i is None:
-            return self._finish(out_v if out_i is None else out_i, reference_points)
+        nodes = []
+        if has_v:
+            nodes.append((x_vehicle, x_img_vehicle, get_vehicle_image_metas(img_metas)))
+        if has_i:
+            nodes.append((x_infrastructure, x_img_infrastructure, get_infrastructure_image_metas(img_metas)))
+        stacked = None
+        with _torch_math(self.precision):
+            built = [self._node_cache(x, x_img, metas, reference_points) for x, x_img, metas in nodes]
+            if len(built) == 2 and self.batch_nodes:
+                # Both nodes in ONE decoder pass: the reference runs the same decoder (shared weights, same reference
+                # points) once per node (cmt_head_coop.py:368-389, :946-1017); frames are independent, so stacking the two
+                # nodes' frames changes no arithmetic -- every small op of the decoder runs once over 2B frames, the
+                # cross-attention is launched per node (their token counts differ), and the V2I max + nan_to_num ride in
+                # the task heads' first kernel.
+                stacked = self.transformer.decode([c for _, c in built], torch.cat([q for q, _ in built], 0), attn_mask)
+            if stacked is None:
+                outs = [self.transformer.decode([c], q, attn_mask) for q, c in built]
+        if stacked is not None:
+            return self._finish(stacked, reference_points, stacked_nodes=True, node_valid=node_valid)
         # max(stack([veh, infra]), 0) (cmt_head_coop.py:383-389) is folded into the task heads' first kernel
-        return self._finish(out_v, reference_points, outs_dec_other=out_i, node_valid=node_valid)
+        return self._finish(outs[0], reference_points, outs_dec_other=outs[1] if len(outs) == 2 else None,
+                            node_valid=node_valid)
 
     def forward(self, vehicle_pts_feats, infrastructure_pts_feats, vehicle_img_feats=None,
                 infrastructure_img_feats=None, img_metas=None, node_valid=None):

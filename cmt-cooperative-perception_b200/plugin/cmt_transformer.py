@@ -21,36 +21,6 @@ from .registry import TRANSFORMER
 _compute_dtype = ops.compute_dtype
 
 
-class RvPosRows:
-    """Image-token position encodings of a sub-range only: rows [a, b) of every frame's V*h*w image tokens, [B, b-a, C]
-    (a rank of the KV-token split runs the rv-PE MLP on its own tokens).  Stands in for rv_pos_embed."""
-
-    def __init__(self, rows, a, b):
-        self.rows, self.a, self.b = rows, a, b
-
-    def contiguous(self):
-        self.rows = self.rows.contiguous()
-        return self
-
-
-class BevTokenSource:
-    """The BEV map BEFORE shared_conv together with the folded conv + BN parameters: handed to the transformer in place
-    of the convolved [B,C,H,W] tensor so that the 3x3 convolution runs as a tcgen05 implicit GEMM whose epilogue writes
-    the BEV token rows of xk / xv directly (cmt_head.py:280-287,481 fused with cmt_transformer.py:105-110 and
-    petr_transformer.py:296-299).  Quacks like the tensor as far as the transformer's forward signature needs."""
-
-    def __init__(self, x_raw, w, bias):
-        self.x = x_raw                      # [B, Cin, H, W] fp32 | bf16 | fp16
-        self.w = w                          # [Cout, 9*Cin] in the compute dtype (bf16 | fp16), tap-major, BN scale folded in
-        self.bias = bias                    # [Cout] fp32
-        self.shape = (x_raw.shape[0], w.shape[0], x_raw.shape[2], x_raw.shape[3])
-        self.device = x_raw.device
-
-    def contiguous(self):
-        self.x = self.x.contiguous()
-        return self
-
-
 class _CmtTransformerBase(nn.Module):
     def __init__(self, encoder=None, decoder=None, init_cfg=None, cross=False):
         super().__init__()
@@ -120,20 +90,21 @@ class _CmtTransformerBase(nn.Module):
         from .. import parallel
         return parallel.kv_split_range(n_kv, dist.get_rank(self.kv_split_group), dist.get_world_size(self.kv_split_group))
 
-    def build_kv_cache(self, x_bev, x_img, bev_pos, rv_pos, B, V, sensor_valid=None):
+    def build_kv_cache(self, x_bev, x_img, bev_pos, rv_pos, B, V, conv=None, rv_rows=None, sensor_valid=None):
         """gather (K4) + all-layer K / V^T projection (K2).  Returns (KVCache, xv [B,n_tok,C]) where n_tok is
         this rank's share of the token axis (all tokens without the KV-token split).
+        conv: None, or the folded shared_conv (w [Cout, 9*Cin] tap-major in the compute dtype with the BN scale folded in,
+        bias [Cout] fp32); x_bev is then the map BEFORE shared_conv, and the 3x3 convolution runs as a tcgen05 implicit
+        GEMM whose epilogue writes the BEV token rows of xk / xv directly (cmt_head.py:280-287,481 fused with
+        cmt_transformer.py:105-110 and petr_transformer.py:296-299).
+        rv_rows: None, or (a, b) when rv_pos holds rows [a, b) of every frame's V*h*w image tokens only, [B, b-a, C] (a
+        rank of the KV-token split runs the rv-PE MLP on its own tokens; a == b: its share holds no image token).
         sensor_valid: optional torch.bool [S, B] device mask, one row per sensor in token order (the BEV map first when
         there is one, then the V cameras).  An absent sensor's tokens become zero rows of xk / xv (the fused shared_conv
         path: zero input rows, hence finite conv rows) and the cache carries the [B, N_kv] key mask that drops them from
         every cross-attention."""
-        if sensor_valid is not None and self.kv_split_group is not None:
-            raise NotImplementedError("sensor_valid together with the multi-GPU KV-token split")
         dt = _compute_dtype(self.precision)
-        rv_rows = None
         n_img_tok = V * x_img.shape[2] * x_img.shape[3] if x_img is not None else 0
-        if isinstance(rv_pos, RvPosRows):
-            rv_pos, rv_rows = rv_pos.rows, (rv_pos.a, rv_pos.b)
         n_kv = (x_bev.shape[2] * x_bev.shape[3] if x_bev is not None else 0) + n_img_tok
         lo, hi = self.kv_token_range(n_kv)
         if rv_rows is not None and rv_rows[1] <= rv_rows[0]:
@@ -144,21 +115,22 @@ class _CmtTransformerBase(nn.Module):
         if hi <= lo:   # more ranks than token tiles: this rank contributes the neutral element of the merge
             return KVCache(None, None, 0, group, peer=self._peer_exchange if self.kv_split_peer else None), None
         # with the split, the gather kernel itself produces only the rank's rows: K1/K4/K2 all shard with the tokens
-        if isinstance(x_bev, BevTokenSource):
+        if conv is not None:
             Hb, Wb = x_bev.shape[2], x_bev.shape[3]
             n_bev = Hb * Wb
-            C = x_bev.shape[1]
+            w, bias = conv
+            C = w.shape[0]
             dev = x_bev.device
             xk = torch.empty((B, hi - lo, C), dtype=dt, device=dev)
             xv = torch.empty((B, hi - lo, C), dtype=dt, device=dev)
-            key = (tuple(x_bev.x.shape), str(dev), dt)
+            key = (tuple(x_bev.shape), str(dev), dt)
             lidar_valid = None if sensor_valid is None else sensor_valid[0]
             if self._xp is None or self._xp[0] != key:   # zero-padded channel-last operand: zeroed once, interior rewritten per call
-                self._xp = (key, ops.nchw_to_padded_nhwc(x_bev.x, dtype=dt, frame_valid=lidar_valid))
+                self._xp = (key, ops.nchw_to_padded_nhwc(x_bev, dtype=dt, frame_valid=lidar_valid))
             else:
-                ops.nchw_to_padded_nhwc(x_bev.x, self._xp[1], dtype=dt, frame_valid=lidar_valid)
+                ops.nchw_to_padded_nhwc(x_bev, self._xp[1], dtype=dt, frame_valid=lidar_valid)
             if lo < n_bev:
-                ops.shared_conv_tokens(self._xp[1], x_bev.w, x_bev.bias, bev_pos, xk, xv, Hb, Wb, tok_range=(lo, min(hi, n_bev)))
+                ops.shared_conv_tokens(self._xp[1], w, bias, bev_pos, xk, xv, Hb, Wb, tok_range=(lo, min(hi, n_bev)))
             if x_img is not None and hi > n_bev:
                 ops.gather_tokens(None, x_img, None, rv_pos, B, V, out_dtype=dt, tok_range=(lo, hi), n_bev_reserved=n_bev,
                                   out=(xk, xv), rv_rows=rv_rows, sensor_valid=sensor_valid)
@@ -201,22 +173,21 @@ class _CmtTransformerBase(nn.Module):
             self._peer = parallel.PeerExchange(self.kv_split_group, device, B, Nq, H, L)
         return self._peer
 
-    def decode_nodes(self, caches, query_embed, attn_masks=None):
-        """One decoder pass over several nodes' frames (query_embed [sum B_i, Nq, C], caches[i] covering B_i frames) when
-        the fused decoder supports the configuration; None otherwise (the caller then decodes node by node)."""
-        if self.training or not self.use_fused_decoder or not fused_decoder.supports(self.decoder, attn_masks, list(caches)):
-            return None
-        return fused_decoder.run(self.decoder, query_embed, list(caches), self.precision)
-
-    def _decode(self, cache, query_embed, attn_masks, reg_branch):
+    def decode(self, caches, query_embed, attn_masks=None):
+        """Decoder pass over the frames of a list of KVCaches: query_embed [sum B_i, Nq, C], caches[i] covering the next
+        B_i frames.  Returns the stacked outputs [L, sum B_i, Nq, C].  The fused decoder takes every cache in one pass
+        when it supports the configuration; otherwise a single cache goes through the module-by-module path and several
+        caches give None (the caller then decodes each cache on its own)."""
         if self.training:
             raise NotImplementedError("libcmtcoop_b200 is forward/inference only (call .eval())")
-        if self.use_fused_decoder and fused_decoder.supports(self.decoder, attn_masks, cache):
-            return fused_decoder.run(self.decoder, query_embed, cache, self.precision)  # [L,B,Nq,C]
+        if self.use_fused_decoder and fused_decoder.supports(self.decoder, attn_masks, caches):
+            return fused_decoder.run(self.decoder, query_embed, caches, self.precision)
+        if len(caches) > 1:
+            return None
         query_embed = query_embed.transpose(0, 1)  # [B,Nq,C] -> [Nq,B,C]
         target = torch.zeros_like(query_embed)
         out_dec = self.decoder(query=target, key=None, value=None, key_pos=None, query_pos=query_embed,
-                               key_padding_mask=None, attn_masks=[attn_masks, None], kv_cache=cache)
+                               key_padding_mask=None, attn_masks=[attn_masks, None], kv_cache=caches[0])
         return out_dec.transpose(1, 2)  # [L,B,Nq,C]
 
 
@@ -224,13 +195,12 @@ class _CmtTransformerBase(nn.Module):
 class CmtTransformer(_CmtTransformerBase):
     """cmt_transformer.py:48-127: BEV + image tokens."""
 
-    def forward(self, x, x_img, query_embed, bev_pos_embed, rv_pos_embed, attn_masks=None, reg_branch=None,
-                sensor_valid=None):
+    def forward(self, x, x_img, query_embed, bev_pos_embed, rv_pos_embed, attn_masks=None, reg_branch=None):
         bs = x.shape[0]
         V = x_img.shape[0] // bs
         cache, xv = self.build_kv_cache(x.contiguous(), x_img.contiguous(), bev_pos_embed.contiguous(),
-                                        rv_pos_embed.contiguous(), bs, V, sensor_valid)
-        out_dec = self._decode(cache, query_embed, attn_masks, reg_branch)
+                                        rv_pos_embed.contiguous(), bs, V)
+        out_dec = self.decode([cache], query_embed, attn_masks)
         return out_dec, (None if xv is None else xv.transpose(0, 1))  # memory as [N_kv,B,C] (compute dtype)
 
 
@@ -239,10 +209,10 @@ class CmtLidarTransformer(_CmtTransformerBase):
     """cmt_transformer.py:130-204: BEV tokens only. `mask` is accepted and ignored like the reference's
     all-zero key_padding_mask."""
 
-    def forward(self, x, mask, query_embed, pos_embed, attn_masks=None, reg_branch=None, sensor_valid=None):
+    def forward(self, x, mask, query_embed, pos_embed, attn_masks=None, reg_branch=None):
         bs = x.shape[0]
-        cache, xv = self.build_kv_cache(x.contiguous(), None, pos_embed.contiguous(), None, bs, 0, sensor_valid)
-        out_dec = self._decode(cache, query_embed, attn_masks, reg_branch)
+        cache, xv = self.build_kv_cache(x.contiguous(), None, pos_embed.contiguous(), None, bs, 0)
+        out_dec = self.decode([cache], query_embed, attn_masks)
         return out_dec, (None if xv is None else xv.transpose(0, 1))
 
 
@@ -250,8 +220,8 @@ class CmtLidarTransformer(_CmtTransformerBase):
 class CmtImageTransformer(_CmtTransformerBase):
     """cmt_transformer.py:207-282: image tokens only."""
 
-    def forward(self, x_img, query_embed, rv_pos_embed, attn_masks=None, reg_branch=None, bs=2, sensor_valid=None):
+    def forward(self, x_img, query_embed, rv_pos_embed, attn_masks=None, reg_branch=None, bs=2):
         V = x_img.shape[0] // bs
-        cache, xv = self.build_kv_cache(None, x_img.contiguous(), None, rv_pos_embed.contiguous(), bs, V, sensor_valid)
-        out_dec = self._decode(cache, query_embed, attn_masks, reg_branch)
+        cache, xv = self.build_kv_cache(None, x_img.contiguous(), None, rv_pos_embed.contiguous(), bs, V)
+        out_dec = self.decode([cache], query_embed, attn_masks)
         return out_dec, (None if xv is None else xv.transpose(0, 1))

@@ -74,12 +74,12 @@ def _ln(norm: nn.LayerNorm):
     return norm.weight.detach(), norm.bias.detach(), norm.eps
 
 
-def supports(decoder, attn_masks, kv_cache) -> bool:
-    """True when the fused path computes exactly what the generic module path would."""
-    if isinstance(kv_cache, (list, tuple)):
-        if not kv_cache or any(c is None or c.group is not None or c.k is None for c in kv_cache):
-            return False
-    if kv_cache is None or decoder.training or not decoder.return_intermediate or decoder.post_norm is None:
+def supports(decoder, attn_masks, caches) -> bool:
+    """True when the fused path computes exactly what the generic module path would.  caches: the list of KVCaches
+    `run` would decode; several caches in one pass need every one unsplit and holding keys."""
+    if len(caches) > 1 and any(c.group is not None or c.k is None for c in caches):
+        return False
+    if decoder.training or not decoder.return_intermediate or decoder.post_norm is None:
         return False
     if attn_masks is not None and any(m is not None for m in (attn_masks if isinstance(attn_masks, (list, tuple))
                                                                else [attn_masks])):
@@ -99,20 +99,12 @@ def supports(decoder, attn_masks, kv_cache) -> bool:
     return True
 
 
-def run(decoder, query_pos: torch.Tensor, cache, precision: str) -> torch.Tensor:
+def run(decoder, query_pos: torch.Tensor, caches, precision: str) -> torch.Tensor:
     """query_pos [B,Nq,C] fp32 (batch-first).  Returns the stacked post-normed outputs [L,B,Nq,C] fp32.
-    cache: one KVCache for all B frames, or a list of KVCaches covering consecutive frame ranges (the cooperative heads:
-    both nodes' frames in ONE decoder pass -- shared weights and the same queries, cmt_head_coop.py:368-389 -- with one
-    cross-attention launch per node because the nodes' token counts differ; every small op runs once over 2B frames)."""
-    if isinstance(cache, (list, tuple)):
-        if len(cache) == 1:
-            cache = cache[0]
-        else:
-            return _run(decoder, query_pos, list(cache), precision)
-    return _run(decoder, query_pos, [cache], precision)
-
-
-def _run(decoder, query_pos, caches, precision):
+    caches: a list of KVCaches covering consecutive frame ranges of the B frames -- one for all of them, or one per node
+    for the cooperative heads: both nodes' frames in ONE decoder pass (shared weights and the same queries,
+    cmt_head_coop.py:368-389) with one cross-attention launch per node because the nodes' token counts differ; every
+    small op runs once over 2B frames."""
     cache = caches[0]
     dt = ops.compute_dtype(precision)
     B, Nq, C = query_pos.shape

@@ -62,6 +62,40 @@ def test_fused_decoder_equals_module_path(kind, precision, tol):
         assert O.rel_l2(fused[0][name].float().cpu(), modular[0][name].float().cpu()) < tol, name
 
 
+@pytest.mark.parametrize("kind", ["CmtHead", "CmtImageHead", "CmtLidarHead"])
+def test_reference_signature_transformer_forward(kind):
+    """`head.transformer(...)` with the reference's arguments (cmt_transformer.py:84-127, :166-204, :243-282), called on
+    the query embedding and position encodings the head computes, returns the head's own decoder output bit for bit
+    and the token memory as [N_kv, B, C]."""
+    cfg, inputs = synth.mini_case(kind)
+    head = build_head(cfg)
+    synth.load_synth_weights(head, 0)
+    head = head.to(DEV).eval()
+    head.apply_shared_conv = False   # the transformer's x is the map after shared_conv
+    d = {k: (torch.from_numpy(v).to(DEV) if isinstance(v, np.ndarray) else v) for k, v in inputs.items()}
+    x, x_img, metas = d.get("pts_feats"), d.get("img_feats"), d["img_metas"]
+    B = len(metas)
+    tr = head.transformer
+    with torch.no_grad():
+        if x is not None:
+            x = head.shared_conv(x).contiguous()
+        ref, attn_mask, _ = head.prepare_for_dn(B, head.reference_points.weight, metas)
+        want = head.get_outs_dec(x, x_img, metas, ref, attn_mask)
+        mats = head._matrices(metas, x_img.device) if x_img is not None else None
+        query = head._query_embeds(ref, metas, mats)
+        if kind == "CmtHead":
+            out_dec, memory = tr(x, x_img, query, head._bev_pos_embed(x.device), head._rv_pe(x_img, metas, mats)[0],
+                                 attn_masks=attn_mask)
+        elif kind == "CmtLidarHead":
+            out_dec, memory = tr(x, None, query, head._bev_pos_embed(x.device), attn_masks=attn_mask)
+        else:
+            out_dec, memory = tr(x_img, query, head._rv_pe(x_img, metas, mats)[0], attn_masks=attn_mask, bs=B)
+    assert torch.isfinite(out_dec).all()   # so the head's nan_to_num leaves its output as the decoder wrote it
+    assert torch.equal(out_dec, want)
+    n_kv = (x.shape[2] * x.shape[3] if x is not None else 0) + (x_img[0, 0].numel() * (x_img.shape[0] // B) if x_img is not None else 0)
+    assert memory.shape == (n_kv, B, out_dec.shape[-1])
+
+
 @pytest.mark.parametrize("precision,tol", [("fp32", 1e-4), ("bf16", 1e-2)])
 def test_flash_mha_key_padding_mask(precision, tol):
     """FlashMHA.forward(q, k, v, key_padding_mask) (attention.py:126-138 -> :76-90) against the oracle's
