@@ -12,6 +12,7 @@ run() {
 run simple tests/test_gpu_kernels.py -k "not gemm and not attention"
 run gemm tests/test_gpu_kernels.py -k "gemm"
 run gemm_geometry tests/test_gpu_gemm_geometry.py
+run forward_replay tests/test_gpu_forward_replay.py
 run attn tests/test_gpu_kernels.py -k "attention"
 run attn_edges tests/test_gpu_attention_edges.py
 run heads tests/test_gpu_heads.py
